@@ -1,8 +1,14 @@
 #!/usr/bin/env python
 """bench.py — planned frames/sec at 1M-frame batches (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
+
+--dump-outputs DIR writes, after the timed steps, what the last timed step computed (rank 0) as
+DIR/<name>.npy in float64, at most 64 MB in all: per-frame (per-rollout) arrays at a fixed seeded
+sample of the frames when all of them do not fit, DIR/sample_index.npy naming the frames.  The
+inputs depend on the arguments alone, so two builds run with the same arguments can be compared
+file for file.
 
 Secondary lines (not the headline): --workload rollouts (BASELINE configs[2], closed-loop
 ego-frames/s), --workload sweep (configs[3], candidate trajectories/s), --cars 64 (configs[4]).
@@ -77,6 +83,45 @@ def peaks():
     return 6650.0, "fallback (B200_PROFILING.md)"
 
 
+DUMP_BYTES = 64_000_000  # --dump-outputs: all files together
+DUMP_SEED = 0xD1
+
+
+def sample_outputs(rows, whole):
+    """--dump-outputs: `rows` (torch tensors or numpy arrays with one row per frame / rollout)
+    at every row, or at a fixed seeded sample of rows when they would not fit in DUMP_BYTES,
+    and `whole` (small arrays) as they are.  Tensors are gathered on their device, so the
+    result survives later work on the buffers and the copy to the host can wait
+    (write_outputs)."""
+    import numpy as np
+    import torch
+    n = len(next(iter(rows.values())))
+    row_bytes = 8 * (1 + sum(int(np.prod(v.shape[1:])) for v in rows.values()))
+    headers = 128 * (1 + len(rows) + len(whole))  # one .npy header per file
+    fit = (DUMP_BYTES - headers - 8 * sum(int(np.prod(v.shape)) for v in whole.values())) // row_bytes
+    idx = np.arange(n) if n <= fit else \
+        np.sort(np.random.default_rng(DUMP_SEED).choice(n, fit, replace=False))
+    out = {"sample_index": idx, **whole}
+    for k, v in rows.items():
+        out[k] = v[torch.from_numpy(idx).to(v.device)] if torch.is_tensor(v) else v[idx]
+    return out
+
+
+def write_outputs(out_dir, arrays):
+    """Each array as out_dir/<name>.npy in float64 (the integers the path computes are below
+    2**53, flags below 2**31)."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in arrays.items():
+        v = v.cpu().numpy() if torch.is_tensor(v) else np.asarray(v)
+        np.save(os.path.join(out_dir, k + ".npy"), v.astype(np.float64))
+
+
+def dump_outputs(out_dir, rows, whole):
+    write_outputs(out_dir, sample_outputs(rows, whole))
+
+
 def cpu_threads():
     try:
         return max(1, len(os.sched_getaffinity(0)))
@@ -126,6 +171,8 @@ def run_reference(args):
         if i >= args.warmup:
             total_t += t
             total_f += n
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, bufs[1].arrays(), {})
     value = total_f / total_t
     line = {
         "impl": "reference", "metric": METRIC, "value": value, "unit": "frames/s",
@@ -189,7 +236,7 @@ def run_rollouts(args):
     sampler = ClockSampler(local, period_s=0.02) if rank == 0 else None
     launches0 = pp.launch_count()
     ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    steps = max(1, args.steps if args.steps != 50 else 1)
+    steps = args.steps
     ev0.record()
     for _ in range(steps):
         ro.run(ticks, args.consume_k)
@@ -205,6 +252,11 @@ def run_rollouts(args):
     ms = float(t[0])
     if rank == 0:
         stats = st.cpu().numpy()
+        if args.dump_outputs:
+            state = ro.state()
+            dump_outputs(args.dump_outputs,
+                         {k: getattr(state, k) for k, _, _ in pp.abi.ROLLOUT_STATE_FIELDS},
+                         {"stats": stats})
         line = {"metric": "closed-loop ego-frames/sec (rollout-ticks)",
                 "value": world * n * ticks * steps / (ms * 1e-3), "unit": "frames/s",
                 "n_gpus": world, "steps": steps, "warmup": 3, "ms_per_step": ms / steps,
@@ -244,7 +296,7 @@ def run_sweep(args):
     n = args.frames if args.frames != FRAMES_PER_GPU else 32768
     frames = pp.synth_frames(m, n, args.cars, seed=SEED, first_frame=rank * n)
     df = pp.DeviceFrames(frames)
-    steps = args.steps if args.steps != 50 else 5
+    steps = args.steps
     for _ in range(max(3, args.warmup)):
         out = pp.sweep_batch(m, df, want_scores=False)
     torch.cuda.synchronize()
@@ -264,6 +316,8 @@ def run_sweep(args):
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
     ms = float(t[0])
     if rank == 0:
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, {k: v for k, v in out.items() if v is not None}, {})
         cands = 384
         best = out["best"].cpu().numpy()
         line = {"metric": "sweep candidates/sec (384 candidate trajectories per frame)",
@@ -456,7 +510,8 @@ def cpu_baseline_legs(pp, m, n, cars):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=50)
+    ap.add_argument("--steps", type=int, default=None,
+                    help="timed steps (default: 50; dense64 3, sweep 5, rollouts 1)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--frames", type=int, default=None,
@@ -479,7 +534,14 @@ def main():
     ap.add_argument("--rollouts", type=int, default=65536, help="rollouts per GPU")
     ap.add_argument("--ticks", type=int, default=1000)
     ap.add_argument("--consume-k", type=int, default=1)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps is None:  # (the reference arm plans the frames workload whatever --workload says)
+        args.steps = 50 if args.impl == "reference" else \
+            {"dense64": 3, "sweep": 5, "rollouts": 1}.get(args.workload, 50)
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     quiet_stdout()
     if args.workload in ("rollouts", "sweep") and args.frames is None:
         args.frames = FRAMES_PER_GPU
@@ -517,8 +579,6 @@ def main():
             n = min(total // world, cap)
         else:
             n = min(total, cap)
-        if args.steps == 50:
-            args.steps = 3
         workload = (f"configs[4]: {total} frames x 64 cars in total, generated in HBM "
                     f"(pp_synth_frames_dev), {n} frames resident per GPU"
                     + (" (the largest single-GPU slice)" if n * world < total else ""))
@@ -580,6 +640,9 @@ def main():
     launches = pp.launch_count() - launches0
     stats = st_buf.cpu().numpy().copy()
     fstats = fs_buf.cpu().numpy().copy()
+    dump = None
+    if args.dump_outputs and rank == 0:  # gathered on the device before the loops below plan into dp again
+        dump = sample_outputs(dp.t, {"stats": stats, "fstats": fstats})
     # pp_plan_batch alone (the pipeline without the statistics pass), for the roofline
     for i in range(args.steps):
         k_start[i].record(stream)
@@ -587,6 +650,8 @@ def main():
         k_stop[i].record(stream)
     fence()
     clocks = sampler.stop() if sampler else None  # (both loops above run the GPU flat out)
+    if dump is not None:
+        write_outputs(args.dump_outputs, dump)
     # Per-kernel breakdown: in the timed region four chunks are in flight at once, so a kernel's
     # own duration cannot be read there.  A few extra (untimed) steps run the same launches
     # strictly one after the other with CUDA events around each kernel.

@@ -6,8 +6,9 @@
                          %.4f by reference src/main.cpp:1200-1208) — the only
                          known-answer data for Map::Init in the reference tree.
   frames_c12.npz         768 synthetic frames (12 cars, 30 % steered into rare
-  frames_c64.npz         branches) / 96 frames (64 cars): inputs AND the outputs
-                         of the reference's own code (oracle/_ref/libppref.so).
+  frames_c64.npz         branches) / 96 frames (64 cars): the inputs, and in
+  frames_<tag>_out.npz   a file of their own (to keep each file below 1 MB) the
+                         outputs of the reference's own code (oracle/_ref/libppref.so).
   units.npz              inputs/outputs of the reference's individual functions.
 
     python tests/golden/make_golden.py
@@ -44,9 +45,10 @@ def frames():
         fb = pp.synth_frames(m, n, cars, seed=seed, rare_permille=300)
         plans = ref.plan(fb, want_flags=True)
         blob = {"in_" + k: v for k, v in fb.arrays().items()}
-        blob.update({"out_" + k: v for k, v in plans.arrays().items()})
         blob["observable_flags"] = np.uint32(ref.observable_flags)
         np.savez_compressed(os.path.join(HERE, f"frames_{tag}.npz"), **blob)
+        np.savez_compressed(os.path.join(HERE, f"frames_{tag}_out.npz"),
+                            **{"out_" + k: v for k, v in plans.arrays().items()})
         print(f"frames_{tag}.npz", n, "frames; flag counts",
               {pp.FLAG_NAMES[i]: int(((plans.flags >> i) & 1).sum()) for i in range(pp.NUM_FLAGS)
                if ((plans.flags >> i) & 1).any()})
