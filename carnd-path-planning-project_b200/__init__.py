@@ -44,7 +44,8 @@ EXPORTS = [
     "pp_dev_alloc", "pp_dev_free", "pp_host_alloc", "pp_host_free", "pp_dev_upload", "pp_dev_download", "pp_dev_sync",
     "pp_dev_set", "pp_stream_create", "pp_stream_sync", "pp_stream_destroy",
     "pp_rollouts_create", "pp_rollouts_destroy", "pp_rollouts_run", "pp_rollouts_last",
-    "pp_rollouts_get_state", "pp_rollouts_stats", "pp_rollouts_set_lean", "pp_rollouts_set_groups", "pp_sweep_batch",
+    "pp_rollouts_get_state", "pp_rollouts_stats", "pp_rollouts_set_lean", "pp_rollouts_set_groups",
+    "pp_rollouts_get_incidents", "pp_rollouts_incident_totals", "pp_sweep_batch",
     "pp_set_pipes", "pp_plan_stats_batch", "pp_synth_frames_dev", "pp_fstats_batch",
     "pp_comm_unique_id", "pp_comm_init_rank", "pp_comm_init_all", "pp_comm_destroy",
     "pp_comm_group_begin", "pp_comm_group_end", "pp_stats_reduce",
@@ -474,6 +475,27 @@ class Rollouts:
         out = torch.zeros(STATS_LEN, dtype=torch.int64, device="cuda")
         _check(lib.pp_rollouts_stats(self._h, C.c_void_p(out.data_ptr()), C.c_void_p(stream)),
                "pp_rollouts_stats")
+        return out
+
+    def incidents(self) -> dict:
+        """The incident monitor's record (include/pp.h, pp_rollout_incidents) as numpy arrays:
+        count [n][INC_KINDS] (columns in the order of abi.INC_NAMES), first_tick / first_kind [n]
+        (-1: none), distance_m, clean_m, best_clean_m, max_speed, max_acc, max_jerk [n]."""
+        out = {name: np.zeros((self.n, abi.INC_KINDS) if kind else (self.n,), dtype=dt)
+               for name, dt, kind in abi.INC_FIELDS}
+        s = abi.RolloutIncidents(*[a.ctypes.data for a in out.values()])
+        _check(lib.pp_rollouts_get_incidents(self._h, C.byref(s)), "pp_rollouts_get_incidents")
+        return out
+
+    def incident_totals(self, stream=None):
+        """pp_rollouts_incident_totals -> int64[INC_TOTALS_LEN] device tensor: counts per kind,
+        rollouts with at least one incident, driven millimetres."""
+        import torch
+        if stream is None:
+            stream = torch.cuda.current_stream().cuda_stream
+        out = torch.empty(abi.INC_TOTALS_LEN, dtype=torch.int64, device="cuda")
+        _check(lib.pp_rollouts_incident_totals(self._h, C.c_void_p(out.data_ptr()),
+                                               C.c_void_p(stream)), "pp_rollouts_incident_totals")
         return out
 
     def close(self):

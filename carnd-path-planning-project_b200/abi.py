@@ -152,6 +152,26 @@ class RolloutState(C.Structure):
     _fields_ = [(n, _dp) for n, _, _ in ROLLOUT_STATE_FIELDS] + [("tick", C.c_int64)]
 
 
+# incident monitor of the rollouts (pp_rollout_incidents): kinds in the order of PP_INC_*
+INC_NAMES = ["collision_front", "collision_rear", "over_speed", "over_acc", "over_jerk",
+             "out_of_lane", "off_road"]
+INC = {name: i for i, name in enumerate(INC_NAMES)}
+INC_KINDS = len(INC_NAMES)
+INC_TOTAL_ROLLOUTS = INC_KINDS      # pp_rollouts_incident_totals: rollouts with an incident
+INC_TOTAL_MM = INC_KINDS + 1        # ... driven distance in millimetres
+INC_TOTALS_LEN = INC_KINDS + 2
+INC_HISTORY = 70                   # driven points the jerk reaches back (PP_INC_HISTORY)
+INC_FIELDS = [  # (name, dtype, inner) ; inner: 0 scalar, 'kinds'
+    ("count", np.int32, "kinds"), ("first_tick", np.int64, 0), ("first_kind", np.int32, 0),
+    ("distance_m", np.float64, 0), ("clean_m", np.float64, 0), ("best_clean_m", np.float64, 0),
+    ("max_speed", np.float64, 0), ("max_acc", np.float64, 0), ("max_jerk", np.float64, 0),
+]
+
+
+class RolloutIncidents(C.Structure):
+    _fields_ = [(n, _dp) for n, _, _ in INC_FIELDS]
+
+
 def default_config() -> Config:
     """The literals of reference src/main.cpp:30,39-49 (also what
     pp_config_default writes; tests check the two agree)."""

@@ -10,6 +10,7 @@
 #include <cstring>
 #include <vector>
 
+#include "pp_device.cuh"
 #include "pp_internal.h"
 
 struct pp_rollouts {
@@ -46,6 +47,12 @@ struct pp_rollouts {
   pp_config graph_cfg;
   int64_t launches_per_tick = 0;
   int groups_wanted = 0;  // pp_rollouts_set_groups: 0 = automatic
+  // incident monitor (pp.h, pp_rollout_incidents); device arrays in `buf`
+  double2 *inc_ring, *inc_ring_acc;
+  int64_t *inc_pts, *inc_first_tick;
+  uint32_t *inc_active;
+  int32_t *inc_off, *inc_count, *inc_first_kind;
+  double *inc_d[6];  // distance_m, clean_m, best_clean_m, max_speed, max_acc, max_jerk
 };
 
 namespace {
@@ -105,20 +112,193 @@ struct Track {
     w %= n;
     if (w < 0) w += n;
   }
-  // position and velocity of a car at (lane, w, u) moving at v
-  __host__ __device__ void car(int lane, int w, double u, double v, double &x, double &y,
-                               double &vx, double &vy) const {
+  // position and unit lane tangent of a car at (lane, w, u)
+  __host__ __device__ void pose(int lane, int w, double u, double &x, double &y, double &tx,
+                                double &ty) const {
     const double *a = row(w - 1), *b = row(w);
     const double ax = a[2 + 2 * lane], ay = a[3 + 2 * lane];
     const double bx = b[2 + 2 * lane], by = b[3 + 2 * lane];
     const double l = b[10 + lane];
     x = ax + (bx - ax) * u;
     y = ay + (by - ay) * u;
-    const double tx = (bx - ax) / l, ty = (by - ay) / l;
+    tx = (bx - ax) / l;
+    ty = (by - ay) / l;
+  }
+  // position and velocity of a car at (lane, w, u) moving at v
+  __host__ __device__ void car(int lane, int w, double u, double v, double &x, double &y,
+                               double &vx, double &vy) const {
+    double tx, ty;
+    pose(lane, w, u, x, y, tx, ty);
     vx = v * tx;
     vy = v * ty;
   }
 };
+
+// Incident monitor state on the device (definitions: pp.h, pp_rollout_incidents).  Per-rollout
+// arrays are indexed by the absolute rollout; [x][R] arrays are row-major in x, so the ego warp's
+// lanes (consecutive rollouts) touch consecutive words.
+struct Monitor {
+  double2 *ring;        // [PP_INC_HISTORY][R]: driven point D_j in row j % PP_INC_HISTORY
+  double2 *ring_acc;    // [PP_INC_HISTORY][R]: A_j beside it (0 while undefined)
+  int64_t *pts;         // [R] index i of the ego's current point D_i
+  uint32_t *active;     // [R] bit per kind: its condition held at the last evaluation
+  int32_t *off_pts;     // [R] driven points off the lane centre in a row
+  int32_t *count;       // [PP_INC_KINDS][R]
+  int64_t *first_tick;  // [R]
+  int32_t *first_kind;  // [R]
+  double *dist, *clean, *best, *vmax, *amax, *jmax;  // [R]
+  const double *ego0_x, *ego0_y;  // [R] the ego before the tick (this tick's frame)
+  int64_t R;
+};
+
+// 0 = no overlap, 1 = overlap with the car ahead of the ego along its lane, 2 = any other
+__host__ __device__ inline int car_overlap(double cx, double cy, double tx, double ty, double ex,
+                                           double ey) {
+  const double dx = cx - ex, dy = cy - ey;
+  const double along = dx * tx + dy * ty;
+  const double across = dx * ty - dy * tx;
+  if (!(fabs(along) < PP_INC_CAR_HALF_LEN && fabs(across) < PP_INC_CAR_HALF_WIDTH)) return 0;
+  return along > 0 ? 1 : 2;
+}
+
+// An incident of `kind` counted at tick t (rare: read-modify-write of the record).
+// Out of line, with plain pointer arguments (a Monitor by reference would be copied to the stack).
+__device__ __forceinline__ void count_incident(int32_t *count, int64_t *first_tick, int32_t *first_kind,
+                                            int64_t R, int64_t r, int kind, int64_t t) {
+  count[kind * R + r] += 1;
+  if (kind == PP_INC_COLLISION_REAR) return;
+  const int64_t ft = first_tick[r];
+  if (ft < 0) {
+    first_tick[r] = t;
+    first_kind[r] = kind;
+  } else if (ft == t && kind < first_kind[r]) {
+    first_kind[r] = kind;
+  }
+}
+__device__ __forceinline__ void monitor_count(const Monitor &mo, int64_t r, int kind, int64_t t) {
+  count_incident(mo.count, mo.first_tick, mo.first_kind, mo.R, r, kind, t);
+}
+
+// a / 0.2, correctly rounded like the division it replaces: Markstein's sequence with
+// RN(1 / 0.2) = 5 (ppd::div_rcp) on the common path, so the generic division's subroutine, which
+// costs this kernel registers and spills, is only reached outside the safe range.  A zero keeps
+// its sign.
+__device__ __forceinline__ double div02(double a) {
+  const bool z = ppd::is_zero(a);
+  if (z || ppd::safe_mag(a)) {
+    const double q = ppd::div_rcp(a, 0.2, 5.0);
+    return z ? a : q;
+  }
+  return a / 0.2;
+}
+
+// The driven points of one tick, a lane per rollout of the ego warp: distance, clean distance,
+// Vbar / A / J, their maxima and the edges of over-speed / -acceleration / -jerk.  The rollout
+// drove k >= 1 points from (ox, oy) through row nx / ny of the new plan.  Returns the active bits
+// with the kinematic ones updated; clean_m is stored, the active bits are left to the caller.
+// A_i is kept beside D_i in the history, so J_i reads A_{i-50} instead of recomputing it from
+// four points (the same operations on the same values: the same bits, fewer registers).
+__device__ __forceinline__ unsigned monitor_points(const Monitor &mo, int64_t r, int k, double ox,
+                                                   double oy, const double *nx, const double *ny,
+                                                   unsigned act, int64_t t) {
+  constexpr int H = PP_INC_HISTORY;
+  constexpr unsigned kKin = (1u << PP_INC_OVER_SPEED) | (1u << PP_INC_OVER_ACC) | (1u << PP_INC_OVER_JERK);
+  const int64_t R = mo.R;
+  int64_t i = mo.pts[r];
+  int slot = (int)(i % H);
+  double px = ox, py = oy;
+  for (int j = 0; j < k; j++) {
+    const double x = nx[j], y = ny[j];
+    i++;
+    slot = slot + 1 == H ? 0 : slot + 1;
+    auto row = [&](int b) {  // history row of D_{i-b}, 10 <= b < H
+      const int s = slot - b;
+      return (int64_t)(s < 0 ? s + H : s) * R + r;
+    };
+    const double sx = x - px, sy = y - py;
+    const double step = sqrt(sx * sx + sy * sy);
+    mo.dist[r] += step;
+    double clean = mo.clean[r] + step;
+    if (clean > mo.best[r]) mo.best[r] = clean;
+    unsigned cond = 0;
+    double2 acc = make_double2(0.0, 0.0);
+    if (i >= 10) {
+      const double2 d10 = mo.ring[row(10)];
+      const double vx = div02(x - d10.x), vy = div02(y - d10.y);
+      const double v = sqrt(vx * vx + vy * vy);
+      if (v > mo.vmax[r]) mo.vmax[r] = v;
+      if (v > PP_INC_MAX_SPEED) cond |= 1u << PP_INC_OVER_SPEED;
+      if (i >= 20) {
+        const double2 d20 = mo.ring[row(20)];
+        const double wx = div02(d10.x - d20.x), wy = div02(d10.y - d20.y);
+        acc.x = div02(vx - wx);
+        acc.y = div02(vy - wy);
+        const double a = sqrt(acc.x * acc.x + acc.y * acc.y);
+        if (a > mo.amax[r]) mo.amax[r] = a;
+        if (a > PP_INC_MAX_ACC) cond |= 1u << PP_INC_OVER_ACC;
+        if (i >= H) {
+          const double2 a50 = mo.ring_acc[row(50)];
+          const double jx = (acc.x - a50.x) / 1.0, jy = (acc.y - a50.y) / 1.0;
+          const double jn = sqrt(jx * jx + jy * jy);
+          if (jn > mo.jmax[r]) mo.jmax[r] = jn;
+          if (jn > PP_INC_MAX_JERK) cond |= 1u << PP_INC_OVER_JERK;
+        }
+      }
+    }
+    mo.ring[(int64_t)slot * R + r] = make_double2(x, y);
+    mo.ring_acc[(int64_t)slot * R + r] = acc;
+    const unsigned rise = cond & ~act;
+    act = (act & ~kKin) | cond;
+    if (rise) {
+      for (int kind = PP_INC_OVER_SPEED; kind <= PP_INC_OVER_JERK; kind++)
+        if ((rise >> kind) & 1u) monitor_count(mo, r, kind, t);
+      clean = 0;
+    }
+    mo.clean[r] = clean;
+    px = x;
+    py = y;
+  }
+  mo.pts[r] = i;
+  return act;
+}
+
+// The lateral position of P, a lane per rollout of a whole warp (the lane matching votes across
+// it): the reference waypoint from the plan's ref_wp +- 3, then Map::lane_matching.  Keeps the
+// off-centre count of a rollout that drove k >= 1 points and returns the out-of-lane / off-road
+// condition bits (0 when it drove none).
+__device__ __forceinline__ unsigned monitor_lateral(const Track &trk, const Monitor &mo, int64_t r,
+                                                    int k, double px, double py, int ref_wp) {
+  const ppd::MapView mv{trk.t, trk.n, trk.n < PPD_PAD ? trk.n : PPD_PAD};
+  int closest = ref_wp - 3;
+  {
+    const double *w0 = ppd::row(mv, closest);
+    double bd = (w0[0] - px) * (w0[0] - px) + (w0[1] - py) * (w0[1] - py);
+    for (int w = ref_wp - 2; w <= ref_wp + 3; w++) {
+      const double *rw = ppd::row(mv, w);
+      const double d = (rw[0] - px) * (rw[0] - px) + (rw[1] - py) * (rw[1] - py);
+      if (d < bd) {
+        closest = w;
+        bd = d;
+      }
+    }
+  }
+  ppd::RefState rs;
+  ppd::finish_reference(mv, px, py, closest, rs);
+  const ppd::Match mt = ppd::lane_match(mv, rs, px, py);
+  if (k <= 0) return 0;
+  const bool off_centre = !mt.ok || fabs(mt.d - ppd::lane_center_offset(mt.lane)) > PP_INC_LANE_TOL;
+  int off = mo.off_pts[r];
+  if (!off_centre) {
+    off = 0;
+  } else if (off < (1 << 30)) {
+    off += k;
+  }
+  mo.off_pts[r] = off;
+  unsigned cond = 0;
+  if (off > PP_INC_OUT_POINTS) cond |= 1u << PP_INC_OUT_OF_LANE;
+  if (!mt.ok || mt.d < PP_INC_ROAD_MIN_D || mt.d > PP_INC_ROAD_MAX_D) cond |= 1u << PP_INC_OFF_ROAD;
+  return cond;
+}
 
 // Simulator state on the device (per rollout unless noted).  The unconsumed points of the last
 // plan are not copied anywhere: they stay in the plan buffer and `path_off` says where they start.
@@ -192,25 +372,41 @@ static_assert(kB >= 7 * 32 && kR == 32, "k_sim_frames: a warp per scalar field, 
 // which add it up as they write the points (plan_batch_scratch, xsum_add): re-reading 800 bytes
 // per rollout for it was two thirds of this kernel's traffic.  For the single-kernel paths of
 // small jobs the block takes it here, over its rollouts' rows (one contiguous run).
+//
+// The incident monitor (pp.h) rides along without a launch of its own.  Before the barrier the
+// ego warp walks the driven points, warp 1 matches the lane of each rollout's last point (in
+// parallel: it is the longest dependent chain of the monitor), and the car-slot threads test each
+// car against the old and the new ego, OR-ing a bit per rollout into shared memory.  After the
+// barrier the ego warp only merges those words into the edge bits (an incident is rare).
 __global__ void __launch_bounds__(kB)
 k_sim_advance(Track trk, int64_t lo, int64_t n, int c, uint64_t seed, int64_t first, int consume_k,
-              SimState st, pp_plans pl, unsigned long long *stats_sum, int do_xsum) {
+              SimState st, pp_plans pl, unsigned long long *stats_sum, int do_xsum, Monitor mo) {
+  __shared__ unsigned s_coll[kR];  // per rollout: bit 0 a front, bit 1 a rear collision began
+  __shared__ unsigned s_lat[kR];   // per rollout: out-of-lane / off-road condition bits
   const int64_t r0 = lo + (int64_t)blockIdx.x * kR;
   int64_t r_end = r0 + kR;
   if (r_end > lo + n) r_end = lo + n;
   const int nr = (int)(r_end - r0);
+  unsigned act = 0, act0 = 0;  // the ego warp's edge bits of its rollout, before and after
+  int64_t tick = 0;
+  bool drove = false;
   if (threadIdx.x < 32) {
+    s_coll[threadIdx.x] = 0;
+    asm volatile("bar.arrive 1, %0;" ::"n"(kB - 32) : "memory");  // the car-slot threads may OR now
     // ---- the ego consumes k points of the new trajectory (one lane per rollout)
     const int ln = threadIdx.x;
     const bool live = ln < nr;
     const int64_t r = r0 + (live ? ln : 0);
     const int np = live ? pl.n_points[r] : 0;
+    const int k = live ? (consume_k < np ? consume_k : np) : 0;
+    const double ox = st.ego_x[r], oy = st.ego_y[r];
+    tick = st.ticks[r];
+    act0 = act = mo.active[r];
+    drove = k > 0;
     int tl = -1, el = -1;
     uint32_t fl = 0;
     if (live) {
-      const int k = consume_k < np ? consume_k : np;
       if (k > 0) {
-        const double ox = st.ego_x[r], oy = st.ego_y[r];
         const double qx = pl.next_x[r * PP_PATH_LEN + k - 1], qy = pl.next_y[r * PP_PATH_LEN + k - 1];
         const double d = sqrt((qx - ox) * (qx - ox) + (qy - oy) * (qy - oy));
         st.ego_x[r] = qx;
@@ -224,6 +420,9 @@ k_sim_advance(Track trk, int64_t lo, int64_t n, int c, uint64_t seed, int64_t fi
       st.target_lane[r] = tl;
       fl = pl.flags[r];
     }
+    if (k > 0)
+      act = monitor_points(mo, r, k, ox, oy, pl.next_x + r * PP_PATH_LEN, pl.next_y + r * PP_PATH_LEN,
+                           act0, tick);
     // counters: lane i ends up holding entry i of the statistics vector
     const unsigned full = 0xffffffffu;
     unsigned long long mine = 0;
@@ -250,9 +449,20 @@ k_sim_advance(Track trk, int64_t lo, int64_t n, int c, uint64_t seed, int64_t fi
       if (ln == PP_STAT_FLAG0 + b) mine = a;
     }
     if (ln < PP_STATS_LEN && ln != PP_STAT_XSUM && mine) atomicAdd(&stats_sum[ln], mine);
+  } else if (threadIdx.x < 64) {
+    // ---- lateral position of the ego after its k points (one lane per rollout)
+    const int ln = threadIdx.x - 32;
+    const bool live = ln < nr;
+    const int64_t r = r0 + (live ? ln : 0);
+    const int np = pl.n_points[r];
+    const int k = live ? (consume_k < np ? consume_k : np) : 0;
+    const double px = k > 0 ? pl.next_x[r * PP_PATH_LEN + k - 1] : mo.ego0_x[r];
+    const double py = k > 0 ? pl.next_y[r * PP_PATH_LEN + k - 1] : mo.ego0_y[r];
+    s_lat[ln] = monitor_lateral(trk, mo, r, k, px, py, pl.ref_wp[r]);
   } else {
+    asm volatile("bar.sync 1, %0;" ::"n"(kB - 32) : "memory");  // s_coll is cleared
     // ---- traffic (one thread per car slot; they read the rollout's tick before it is counted)
-    for (int64_t q = r0 * c + (threadIdx.x - 32); q < r_end * c; q += kB - 32) {
+    for (int64_t q = r0 * c + (threadIdx.x - 64); q < r_end * c; q += kB - 64) {
       const int64_t r = q / c;
       const int j = (int)(q - r * c);
       const int np = pl.n_points[r];
@@ -260,6 +470,12 @@ k_sim_advance(Track trk, int64_t lo, int64_t n, int c, uint64_t seed, int64_t fi
       const double dt = kTick * (k > 0 ? k : 1);
       int lane = st.car_lane[q], w = st.car_wp[q];
       double u = st.car_ratio[q], v = st.car_speed[q];
+      int was;  // overlap of the car before its advance with the ego before the tick
+      {
+        double cx, cy, tx, ty;
+        trk.pose(lane, w, u, cx, cy, tx, ty);
+        was = car_overlap(cx, cy, tx, ty, mo.ego0_x[r], mo.ego0_y[r]);
+      }
       const int m_lane = pl.car_lane[q];
       const double m_s = pl.car_s[q];
       if (m_lane < 0 || m_s < -100.0 || m_s > 300.0) {  // respawn
@@ -286,6 +502,14 @@ k_sim_advance(Track trk, int64_t lo, int64_t n, int c, uint64_t seed, int64_t fi
       st.car_wp[q] = w;
       st.car_ratio[q] = u;
       st.car_speed[q] = v;
+      {  // the same pair now: the car advanced, the ego at its last driven point
+        double cx, cy, tx, ty;
+        trk.pose(lane, w, u, cx, cy, tx, ty);
+        const double ex = k > 0 ? pl.next_x[r * PP_PATH_LEN + k - 1] : mo.ego0_x[r];
+        const double ey = k > 0 ? pl.next_y[r * PP_PATH_LEN + k - 1] : mo.ego0_y[r];
+        const int now = car_overlap(cx, cy, tx, ty, ex, ey);
+        if (now && !was) atomicOr(&s_coll[r - r0], (unsigned)now);
+      }
     }
   }
   if (do_xsum) {  // ---- checksum of the block's rows, unless the planning kernels added it
@@ -304,7 +528,42 @@ k_sim_advance(Track trk, int64_t lo, int64_t n, int c, uint64_t seed, int64_t fi
     if ((threadIdx.x & 31) == 0 && v) atomicAdd(&stats_sum[PP_STAT_XSUM], v);
   }
   __syncthreads();
-  if (threadIdx.x < nr) st.ticks[r0 + threadIdx.x] += 1;
+  if (threadIdx.x < nr) {  // the ego warp: lateral edges, then collisions
+    const int64_t r = r0 + threadIdx.x;
+    constexpr unsigned kLat = (1u << PP_INC_OUT_OF_LANE) | (1u << PP_INC_OFF_ROAD);
+    const unsigned cb = s_coll[threadIdx.x];
+    if (drove) act = (act & ~kLat) | s_lat[threadIdx.x];
+    const unsigned rise = act & ~act0 & kLat;
+    if (act != act0) mo.active[r] = act;
+    if (rise | cb) {
+      for (int kind = PP_INC_OUT_OF_LANE; kind <= PP_INC_OFF_ROAD; kind++)
+        if ((rise >> kind) & 1u) monitor_count(mo, r, kind, tick);
+      if (cb & 1u) monitor_count(mo, r, PP_INC_COLLISION_FRONT, tick);
+      if (cb & 2u) monitor_count(mo, r, PP_INC_COLLISION_REAR, tick);
+      if (rise | (cb & 1u)) mo.clean[r] = 0;
+    }
+    st.ticks[r] += 1;
+  }
+}
+
+// pp_rollouts_incident_totals: counts per kind, rollouts with an incident, millimetres driven.
+__global__ void __launch_bounds__(kB) k_incident_totals(Monitor mo, unsigned long long *tot) {
+  unsigned long long acc[PP_INC_TOTALS_LEN];
+#pragma unroll
+  for (int e = 0; e < PP_INC_TOTALS_LEN; e++) acc[e] = 0;
+  for (int64_t r = (int64_t)blockIdx.x * kB + threadIdx.x; r < mo.R; r += (int64_t)gridDim.x * kB) {
+#pragma unroll
+    for (int e = 0; e < PP_INC_KINDS; e++) acc[e] += (unsigned long long)mo.count[e * mo.R + r];
+    acc[PP_INC_TOTAL_ROLLOUTS] += mo.first_tick[r] >= 0 ? 1u : 0u;
+    acc[PP_INC_TOTAL_MM] += (unsigned long long)llround(mo.dist[r] * 1000.0);
+  }
+#pragma unroll
+  for (int e = 0; e < PP_INC_TOTALS_LEN; e++) {
+    unsigned long long v = acc[e];
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) v += __shfl_down_sync(0xffffffffu, v, o);
+    if ((threadIdx.x & 31) == 0 && v) atomicAdd(&tot[e], v);
+  }
 }
 static_assert(PP_STATS_LEN <= 32, "k_sim_advance: a lane per statistics entry");
 
@@ -361,6 +620,12 @@ extern "C" int pp_rollouts_create(const pp_map *map, int64_t n, int32_t c, uint6
                p_cl = take(NC * 4), p_cw = take(NC * 4);
   const size_t o_ss = take(PP_STATS_LEN * 8);
   const size_t o_tk = take(N * 8);
+  // incident monitor
+  const size_t m_ring = take(N * PP_INC_HISTORY * 16), m_racc = take(N * PP_INC_HISTORY * 16), m_pts = take(N * 8), m_ft = take(N * 8),
+               m_act = take(N * 4), m_off = take(N * 4), m_cnt = take(N * PP_INC_KINDS * 4),
+               m_fk = take(N * 4);
+  size_t m_d[6];
+  for (int i = 0; i < 6; i++) m_d[i] = take(N * 8);
   cudaError_t e = cudaMalloc((void **)&r->buf, off);
   if (e != cudaSuccess) {
     delete r;
@@ -422,6 +687,17 @@ extern "C" int pp_rollouts_create(const pp_map *map, int64_t n, int32_t c, uint6
   p.car_next_wp = (int32_t *)(b + p_cw);
   r->stats_sum = (int64_t *)(b + o_ss);
   r->tick_dev = (int64_t *)(b + o_tk);
+  r->inc_ring = (double2 *)(b + m_ring);
+  r->inc_ring_acc = (double2 *)(b + m_racc);
+  r->inc_pts = (int64_t *)(b + m_pts);
+  r->inc_first_tick = (int64_t *)(b + m_ft);
+  r->inc_active = (uint32_t *)(b + m_act);
+  r->inc_off = (int32_t *)(b + m_off);
+  r->inc_count = (int32_t *)(b + m_cnt);
+  r->inc_first_kind = (int32_t *)(b + m_fk);
+  for (int i = 0; i < 6; i++) r->inc_d[i] = (double *)(b + m_d[i]);
+  cudaMemset(r->inc_first_tick, 0xff, N * 8);  // -1: no incident yet
+  cudaMemset(r->inc_first_kind, 0xff, N * 4);
 
   // ---- initial state on the host: a pure function of (seed, first + r)
   std::vector<double> ex(N), ey(N), yaw(N), mph(N), cr(NC), cs(NC);
@@ -466,6 +742,14 @@ extern "C" int pp_rollouts_create(const pp_map *map, int64_t n, int32_t c, uint6
   up(r->ego_yaw, yaw.data(), N * 8);
   up(r->ego_mph, mph.data(), N * 8);
   up(r->target_lane, tl.data(), N * 4);
+  {  // D_0, the initial pose, in row 0 of the monitor's history
+    std::vector<double> d0(2 * N);
+    for (size_t i = 0; i < N; i++) {
+      d0[2 * i] = ex[i];
+      d0[2 * i + 1] = ey[i];
+    }
+    up(r->inc_ring, d0.data(), N * 16);
+  }
   if (c > 0) {
     up(r->car_lane, cl.data(), NC * 4);
     up(r->car_wp, cw.data(), NC * 4);
@@ -562,12 +846,15 @@ int issue_tick(pp_rollouts *r, const pp_config *cfg, int32_t consume_k, cudaStre
       if (need && cudaMalloc((void **)&r->scratch[g], need) != cudaSuccess)
         return cuda_fail("cudaMalloc(rollout scratch)", cudaGetLastError());
     }
+    const Monitor mo{r->inc_ring, r->inc_ring_acc, r->inc_pts, r->inc_active, r->inc_off, r->inc_count,
+                     r->inc_first_tick, r->inc_first_kind, r->inc_d[0], r->inc_d[1], r->inc_d[2],
+                     r->inc_d[3], r->inc_d[4], r->inc_d[5], r->fr.ego_x, r->fr.ego_y, r->n};
     const bool plan_sums = ppi::plan_adds_checksum(cnt);
     int rc = ppi::plan_batch_scratch(r->map, cfg, &fr, &pl, cnt, gs, r->scratch[g], nullptr,
                                      (unsigned long long *)r->stats_sum + PP_STAT_XSUM);
     if (rc != PP_OK) return rc;
     k_sim_advance<<<grid, kB, 0, gs>>>(trk, lo, cnt, r->c, r->seed, r->first, consume_k, sst, r->pl,
-                                       (unsigned long long *)r->stats_sum, plan_sums ? 0 : 1);
+                                       (unsigned long long *)r->stats_sum, plan_sums ? 0 : 1, mo);
     ppi::count_launch(2);
   }
   r->launches_per_tick = pp_launch_count() - launches0;
@@ -745,5 +1032,51 @@ extern "C" int pp_rollouts_stats(const pp_rollouts *r, int64_t *stats_dev, void 
   cudaError_t e = cudaMemcpyAsync(stats_dev, r->stats_sum, PP_STATS_LEN * sizeof(int64_t),
                                   cudaMemcpyDeviceToDevice, (cudaStream_t)cuda_stream);
   if (e != cudaSuccess) return cuda_fail("pp_rollouts_stats", e);
+  return PP_OK;
+}
+
+extern "C" int pp_rollouts_get_incidents(const pp_rollouts *r, pp_rollout_incidents *h) {
+  if (!r || !h) return PP_E_ARG;
+  cudaError_t e = cudaDeviceSynchronize();
+  if (e != cudaSuccess) return cuda_fail("pp_rollouts_get_incidents", e);
+  const size_t N = (size_t)r->n;
+  bool ok = true;
+  auto dn = [&](void *dst, const void *src, size_t bytes) {
+    if (dst && cudaMemcpy(dst, src, bytes, cudaMemcpyDeviceToHost) != cudaSuccess) ok = false;
+  };
+  if (h->count) {  // [kind][R] on the device, [R][kind] for the caller
+    std::vector<int32_t> cnt(N * PP_INC_KINDS);
+    dn(cnt.data(), r->inc_count, N * PP_INC_KINDS * 4);
+    for (size_t i = 0; i < N; i++)
+      for (int k = 0; k < PP_INC_KINDS; k++) h->count[i * PP_INC_KINDS + k] = cnt[k * N + i];
+  }
+  dn(h->first_tick, r->inc_first_tick, N * 8);
+  dn(h->first_kind, r->inc_first_kind, N * 4);
+  double *const outs[6] = {h->distance_m, h->clean_m, h->best_clean_m, h->max_speed, h->max_acc,
+                           h->max_jerk};
+  for (int i = 0; i < 6; i++) dn(outs[i], r->inc_d[i], N * 8);
+  if (!ok) return cuda_fail("pp_rollouts_get_incidents copy", cudaGetLastError());
+  return PP_OK;
+}
+
+extern "C" int pp_rollouts_incident_totals(const pp_rollouts *r, int64_t *totals_dev,
+                                           void *cuda_stream) {
+  if (!r || !totals_dev) return PP_E_ARG;
+  {
+    const int rc = ppi::check_map_device(r->map, "pp_rollouts_incident_totals");
+    if (rc != PP_OK) return rc;
+  }
+  cudaStream_t st = (cudaStream_t)cuda_stream;
+  cudaError_t e = cudaMemsetAsync(totals_dev, 0, PP_INC_TOTALS_LEN * sizeof(int64_t), st);
+  if (e != cudaSuccess) return cuda_fail("pp_rollouts_incident_totals", e);
+  const Monitor mo{r->inc_ring, r->inc_ring_acc, r->inc_pts, r->inc_active, r->inc_off, r->inc_count,
+                   r->inc_first_tick, r->inc_first_kind, r->inc_d[0], r->inc_d[1], r->inc_d[2],
+                   r->inc_d[3], r->inc_d[4], r->inc_d[5], r->fr.ego_x, r->fr.ego_y, r->n};
+  const int64_t blocks = (r->n + kB - 1) / kB;
+  k_incident_totals<<<(int)(blocks < 1184 ? blocks : 1184), kB, 0, st>>>(
+      mo, (unsigned long long *)totals_dev);
+  ppi::count_launch(1);
+  e = cudaGetLastError();
+  if (e != cudaSuccess) return cuda_fail("k_incident_totals", e);
   return PP_OK;
 }

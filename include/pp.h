@@ -559,6 +559,85 @@ int pp_rollouts_get_state(const pp_rollouts *r, pp_rollout_state *host_out);
  * (device, int64).  The multi-GPU job all-reduces this. */
 int pp_rollouts_stats(const pp_rollouts *r, int64_t *stats_dev, void *cuda_stream);
 
+/* ---- incident monitor of the rollouts ----------------------------------------------------
+ * The reference was judged by the simulator's "distance without incident" and its acceleration
+ * and jerk readouts.  The monitor is the simulator model's own referee, part of the model above,
+ * evaluated on the device inside the simulator step; it changes nothing the model computes.
+ * Its thresholds are fixed here and do not depend on pp_config (the planner's tunables must not
+ * move the referee).  Every operation is IEEE double + - * / and sqrt, left to right, per
+ * component, without fused multiply-add, so the CPU restatement is bit-identical.
+ *
+ * Driven points.  D_0 is the ego's initial pose.  A tick that consumes k points drives through
+ * points 0..k-1 of its new plan, which become D_{i+1} .. D_{i+k}; each point is 0.02 s after the
+ * one before.  A tick with an empty plan drives no point.
+ * Kinematics.  The simulator's own formula is not published; this model takes the windows of
+ * the Udacity project description (acceleration = change of the average velocity over 0.2 s,
+ * jerk over 1 s):
+ *   Vbar_i = (D_i - D_{i-10}) / 0.2      defined for i >= 10
+ *   A_i    = (Vbar_i - Vbar_{i-10}) / 0.2 defined for i >= 20
+ *   J_i    = (A_i - A_{i-50}) / 1.0      defined for i >= 70
+ * and their norms sqrt(x*x + y*y).  over-speed: |Vbar_i| > PP_INC_MAX_SPEED, over-acceleration:
+ * |A_i| > PP_INC_MAX_ACC, over-jerk: |J_i| > PP_INC_MAX_JERK, each evaluated at every driven point.
+ * Lateral position, once per tick at the tick's last driven point P: the reference waypoint of P
+ * is the closest of the rows ref_wp-3 .. ref_wp+3 (ref_wp of this tick's plan; strict <, lowest
+ * row wins), completed as Map::init_reference_waypoint does, and (ok, lane, d) is
+ * Map::lane_matching(P) from that reference.  The ego is off centre when !ok or
+ * |d - 4 (lane + 0.5)| > PP_INC_LANE_TOL; an off-centre count of driven points grows by k per
+ * off-centre tick and returns to 0 otherwise.  out-of-lane: that count > PP_INC_OUT_POINTS
+ * (3.0 s).  off-road: !ok, d < PP_INC_ROAD_MIN_D or d > PP_INC_ROAD_MAX_D.
+ * Collisions, at the end of the tick: the ego at P (its position before the tick when no point
+ * was driven) against every car at its advanced (lane, wp, ratio), positioned as the frames
+ * position it; t = the car's lane tangent, delta = car - ego.  A pair overlaps when
+ * |delta.t| < PP_INC_CAR_HALF_LEN and |delta x t| < PP_INC_CAR_HALF_WIDTH.  A collision is an
+ * overlap that BEGINS: the pair did not overlap at the previous positions (the ego of this tick's
+ * frame, the car before its advance), so a car placed on top of the ego never counts.
+ * collision_front: delta.t > 0, the ego drove into the car.  collision_rear: any other; the
+ * traffic of this model never brakes, so a rear collision is the traffic model's doing: it is
+ * counted but is NOT an incident for clean_m, first_tick or the incident-free share.
+ * Counting.  Every kind is edge-triggered: counted when its condition becomes true (an active
+ * bit per kind per rollout), not while it stays true; a collision counts once per tick and side
+ * in which some overlap begins.  distance_m = sum |D_i - D_{i-1}| in driving order; clean_m =
+ * distance since the last incident (the simulator's "distance without incident"): the step is
+ * added, best_clean_m = max(best_clean_m, clean_m), then any incident at that point resets
+ * clean_m to 0.  Order within a tick: the driven points in order, then the lateral checks, then
+ * the collisions.  first_tick is the rollout's tick counter (0 = its first tick) of the first
+ * incident, first_kind the smallest kind counted in that tick. */
+#define PP_INC_COLLISION_FRONT 0
+#define PP_INC_COLLISION_REAR 1
+#define PP_INC_OVER_SPEED 2
+#define PP_INC_OVER_ACC 3
+#define PP_INC_OVER_JERK 4
+#define PP_INC_OUT_OF_LANE 5
+#define PP_INC_OFF_ROAD 6
+#define PP_INC_KINDS 7
+#define PP_INC_MAX_SPEED 22.352    /* m/s = 50 mph */
+#define PP_INC_MAX_ACC 10.0        /* m/s^2 */
+#define PP_INC_MAX_JERK 10.0       /* m/s^3 */
+#define PP_INC_LANE_TOL 1.0        /* m from the lane centre */
+#define PP_INC_OUT_POINTS 150      /* driven points off centre (3.0 s) before out-of-lane */
+#define PP_INC_ROAD_MIN_D 1.0      /* m */
+#define PP_INC_ROAD_MAX_D 11.0     /* m */
+#define PP_INC_CAR_HALF_LEN 4.5    /* m along the car's lane */
+#define PP_INC_CAR_HALF_WIDTH 2.0  /* m across it */
+#define PP_INC_HISTORY 70          /* driven points J_i reaches back */
+typedef struct pp_rollout_incidents { /* host arrays, R rollouts; any pointer may be NULL */
+  int32_t *count;                     /* [R][PP_INC_KINDS] */
+  int64_t *first_tick;                /* [R] tick of the first incident (not rear), -1 none */
+  int32_t *first_kind;                /* [R] its kind, -1 none */
+  double *distance_m, *clean_m, *best_clean_m; /* [R] */
+  double *max_speed, *max_acc, *max_jerk;      /* [R] maxima of the defined |Vbar|, |A|, |J| (0 before) */
+} pp_rollout_incidents;
+/* Copy the incident record out (synchronises the device). */
+int pp_rollouts_get_incidents(const pp_rollouts *r, pp_rollout_incidents *host_out);
+/* totals_dev[PP_INC_KINDS + 2] (device, int64, overwritten; asynchronous on cuda_stream): the
+ * counts per kind summed over the rollouts, then the number of rollouts with at least one incident
+ * (first_tick >= 0), then the driven distance in millimetres, sum of llround(distance_m * 1000).
+ * All int64, so a multi-GPU job all-reduces it with ncclSum to the same bits on any GPU count. */
+#define PP_INC_TOTAL_ROLLOUTS PP_INC_KINDS
+#define PP_INC_TOTAL_MM (PP_INC_KINDS + 1)
+#define PP_INC_TOTALS_LEN (PP_INC_KINDS + 2)
+int pp_rollouts_incident_totals(const pp_rollouts *r, int64_t *totals_dev, void *cuda_stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -781,6 +781,32 @@ class Rollouts {
     e.tick = st.tick;
     return e;
   }
+  // The incident monitor's record (pp.h, pp_rollout_incidents); count is [n][PP_INC_KINDS].
+  struct Incidents {
+    std::vector<int32_t> count, first_kind;
+    std::vector<int64_t> first_tick;
+    std::vector<double> distance_m, clean_m, best_clean_m, max_speed, max_acc, max_jerk;
+  };
+  Incidents incidents() const {
+    Incidents r;
+    r.count.resize((size_t)n_ * PP_INC_KINDS);
+    r.first_kind.resize(n_);
+    r.first_tick.resize(n_);
+    for (auto *v : {&r.distance_m, &r.clean_m, &r.best_clean_m, &r.max_speed, &r.max_acc, &r.max_jerk})
+      v->resize(n_);
+    pp_rollout_incidents h;
+    h.count = r.count.data();
+    h.first_tick = r.first_tick.data();
+    h.first_kind = r.first_kind.data();
+    h.distance_m = r.distance_m.data();
+    h.clean_m = r.clean_m.data();
+    h.best_clean_m = r.best_clean_m.data();
+    h.max_speed = r.max_speed.data();
+    h.max_acc = r.max_acc.data();
+    h.max_jerk = r.max_jerk.data();
+    check(pp_rollouts_get_incidents(h_, &h), "pp_rollouts_get_incidents");
+    return r;
+  }
 
  private:
   pp_rollouts *h_ = nullptr;
