@@ -45,7 +45,8 @@ EXPORTS = [
     "pp_dev_set", "pp_stream_create", "pp_stream_sync", "pp_stream_destroy",
     "pp_rollouts_create", "pp_rollouts_destroy", "pp_rollouts_run", "pp_rollouts_last",
     "pp_rollouts_get_state", "pp_rollouts_stats", "pp_rollouts_set_lean", "pp_rollouts_set_groups",
-    "pp_rollouts_get_incidents", "pp_rollouts_incident_totals", "pp_sweep_batch",
+    "pp_rollouts_get_incidents", "pp_rollouts_incident_totals", "pp_rollouts_set_traffic",
+    "pp_rollouts_get_traffic", "pp_sweep_batch",
     "pp_set_pipes", "pp_plan_stats_batch", "pp_synth_frames_dev", "pp_fstats_batch",
     "pp_comm_unique_id", "pp_comm_init_rank", "pp_comm_init_all", "pp_comm_destroy",
     "pp_comm_group_begin", "pp_comm_group_end", "pp_stats_reduce",
@@ -485,6 +486,24 @@ class Rollouts:
                for name, dt, kind in abi.INC_FIELDS}
         s = abi.RolloutIncidents(*[a.ctypes.data for a in out.values()])
         _check(lib.pp_rollouts_get_incidents(self._h, C.byref(s)), "pp_rollouts_get_incidents")
+        return out
+
+    def set_traffic(self, model):
+        """Select the traffic model before the first tick: abi.TRAFFIC_CONSTANT (default) or
+        abi.TRAFFIC_IDM (car following, include/pp.h), or their names "constant" / "idm"."""
+        if isinstance(model, str):
+            model = abi.TRAFFIC_MODELS[model]
+        _check(lib.pp_rollouts_set_traffic(self._h, C.c_int(model)), "pp_rollouts_set_traffic")
+
+    def traffic(self) -> dict:
+        """The IDM traffic state (only under abi.TRAFFIC_IDM) as numpy arrays: car_v0, car_acc
+        [n][n_cars], and the ego's lane state the next tick reads, ego_lanes [n] (bit L: the ego
+        leads lane L) and ego_s [n][3]."""
+        inner = {"cars": (self.n_cars,), 0: (), "lanes": (3,)}
+        out = {name: np.zeros((self.n,) + inner[kind], dtype=dt)
+               for name, dt, kind in abi.TRAFFIC_FIELDS}
+        s = abi.RolloutTraffic(*[a.ctypes.data for a in out.values()])
+        _check(lib.pp_rollouts_get_traffic(self._h, C.byref(s)), "pp_rollouts_get_traffic")
         return out
 
     def incident_totals(self, stream=None):

@@ -172,6 +172,27 @@ class RolloutIncidents(C.Structure):
     _fields_ = [(n, _dp) for n, _, _ in INC_FIELDS]
 
 
+# traffic models of the rollouts (pp_rollouts_set_traffic) and the IDM parameters (PP_TRF_*)
+TRAFFIC_CONSTANT = 0
+TRAFFIC_IDM = 1
+TRAFFIC_MODELS = {"constant": TRAFFIC_CONSTANT, "idm": TRAFFIC_IDM}
+TRF_ACC = 1.5
+TRF_DEC = 3.0
+TRF_MAX_DEC = 9.0
+TRF_HEADWAY = 1.2
+TRF_MIN_GAP = 2.0
+TRF_GAP_FLOOR = 0.1
+TRF_EGO_CORRIDOR = 3.0
+TRAFFIC_FIELDS = [  # (name, dtype, inner) ; inner: 'cars', 0 scalar, 'lanes'
+    ("car_v0", np.float64, "cars"), ("car_acc", np.float64, "cars"),
+    ("ego_lanes", np.int32, 0), ("ego_s", np.float64, "lanes"),
+]
+
+
+class RolloutTraffic(C.Structure):
+    _fields_ = [(n, _dp) for n, _, _ in TRAFFIC_FIELDS]
+
+
 def default_config() -> Config:
     """The literals of reference src/main.cpp:30,39-49 (also what
     pp_config_default writes; tests check the two agree)."""

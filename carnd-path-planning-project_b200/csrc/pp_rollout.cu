@@ -53,6 +53,12 @@ struct pp_rollouts {
   uint32_t *inc_active;
   int32_t *inc_off, *inc_count, *inc_first_kind;
   double *inc_d[6];  // distance_m, clean_m, best_clean_m, max_speed, max_acc, max_jerk
+  // traffic model (pp.h, pp_rollouts_set_traffic); the IDM state has an allocation of its own,
+  // made only when that model is selected
+  int traffic = PP_TRAFFIC_CONSTANT;
+  char *trf_buf = nullptr;
+  double *trf_v0 = nullptr, *trf_acc = nullptr, *trf_cum = nullptr, *trf_ego_s = nullptr;
+  int32_t *trf_ego_lanes = nullptr;
 };
 
 namespace {
@@ -150,6 +156,65 @@ struct Monitor {
   const double *ego0_x, *ego0_y;  // [R] the ego before the tick (this tick's frame)
   int64_t R;
 };
+
+// State of the IDM traffic model on the device (pp.h, PP_TRAFFIC_IDM).  The ego's lane state is
+// double-buffered by the rollout's tick parity: tick t reads copy t % 2 (its pre-tick state) and
+// writes copy (t + 1) % 2.
+struct Traffic {
+  double *v0, *acc;          // [R][C] desired speed, last applied acceleration
+  const double *cum;         // [3][n + 1] cum(L, w); Lambda_L = cum[L][n]
+  int32_t *ego_lanes;        // [2][R] bit L: the ego leads lane L
+  double *ego_s;             // [2][3][R] S_ego per lane
+  const double *ego0_mph;    // [R] the ego's speed before the tick (this tick's frame)
+  int64_t R;
+};
+
+// The ego's lane state from its reference and lane match (pp.h, PP_TRAFFIC_IDM).
+__device__ __forceinline__ void traffic_ego_state(const Track &trk, const Traffic &tf, int64_t r,
+                                                  int buf, const ppd::RefState &rs,
+                                                  const ppd::Match &mt) {
+  int w = rs.wp % trk.n;
+  if (w < 0) w += trk.n;
+  int lanes = 0;
+#pragma unroll
+  for (int L = 0; L < 3; L++) {
+    if (mt.ok && fabs(mt.d - (4.0 * L + 2.0)) < PP_TRF_EGO_CORRIDOR) lanes |= 1 << L;
+    tf.ego_s[((int64_t)buf * 3 + L) * tf.R + r] = tf.cum[L * (trk.n + 1) + w] + rs.ratio[L] * trk.len(rs.wp, L);
+  }
+  tf.ego_lanes[buf * tf.R + r] = lanes;
+}
+
+// Reduce Delta = S_c - S_f into [0, lam) with at most one addition or subtraction.
+__host__ __device__ inline double traffic_delta(double sc, double sf, double lam) {
+  double d = sc - sf;
+  if (d < 0) {
+    d += lam;
+  } else if (d >= lam) {
+    d -= lam;
+  }
+  return d;
+}
+
+// The IDM acceleration of a car at speed v with desired speed v0 behind a leader Delta ahead at
+// speed vl (has_lead false: free road), clamped.
+__host__ __device__ inline double traffic_idm_acc(double v, double v0, bool has_lead, double delta,
+                                                  double vl) {
+  const double q = v / v0, q2 = q * q;
+  double inter = 0.0;
+  if (has_lead) {
+    double gap = delta - PP_INC_CAR_HALF_LEN;
+    if (gap < PP_TRF_GAP_FLOOR) gap = PP_TRF_GAP_FLOOR;
+    double dyn = v * PP_TRF_HEADWAY + v * (v - vl) / (2.0 * sqrt(PP_TRF_ACC * PP_TRF_DEC));
+    if (dyn < 0.0) dyn = 0.0;
+    const double s_star = PP_TRF_MIN_GAP + dyn;
+    const double z = s_star / gap;
+    inter = z * z;
+  }
+  double acc = PP_TRF_ACC * (1.0 - q2 * q2 - inter);
+  if (acc < -PP_TRF_MAX_DEC) acc = -PP_TRF_MAX_DEC;
+  if (acc > PP_TRF_ACC) acc = PP_TRF_ACC;
+  return acc;
+}
 
 // 0 = no overlap, 1 = overlap with the car ahead of the ego along its lane, 2 = any other
 __host__ __device__ inline int car_overlap(double cx, double cy, double tx, double ty, double ex,
@@ -265,9 +330,10 @@ __device__ __forceinline__ unsigned monitor_points(const Monitor &mo, int64_t r,
 // The lateral position of P, a lane per rollout of a whole warp (the lane matching votes across
 // it): the reference waypoint from the plan's ref_wp +- 3, then Map::lane_matching.  Keeps the
 // off-centre count of a rollout that drove k >= 1 points and returns the out-of-lane / off-road
-// condition bits (0 when it drove none).
+// condition bits (0 when it drove none).  The reference and the match are left in rs / mt.
 __device__ __forceinline__ unsigned monitor_lateral(const Track &trk, const Monitor &mo, int64_t r,
-                                                    int k, double px, double py, int ref_wp) {
+                                                    int k, double px, double py, int ref_wp,
+                                                    ppd::RefState &rs, ppd::Match &mt) {
   const ppd::MapView mv{trk.t, trk.n, trk.n < PPD_PAD ? trk.n : PPD_PAD};
   int closest = ref_wp - 3;
   {
@@ -282,9 +348,8 @@ __device__ __forceinline__ unsigned monitor_lateral(const Track &trk, const Moni
       }
     }
   }
-  ppd::RefState rs;
   ppd::finish_reference(mv, px, py, closest, rs);
-  const ppd::Match mt = ppd::lane_match(mv, rs, px, py);
+  mt = ppd::lane_match(mv, rs, px, py);
   if (k <= 0) return 0;
   const bool off_centre = !mt.ok || fabs(mt.d - ppd::lane_center_offset(mt.lane)) > PP_INC_LANE_TOL;
   int off = mo.off_pts[r];
@@ -378,9 +443,19 @@ static_assert(kB >= 7 * 32 && kR == 32, "k_sim_frames: a warp per scalar field, 
 // parallel: it is the longest dependent chain of the monitor), and the car-slot threads test each
 // car against the old and the new ego, OR-ing a bit per rollout into shared memory.  After the
 // barrier the ego warp only merges those words into the edge bits (an incident is rare).
+//
+// kTraffic selects the traffic model (pp.h); the constant-speed instantiation ignores `tf`.
+// Under PP_TRAFFIC_IDM the car-slot warps first stage the pre-tick (lane, S, v) of their
+// rollouts' cars in dynamic shared memory ([slot][rollout], so the lanes of a warp scanning
+// different rollouts read different banks and those of one rollout read the same word) and
+// meet at a barrier of their own, while warps 0 and 1 go on; warp 1 also stores the ego's lane
+// state for the next tick.
+template <int kTraffic>
 __global__ void __launch_bounds__(kB)
 k_sim_advance(Track trk, int64_t lo, int64_t n, int c, uint64_t seed, int64_t first, int consume_k,
-              SimState st, pp_plans pl, unsigned long long *stats_sum, int do_xsum, Monitor mo) {
+              SimState st, pp_plans pl, unsigned long long *stats_sum, int do_xsum, Monitor mo,
+              Traffic tf) {
+  constexpr bool kIdm = kTraffic == PP_TRAFFIC_IDM;
   __shared__ unsigned s_coll[kR];  // per rollout: bit 0 a front, bit 1 a rear collision began
   __shared__ unsigned s_lat[kR];   // per rollout: out-of-lane / off-road condition bits
   const int64_t r0 = lo + (int64_t)blockIdx.x * kR;
@@ -458,9 +533,58 @@ k_sim_advance(Track trk, int64_t lo, int64_t n, int c, uint64_t seed, int64_t fi
     const int k = live ? (consume_k < np ? consume_k : np) : 0;
     const double px = k > 0 ? pl.next_x[r * PP_PATH_LEN + k - 1] : mo.ego0_x[r];
     const double py = k > 0 ? pl.next_y[r * PP_PATH_LEN + k - 1] : mo.ego0_y[r];
-    s_lat[ln] = monitor_lateral(trk, mo, r, k, px, py, pl.ref_wp[r]);
+    ppd::RefState rs;
+    ppd::Match mt;
+    s_lat[ln] = monitor_lateral(trk, mo, r, k, px, py, pl.ref_wp[r], rs, mt);
+    if constexpr (kIdm) {
+      if (live) traffic_ego_state(trk, tf, r, (int)((st.ticks[r] + 1) & 1), rs, mt);
+    }
   } else {
     asm volatile("bar.sync 1, %0;" ::"n"(kB - 32) : "memory");  // s_coll is cleared
+    extern __shared__ double s_trf[];  // IDM: S [c][kR], v [c][kR], then lane [c][kR] (int)
+    double *const s_S = s_trf, *const s_v = s_trf + c * kR;
+    int *const s_ln = (int *)(s_trf + 2 * c * kR);
+    if constexpr (kIdm) {  // ---- stage the cars before the tick
+      for (int b = threadIdx.x - 64; b < nr * c; b += kB - 64) {  // b: car slot of the block
+        const int rr = b / c, j = b - rr * c, e = j * kR + rr;
+        const int64_t q = r0 * c + b;
+        const int lane = st.car_lane[q], w = st.car_wp[q];
+        s_S[e] = tf.cum[lane * (trk.n + 1) + w] + st.car_ratio[q] * trk.len(w, lane);
+        s_v[e] = st.car_speed[q];
+        s_ln[e] = lane;
+      }
+      asm volatile("bar.sync 2, %0;" ::"n"(kB - 64) : "memory");  // the car-slot warps only
+      // ---- every car's acceleration from its leader, stored to tf.acc for the advance below
+      // (a pass of its own: the scan's registers are free again when the advance runs)
+      for (int b = threadIdx.x - 64; b < nr * c; b += kB - 64) {
+        const int rr = b / c, j = b - rr * c;
+        const int64_t q = r0 * c + b, r = r0 + rr;
+        const int lane = s_ln[j * kR + rr];
+        const double sf = s_S[j * kR + rr];
+        const double lam = tf.cum[lane * (trk.n + 1) + trk.n], half = lam / 2;
+        bool has = false;
+        double best = 0.0, vl = 0.0;
+        for (int i = 0; i < c; i++) {
+          if (s_ln[i * kR + rr] != lane) continue;
+          const double d = traffic_delta(s_S[i * kR + rr], sf, lam);
+          if (((d > 0 && d < half) || (d == 0 && i > j)) && (!has || d < best)) {
+            has = true;
+            best = d;
+            vl = s_v[i * kR + rr];
+          }
+        }
+        const int par = (int)(st.ticks[r] & 1);
+        if ((tf.ego_lanes[par * tf.R + r] >> lane) & 1) {
+          const double d = traffic_delta(tf.ego_s[((int64_t)par * 3 + lane) * tf.R + r], sf, lam);
+          if (((d > 0 && d < half) || d == 0) && (!has || d < best)) {
+            has = true;
+            best = d;
+            vl = tf.ego0_mph[r] / 2.237;
+          }
+        }
+        tf.acc[q] = traffic_idm_acc(s_v[j * kR + rr], tf.v0[q], has, best, vl);
+      }
+    }
     // ---- traffic (one thread per car slot; they read the rollout's tick before it is counted)
     for (int64_t q = r0 * c + (threadIdx.x - 64); q < r_end * c; q += kB - 64) {
       const int64_t r = q / c;
@@ -490,6 +614,22 @@ k_sim_advance(Track trk, int64_t lo, int64_t n, int c, uint64_t seed, int64_t fi
         w = pl.ref_wp[r];
         u = 0.5;
         trk.walk(w, u, lane, ds);
+        if constexpr (kIdm) {
+          tf.v0[q] = v;
+          tf.acc[q] = 0.0;
+        }
+      } else if constexpr (kIdm) {  // the IDM step with the acceleration of the pass above
+        const double acc = tf.acc[q];
+        double v1 = v + acc * dt;
+        if (v1 < 0) v1 = 0;
+        const double ds = (v + v1) * 0.5 * dt;
+        u += ds / trk.len(w, lane);
+        for (int guard = 0; guard < 64 && u >= 1; guard++) {
+          const double left = (u - 1) * trk.len(w, lane);
+          w = w + 1 == trk.n ? 0 : w + 1;
+          u = left / trk.len(w, lane);
+        }
+        v = v1;
       } else {  // constant speed along the lane centre line
         u += (v * dt) / trk.len(w, lane);
         for (int guard = 0; guard < 64 && u >= 1; guard++) {
@@ -566,6 +706,20 @@ __global__ void __launch_bounds__(kB) k_incident_totals(Monitor mo, unsigned lon
   }
 }
 static_assert(PP_STATS_LEN <= 32, "k_sim_advance: a lane per statistics entry");
+
+// The ego's lane state before the first tick (pp.h, PP_TRAFFIC_IDM): the full reference search
+// of Map::init_reference_waypoint at the initial pose, then the lane match.  Whole warps run the
+// match (it votes across the warp); lanes past the end repeat the last rollout and store nothing.
+__global__ void __launch_bounds__(kB) k_traffic_init(Track trk, const double *ex, const double *ey,
+                                                     Traffic tf) {
+  const int64_t i = (int64_t)blockIdx.x * kB + threadIdx.x;
+  const int64_t r = i < tf.R ? i : tf.R - 1;
+  const ppd::MapView mv{trk.t, trk.n, trk.n < PPD_PAD ? trk.n : PPD_PAD};
+  ppd::RefState rs;
+  ppd::init_reference(mv, ex[r], ey[r], rs);
+  const ppd::Match mt = ppd::lane_match(mv, rs, ex[r], ey[r]);
+  if (i < tf.R) traffic_ego_state(trk, tf, r, 0, rs, mt);
+}
 
 inline size_t al(size_t v) { return (v + 255) & ~(size_t)255; }
 
@@ -794,10 +948,19 @@ extern "C" void pp_rollouts_destroy(pp_rollouts *r) {
   if (r->o_fork) cudaEventDestroy(r->o_fork);
   if (r->o_join) cudaEventDestroy(r->o_join);
   if (r->buf) cudaFree(r->buf);
+  if (r->trf_buf) cudaFree(r->trf_buf);
   delete r;
 }
 
 namespace {
+
+Traffic traffic_view(const pp_rollouts *r) {
+  return Traffic{r->trf_v0, r->trf_acc, r->trf_cum, r->trf_ego_lanes, r->trf_ego_s,
+                 r->fr.ego_speed_mph, r->n};
+}
+
+// dynamic shared memory of the IDM k_sim_advance: S and v (double) and lane (int) per car slot
+size_t traffic_smem_bytes(int c) { return (size_t)c * kR * (8 + 8 + 4); }
 
 // One tick of every group: issued on the group streams, forked from / joined to `st`.
 // One tick of every group.  Groups are independent (a rollout's tick t+1 depends on its own tick
@@ -853,8 +1016,15 @@ int issue_tick(pp_rollouts *r, const pp_config *cfg, int32_t consume_k, cudaStre
     int rc = ppi::plan_batch_scratch(r->map, cfg, &fr, &pl, cnt, gs, r->scratch[g], nullptr,
                                      (unsigned long long *)r->stats_sum + PP_STAT_XSUM);
     if (rc != PP_OK) return rc;
-    k_sim_advance<<<grid, kB, 0, gs>>>(trk, lo, cnt, r->c, r->seed, r->first, consume_k, sst, r->pl,
-                                       (unsigned long long *)r->stats_sum, plan_sums ? 0 : 1, mo);
+    const Traffic tf = traffic_view(r);
+    if (r->traffic == PP_TRAFFIC_IDM)
+      k_sim_advance<PP_TRAFFIC_IDM><<<grid, kB, traffic_smem_bytes(r->c), gs>>>(
+          trk, lo, cnt, r->c, r->seed, r->first, consume_k, sst, r->pl,
+          (unsigned long long *)r->stats_sum, plan_sums ? 0 : 1, mo, tf);
+    else
+      k_sim_advance<PP_TRAFFIC_CONSTANT><<<grid, kB, 0, gs>>>(
+          trk, lo, cnt, r->c, r->seed, r->first, consume_k, sst, r->pl,
+          (unsigned long long *)r->stats_sum, plan_sums ? 0 : 1, mo, tf);
     ppi::count_launch(2);
   }
   r->launches_per_tick = pp_launch_count() - launches0;
@@ -1032,6 +1202,88 @@ extern "C" int pp_rollouts_stats(const pp_rollouts *r, int64_t *stats_dev, void 
   cudaError_t e = cudaMemcpyAsync(stats_dev, r->stats_sum, PP_STATS_LEN * sizeof(int64_t),
                                   cudaMemcpyDeviceToDevice, (cudaStream_t)cuda_stream);
   if (e != cudaSuccess) return cuda_fail("pp_rollouts_stats", e);
+  return PP_OK;
+}
+
+extern "C" int pp_rollouts_set_traffic(pp_rollouts *r, int model) {
+  if (!r || r->tick != 0 || (model != PP_TRAFFIC_CONSTANT && model != PP_TRAFFIC_IDM))
+    return PP_E_ARG;
+  r->traffic = model;
+  if (model != PP_TRAFFIC_IDM) return PP_OK;
+  {
+    const int rc = ppi::check_map_device(r->map, "pp_rollouts_set_traffic");
+    if (rc != PP_OK) return rc;
+  }
+  const int nw = r->map->n;
+  const size_t N = (size_t)r->n, NC = (size_t)r->n * (size_t)r->c;
+  if (!r->trf_buf) {
+    const size_t bytes = al(NC * 8) * 2 + al(3 * (size_t)(nw + 1) * 8) + al(2 * N * 4) + al(6 * N * 8);
+    cudaError_t e = cudaMalloc((void **)&r->trf_buf, bytes);
+    if (e != cudaSuccess) {
+      r->traffic = PP_TRAFFIC_CONSTANT;
+      return cuda_fail("cudaMalloc(rollout traffic)", e);
+    }
+    char *b = r->trf_buf;
+    r->trf_v0 = (double *)b;
+    b += al(NC * 8);
+    r->trf_acc = (double *)b;
+    b += al(NC * 8);
+    r->trf_cum = (double *)b;
+    b += al(3 * (size_t)(nw + 1) * 8);
+    r->trf_ego_lanes = (int32_t *)b;
+    b += al(2 * N * 4);
+    r->trf_ego_s = (double *)b;
+  }
+  // cum(L, w), summed on the host in ascending w
+  std::vector<double> cum(3 * (size_t)(nw + 1));
+  for (int L = 0; L < 3; L++) {
+    double acc = 0.0;
+    cum[(size_t)L * (nw + 1)] = 0.0;
+    for (int w = 0; w < nw; w++) {
+      acc += r->map->table[(size_t)w * PP_MAP_STRIDE + 10 + L];
+      cum[(size_t)L * (nw + 1) + w + 1] = acc;
+    }
+  }
+  cudaError_t e = cudaMemcpy(r->trf_cum, cum.data(), cum.size() * 8, cudaMemcpyHostToDevice);
+  if (e == cudaSuccess && NC)
+    e = cudaMemcpy(r->trf_v0, r->car_speed, NC * 8, cudaMemcpyDeviceToDevice);
+  if (e == cudaSuccess && NC) e = cudaMemset(r->trf_acc, 0, NC * 8);
+  if (e != cudaSuccess) {
+    r->traffic = PP_TRAFFIC_CONSTANT;
+    return cuda_fail("pp_rollouts_set_traffic", e);
+  }
+  const Track trk{r->map->dev_table + (size_t)PPD_PAD_ROWS * PP_MAP_STRIDE, nw, PP_MAP_STRIDE};
+  k_traffic_init<<<(int)((r->n + kB - 1) / kB), kB>>>(trk, r->ego_x, r->ego_y, traffic_view(r));
+  ppi::count_launch(1);
+  e = cudaDeviceSynchronize();
+  if (e == cudaSuccess) e = cudaGetLastError();
+  if (e != cudaSuccess) {
+    r->traffic = PP_TRAFFIC_CONSTANT;
+    return cuda_fail("k_traffic_init", e);
+  }
+  return PP_OK;
+}
+
+extern "C" int pp_rollouts_get_traffic(const pp_rollouts *r, pp_rollout_traffic *h) {
+  if (!r || !h || r->traffic != PP_TRAFFIC_IDM) return PP_E_ARG;
+  cudaError_t e = cudaDeviceSynchronize();
+  if (e != cudaSuccess) return cuda_fail("pp_rollouts_get_traffic", e);
+  const size_t N = (size_t)r->n, NC = (size_t)r->n * (size_t)r->c;
+  const int buf = (int)(r->tick & 1);  // the copy the next tick reads
+  bool ok = true;
+  auto dn = [&](void *dst, const void *src, size_t bytes) {
+    if (dst && bytes && cudaMemcpy(dst, src, bytes, cudaMemcpyDeviceToHost) != cudaSuccess) ok = false;
+  };
+  dn(h->car_v0, r->trf_v0, NC * 8);
+  dn(h->car_acc, r->trf_acc, NC * 8);
+  dn(h->ego_lanes, r->trf_ego_lanes + buf * N, N * 4);
+  if (h->ego_s) {  // [L][R] on the device, [R][L] for the caller
+    std::vector<double> s(3 * N);
+    dn(s.data(), r->trf_ego_s + buf * 3 * N, 3 * N * 8);
+    for (size_t i = 0; i < N; i++)
+      for (int L = 0; L < 3; L++) h->ego_s[i * 3 + L] = s[L * N + i];
+  }
+  if (!ok) return cuda_fail("pp_rollouts_get_traffic copy", cudaGetLastError());
   return PP_OK;
 }
 

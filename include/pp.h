@@ -517,7 +517,8 @@ int pp_sweep_batch(const pp_map *map, const pp_config *cfg, const pp_frames *in,
  *     is carried over (:1195);  speed_mph = distance moved / (0.02 k) * 2.237;
  *     yaw stays at its initial value (the planner only reads it on a cold start);
  *   - each car keeps (lane, segment, ratio, speed) and advances along its lane
- *     centre line at constant speed; x, y, vx, vy are derived from that;
+ *     centre line at constant speed (or, with pp_rollouts_set_traffic, follows the
+ *     car ahead: PP_TRAFFIC_IDM below); x, y, vx, vy are derived from that;
  *   - a car whose ego-centred s (as matched by the planner this tick) leaves
  *     [-100, 300] m, or that the planner dropped, is respawned ahead (200-300 m)
  *     if it fell behind, behind (60-100 m) otherwise, in a random lane at
@@ -637,6 +638,65 @@ int pp_rollouts_get_incidents(const pp_rollouts *r, pp_rollout_incidents *host_o
 #define PP_INC_TOTAL_MM (PP_INC_KINDS + 1)
 #define PP_INC_TOTALS_LEN (PP_INC_KINDS + 2)
 int pp_rollouts_incident_totals(const pp_rollouts *r, int64_t *totals_dev, void *cuda_stream);
+
+/* ---- traffic models of the rollouts ------------------------------------------------------
+ * PP_TRAFFIC_CONSTANT (the default) is the model above: every car keeps its speed.
+ * PP_TRAFFIC_IDM replaces the constant-speed advance of a car that is not respawned by the
+ * Intelligent Driver Model (Treiber, Hennecke, Helbing 2000): every car follows the nearest car,
+ * or the ego, ahead of it in its lane.  Like the monitor, it is IEEE double + - * / and sqrt,
+ * left to right, without fused multiply-add, and its parameters below are fixed, independent of
+ * pp_config (the planner's tunables must not move the traffic).
+ *
+ * Along-lane coordinate.  cum(L, w) = sum of len(i, L) for i = 0 .. w-1 in ascending i (len = the
+ * table's lane length, column 10 + L); Lambda_L = cum(L, n).  A car at (L, w, u) sits at
+ * S = cum(L, w) + u * len(w, L): the segment from row w-1 to row w, as the frames position it.
+ * From follower f to candidate c, Delta = S_c - S_f, reduced into [0, Lambda_L) by at most one
+ * addition or subtraction of Lambda_L (+ when Delta < 0, - when Delta >= Lambda_L).  c is AHEAD
+ * of f when 0 < Delta < Lambda_L / 2, or Delta == 0 and c's slot is higher; the ego is slot C.
+ * The leader is the candidate ahead with the smallest Delta, the lowest slot among equal ones.
+ *
+ * The ego as a leader, at its position before the tick: bit L of `lanes` is set when the lane
+ * match of that position is ok and |d - (4 L + 2)| < PP_TRF_EGO_CORRIDOR (an ego changing lanes
+ * is in two), and S_ego[L] = cum(L, wrap(rs.wp)) + rs.ratio[L] * len(rs.wp, L), with (rs, d) the
+ * reference and the lane match of the monitor's lateral check at the tick's last driven point
+ * (RefState::ratio[L] is measured on the segment from row wp-1 to row wp, the one a car at
+ * w = wp sits on).  Tick t stores it and tick t+1 reads it.  Before the first tick it comes from
+ * Map::init_reference_waypoint's full search at the initial pose.  Its speed is
+ * ego_speed_mph / 2.237 (src/main.cpp:1239) of the frame.
+ *
+ * Step, synchronous: every car's acceleration is taken from the state of all cars before the
+ * tick (a car respawned this tick still counts at its old place), with v its speed and v0 its
+ * desired speed:
+ *   gap  = max(Delta_leader - PP_INC_CAR_HALF_LEN, PP_TRF_GAP_FLOOR)    (0: the monitor's overlap)
+ *   s*   = PP_TRF_MIN_GAP + max(0, v * T + v * (v - v_leader) / (2 * sqrt(a * b)))
+ *   q = v / v0, q2 = q * q;  acc = a * (1 - q2 * q2 - (s* / gap) * (s* / gap))   (the last
+ *          term is 0 without a leader), then clamped to [-PP_TRF_MAX_DEC, a]
+ *   v'   = v + acc * dt, floored at 0;  ds = (v + v') * 0.5 * dt;  dt = 0.02 k as before
+ * and the car advances ds along its lane with the constant model's segment carry (u += ds / len,
+ * ...).  A respawn draws as before; the drawn speed is the car's v0 and its current speed, and its
+ * acc is 0.  Selecting the model sets every car's v0 to its speed and its acc to 0.
+ * The incident monitor's definitions do not change. */
+#define PP_TRAFFIC_CONSTANT 0       /* constant speed (default) */
+#define PP_TRAFFIC_IDM 1            /* Intelligent Driver Model car following */
+#define PP_TRF_ACC 1.5              /* m/s^2, maximum acceleration a */
+#define PP_TRF_DEC 3.0              /* m/s^2, comfortable deceleration b */
+#define PP_TRF_MAX_DEC 9.0          /* m/s^2, clamp on braking */
+#define PP_TRF_HEADWAY 1.2          /* s, time headway T */
+#define PP_TRF_MIN_GAP 2.0          /* m, standstill gap s0 */
+#define PP_TRF_GAP_FLOOR 0.1        /* m, smallest gap the formula is given */
+#define PP_TRF_EGO_CORRIDOR 3.0     /* m, |d - lane centre| within which the ego leads a lane
+                                       (the reference's "car ahead" corridor, src/main.cpp:1383-1411) */
+/* Select the traffic model: before the first tick only (PP_E_ARG afterwards, or for an unknown
+ * model).  PP_TRAFFIC_IDM allocates its state and computes the ego's initial lane state. */
+int pp_rollouts_set_traffic(pp_rollouts *r, int model);
+typedef struct pp_rollout_traffic { /* host arrays; any pointer may be NULL */
+  double *car_v0, *car_acc;         /* [R][C] desired speed, last applied acceleration */
+  int32_t *ego_lanes;               /* [R] bit L: the ego is a leader in lane L */
+  double *ego_s;                    /* [R][3] S_ego per lane */
+} pp_rollout_traffic;
+/* Copy the IDM state out (synchronises the device); the ego part is what the next tick reads.
+ * PP_E_ARG unless PP_TRAFFIC_IDM is selected. */
+int pp_rollouts_get_traffic(const pp_rollouts *r, pp_rollout_traffic *host_out);
 
 #ifdef __cplusplus
 }

@@ -748,7 +748,7 @@ class Planner {
 class Rollouts {
  public:
   Rollouts(const Map &map, int64_t n, int n_cars = 12, uint64_t seed = 0x5EED, int64_t first = 0)
-      : n_(n), cfg_(default_config()) {
+      : n_(n), n_cars_(n_cars), cfg_(default_config()) {
     check(pp_rollouts_create(map.handle(), n, n_cars, seed, first, &h_), "pp_rollouts_create");
   }
   ~Rollouts() { pp_rollouts_destroy(h_); }
@@ -807,10 +807,32 @@ class Rollouts {
     check(pp_rollouts_get_incidents(h_, &h), "pp_rollouts_get_incidents");
     return r;
   }
+  // Traffic model (pp.h, PP_TRAFFIC_*), before the first tick only.
+  void set_traffic(int model) { check(pp_rollouts_set_traffic(h_, model), "pp_rollouts_set_traffic"); }
+  // The IDM traffic state (PP_TRAFFIC_IDM only); ego_s is [n][3].
+  struct Traffic {
+    std::vector<double> car_v0, car_acc, ego_s;
+    std::vector<int32_t> ego_lanes;
+  };
+  Traffic traffic() const {
+    Traffic t;
+    t.car_v0.resize((size_t)n_ * n_cars_);
+    t.car_acc.resize((size_t)n_ * n_cars_);
+    t.ego_lanes.resize(n_);
+    t.ego_s.resize((size_t)n_ * 3);
+    pp_rollout_traffic h;
+    h.car_v0 = t.car_v0.data();
+    h.car_acc = t.car_acc.data();
+    h.ego_lanes = t.ego_lanes.data();
+    h.ego_s = t.ego_s.data();
+    check(pp_rollouts_get_traffic(h_, &h), "pp_rollouts_get_traffic");
+    return t;
+  }
 
  private:
   pp_rollouts *h_ = nullptr;
   int64_t n_;
+  int n_cars_;
   pp_config cfg_;
 };
 

@@ -1,13 +1,16 @@
 """Incidents of closed-loop rollouts: which planner configuration drives further without one.
 
-    python profiles/rollout_incidents.py [--rollouts 65536] [--ticks 3000] [--cfg stock|fast_lane_change]
+    python profiles/rollout_incidents.py [--rollouts 65536] [--ticks 3000] [--cars 12]
+                                         [--cfg stock|fast_lane_change] [--traffic constant|idm]
 
 R rollouts x T ticks (default 65,536 x 3,000 = 60 s of driving each, consume_k = 1) with the
 incident monitor of include/pp.h; prints one JSON line: ego-frames/s of the timed run, miles
 driven, incidents per kind per 100 miles, the share of incident-free rollouts (collision_rear
 excluded, as in the monitor's definition) and best_clean_m in miles (min, median, p99, max),
-with the card's name and power limit.  --cfg fast_lane_change sets the planner's
-test_fast_lane_change = 1, everything else stays at the stock tunables.
+the planner's flag counts (BRAKE, MAXBRAKE, ADJUST, KEEP, ... summed over every frame), with the
+card's name and power limit.  --cfg fast_lane_change sets the planner's test_fast_lane_change = 1,
+everything else stays at the stock tunables.  --traffic idm selects the car-following traffic
+model (pp_rollouts_set_traffic, include/pp.h) instead of the constant-speed one.
 """
 from __future__ import annotations
 
@@ -42,6 +45,7 @@ def main():
     ap.add_argument("--consume-k", type=int, default=1)
     ap.add_argument("--seed", type=int, default=2026)
     ap.add_argument("--cfg", choices=["stock", "fast_lane_change"], default="stock")
+    ap.add_argument("--traffic", choices=["constant", "idm"], default="constant")
     args = ap.parse_args()
 
     import torch
@@ -52,6 +56,7 @@ def main():
     if args.cfg == "fast_lane_change":
         cfg.test_fast_lane_change = 1
     ro = pp.Rollouts(pp.Map(), args.rollouts, args.cars, seed=args.seed, lean=True)
+    ro.set_traffic(args.traffic)
     ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     ev0.record()
     ro.run(args.ticks, args.consume_k, cfg=cfg)
@@ -60,11 +65,12 @@ def main():
     ms = ev0.elapsed_time(ev1)
     tot = ro.incident_totals().cpu().numpy()
     rec = ro.incidents()
+    stats = ro.stats().cpu().numpy()
     miles = tot[pp.abi.INC_TOTAL_MM] / 1000.0 / METRES_PER_MILE
     best = rec["best_clean_m"] / METRES_PER_MILE
     name, power = card()
     line = {
-        "metric": "closed-loop incidents", "cfg": args.cfg,
+        "metric": "closed-loop incidents", "cfg": args.cfg, "traffic": args.traffic,
         "config": f"{args.rollouts} rollouts x {args.ticks} ticks, {args.cars} cars, "
                   f"consume_k={args.consume_k}, seed {args.seed}",
         "gpu": name or torch.cuda.get_device_name(0), "power_limit": power,
@@ -74,8 +80,11 @@ def main():
                                     for i, k in enumerate(pp.abi.INC_NAMES)},
         "incidents": {k: int(tot[i]) for i, k in enumerate(pp.abi.INC_NAMES)},
         "incident_free_share": 1.0 - float(tot[pp.abi.INC_TOTAL_ROLLOUTS]) / args.rollouts,
+        # an ego whose position became NaN or infinite poisons the millimetre total (llround)
+        "rollouts_nonfinite_distance": int((~np.isfinite(rec["distance_m"])).sum()),
         "best_clean_miles": {"min": float(best.min()), "median": float(np.median(best)),
                              "p99": float(np.percentile(best, 99)), "max": float(best.max())},
+        "flags": {f: int(stats[pp.abi.STAT_FLAG0 + i]) for i, f in enumerate(pp.abi.FLAG_NAMES)},
     }
     print(json.dumps(line))
 
