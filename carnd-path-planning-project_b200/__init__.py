@@ -46,7 +46,8 @@ EXPORTS = [
     "pp_rollouts_create", "pp_rollouts_destroy", "pp_rollouts_run", "pp_rollouts_last",
     "pp_rollouts_get_state", "pp_rollouts_stats", "pp_rollouts_set_lean", "pp_rollouts_set_groups",
     "pp_rollouts_get_incidents", "pp_rollouts_incident_totals", "pp_rollouts_set_traffic",
-    "pp_rollouts_get_traffic", "pp_sweep_batch",
+    "pp_rollouts_get_traffic", "pp_rollouts_set_recorder", "pp_rollouts_get_recording",
+    "pp_sweep_batch",
     "pp_set_pipes", "pp_plan_stats_batch", "pp_synth_frames_dev", "pp_fstats_batch",
     "pp_comm_unique_id", "pp_comm_init_rank", "pp_comm_init_all", "pp_comm_destroy",
     "pp_comm_group_begin", "pp_comm_group_end", "pp_stats_reduce",
@@ -504,6 +505,48 @@ class Rollouts:
                for name, dt, kind in abi.TRAFFIC_FIELDS}
         s = abi.RolloutTraffic(*[a.ctypes.data for a in out.values()])
         _check(lib.pp_rollouts_get_traffic(self._h, C.byref(s)), "pp_rollouts_get_traffic")
+        return out
+
+    def set_recorder(self, window: int, triggers=0):
+        """Switch the flight recorder on before the first tick (include/pp.h): keep each rollout's
+        frames of its last `window` ticks (0 = off) and freeze them at the first tick in which a
+        trigger fires.  `triggers` is a bit mask or an iterable of names of abi.REC_NAMES (the
+        incident kinds of abi.INC_NAMES and "nonfinite")."""
+        mask = abi.rec_mask(triggers)
+        if not 0 <= mask < 1 << 32 or not -2**31 <= window < 2**31:
+            raise PPError(f"pp_rollouts_set_recorder failed: window {window} / mask {mask:#x}")
+        _check(lib.pp_rollouts_set_recorder(self._h, C.c_int32(window), C.c_uint32(mask)),
+               "pp_rollouts_set_recorder")
+        self.rec_window = int(window)
+
+    def recorder_triggers(self) -> dict:
+        """trigger_tick (int64, -1: not frozen) and trigger_bits (uint32) of every rollout."""
+        out = {"trigger_tick": np.zeros(self.n, np.int64), "trigger_bits": np.zeros(self.n, np.uint32)}
+        s = abi.RolloutRecording(trigger_tick=out["trigger_tick"].ctypes.data,
+                                 trigger_bits=out["trigger_bits"].ctypes.data)
+        _check(lib.pp_rollouts_get_recording(self._h, None, C.c_int64(self.n), C.byref(s)),
+               "pp_rollouts_get_recording")
+        return out
+
+    def recording(self, rollouts=None) -> dict:
+        """The recorded windows of `rollouts` (indices; None: all) -> dict: trigger_tick,
+        trigger_bits [m], tick, consume_k [m][W] (oldest first; tick -1: slot not filled) and
+        "frames", a FrameBatch of m * W frames (frame (i, j) at i * W + j; unfilled slots are all
+        0), ready for the device planner or the CPU oracle."""
+        rows = None if rollouts is None else np.ascontiguousarray(rollouts, dtype=np.int64).reshape(-1)
+        m = self.n if rows is None else len(rows)
+        w = getattr(self, "rec_window", 0)
+        fb = FrameBatch(m * w, max(self.n_cars, 1))
+        out = {"trigger_tick": np.zeros(m, np.int64), "trigger_bits": np.zeros(m, np.uint32),
+               "tick": np.zeros((m, w), np.int64), "consume_k": np.zeros((m, w), np.int32)}
+        s = abi.RolloutRecording()
+        for name, _, kind in abi.REC_FIELDS:
+            a = out[name] if kind != "frame" else getattr(fb, name)
+            setattr(s, name, a.ctypes.data if a.size else None)
+        # a raw address must cross as c_void_p: a bare int is passed as a 32-bit C int
+        _check(lib.pp_rollouts_get_recording(self._h, None if rows is None else C.c_void_p(rows.ctypes.data),
+                                             C.c_int64(m), C.byref(s)), "pp_rollouts_get_recording")
+        out["frames"] = fb
         return out
 
     def incident_totals(self, stream=None):

@@ -193,6 +193,40 @@ class RolloutTraffic(C.Structure):
     _fields_ = [(n, _dp) for n, _, _ in TRAFFIC_FIELDS]
 
 
+# flight recorder of the rollouts (pp_rollouts_set_recorder): trigger bits are the PP_INC_* kinds
+# plus REC_NONFINITE (distance_m not finite)
+REC_NONFINITE = INC_KINDS
+REC_NAMES = INC_NAMES + ["nonfinite"]
+REC_MAX_WINDOW = 1024
+REC_FIELDS = [  # (name, dtype, inner) ; inner: 0 per row, 'window' per slot, else a frame field
+    ("trigger_tick", np.int64, 0), ("trigger_bits", np.uint32, 0),
+    ("tick", np.int64, "window"), ("consume_k", np.int32, "window"),
+    ("ego_x", np.float64, "frame"), ("ego_y", np.float64, "frame"),
+    ("ego_yaw_deg", np.float64, "frame"), ("ego_speed_mph", np.float64, "frame"),
+    ("prev_x", np.float64, "frame"), ("prev_y", np.float64, "frame"),
+    ("car_x", np.float64, "frame"), ("car_y", np.float64, "frame"),
+    ("car_vx", np.float64, "frame"), ("car_vy", np.float64, "frame"),
+    ("prev_n", np.int32, "frame"), ("target_lane_in", np.int32, "frame"),
+    ("n_cars", np.int32, "frame"), ("car_id", np.int32, "frame"),
+]
+
+
+class RolloutRecording(C.Structure):
+    _fields_ = [(n, _dp) for n, _, _ in REC_FIELDS]
+
+
+def rec_mask(triggers) -> int:
+    """Recorder trigger mask from an int or an iterable of names of REC_NAMES."""
+    if isinstance(triggers, (int, np.integer)):
+        return int(triggers)
+    mask = 0
+    for name in triggers:
+        if name not in REC_NAMES:
+            raise ValueError(f"unknown recorder trigger {name!r}; expected one of {REC_NAMES}")
+        mask |= 1 << REC_NAMES.index(name)
+    return mask
+
+
 def default_config() -> Config:
     """The literals of reference src/main.cpp:30,39-49 (also what
     pp_config_default writes; tests check the two agree)."""

@@ -8,6 +8,7 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <utility>
 #include <vector>
 
 #include "pp_device.cuh"
@@ -59,6 +60,17 @@ struct pp_rollouts {
   char *trf_buf = nullptr;
   double *trf_v0 = nullptr, *trf_acc = nullptr, *trf_cum = nullptr, *trf_ego_s = nullptr;
   int32_t *trf_ego_lanes = nullptr;
+  // flight recorder (pp.h, pp_rollouts_set_recorder); an allocation of its own, made only when
+  // it is switched on
+  int rec_w = 0;  // window W, 0 = off
+  uint32_t rec_mask = 0;
+  char *rec_buf = nullptr;
+  double *rec_ring = nullptr;
+  int64_t *rec_trig_tick = nullptr;
+  uint32_t *rec_trig_bits = nullptr;
+  // (first tick, consume_k) of every stretch of ticks run with one consume_k.  All rollouts tick
+  // together, so the host knows each tick's k; a window frozen long ago still finds its k here.
+  std::vector<std::pair<int64_t, int32_t>> rec_k;
 };
 
 namespace {
@@ -169,6 +181,25 @@ struct Traffic {
   int64_t R;
 };
 
+// The flight recorder on the device (pp.h, pp_rollouts_set_recorder).  The ring is W slots of
+// R * (25 + 4C) words, each laid out like the frames ([field][R...]), so a slot's stores coalesce
+// exactly like the frame stores beside them.  Within a slot, in units of R words: ego_x 0, ego_y 1,
+// ego_yaw_deg 2, ego_speed_mph 3, prev_x 4 (x10), prev_y 14 (x10), car_x 24, car_y 24 + C,
+// car_vx 24 + 2C, car_vy 24 + 3C (xC each), then prev_n and target_lane_in as int32 [R] each.
+struct Recorder {
+  double *ring;
+  int64_t *trig_tick;   // [R] tick the rollout froze in, -1 while it records
+  uint32_t *trig_bits;  // [R]
+  int64_t R;
+  int c, W;
+  unsigned mask;
+  __host__ __device__ int64_t slot_words() const { return (int64_t)(25 + 4 * c) * R; }
+  __device__ double *slot(int s) const { return ring + s * slot_words(); }
+  __device__ int32_t *ints(int s) const { return (int32_t *)(slot(s) + (int64_t)(24 + 4 * c) * R); }
+};
+static_assert(PP_INC_COLLISION_FRONT == 0 && PP_INC_COLLISION_REAR == 1,
+              "k_sim_advance: the collision word's bits are the trigger bits");
+
 // The ego's lane state from its reference and lane match (pp.h, PP_TRAFFIC_IDM).
 __device__ __forceinline__ void traffic_ego_state(const Track &trk, const Traffic &tf, int64_t r,
                                                   int buf, const ppd::RefState &rs,
@@ -263,9 +294,11 @@ __device__ __forceinline__ double div02(double a) {
 // with the kinematic ones updated; clean_m is stored, the active bits are left to the caller.
 // A_i is kept beside D_i in the history, so J_i reads A_{i-50} instead of recomputing it from
 // four points (the same operations on the same values: the same bits, fewer registers).
+// kRec: the kinds counted are also OR-ed into `fired` (the recorder's triggers).
+template <bool kRec>
 __device__ __forceinline__ unsigned monitor_points(const Monitor &mo, int64_t r, int k, double ox,
                                                    double oy, const double *nx, const double *ny,
-                                                   unsigned act, int64_t t) {
+                                                   unsigned act, int64_t t, unsigned &fired) {
   constexpr int H = PP_INC_HISTORY;
   constexpr unsigned kKin = (1u << PP_INC_OVER_SPEED) | (1u << PP_INC_OVER_ACC) | (1u << PP_INC_OVER_JERK);
   const int64_t R = mo.R;
@@ -318,6 +351,7 @@ __device__ __forceinline__ unsigned monitor_points(const Monitor &mo, int64_t r,
       for (int kind = PP_INC_OVER_SPEED; kind <= PP_INC_OVER_JERK; kind++)
         if ((rise >> kind) & 1u) monitor_count(mo, r, kind, t);
       clean = 0;
+      if constexpr (kRec) fired |= rise;
     }
     mo.clean[r] = clean;
     px = x;
@@ -384,12 +418,26 @@ constexpr int kR = 32;  // rollouts per block (one warp's worth: the ego part is
 
 // frame <- state.  The block's threads sweep the rollouts' scalars (a warp per field), their
 // kept points and their car slots, all coalesced.
+// kRec: the frame also goes to the recorder's slot tick % W of each rollout that is not frozen.
+template <bool kRec>
 __global__ void __launch_bounds__(kB, 6)
-k_sim_frames(Track trk, int64_t lo, int64_t n, int c, SimState st, pp_plans pl, pp_frames fr) {
+k_sim_frames(Track trk, int64_t lo, int64_t n, int c, SimState st, pp_plans pl, pp_frames fr,
+             Recorder rc) {
   const int64_t r0 = lo + (int64_t)blockIdx.x * kR;
   int64_t r_end = r0 + kR;
   if (r_end > lo + n) r_end = lo + n;
   const int nr = (int)(r_end - r0);
+  int *s_slot = nullptr;  // kRec: per rollout of the block, its slot, -1 frozen (or past the end)
+  if constexpr (kRec) {
+    __shared__ int slot_[kR];
+    if (threadIdx.x < kR) {
+      const int64_t r = r0 + threadIdx.x;
+      slot_[threadIdx.x] =
+          (int)threadIdx.x < nr && rc.trig_tick[r] < 0 ? (int)(st.ticks[r] % rc.W) : -1;
+    }
+    __syncthreads();
+    s_slot = slot_;
+  }
   {  // ego scalars: warp w copies field w
     const int field = threadIdx.x >> 5, rr = threadIdx.x & 31;
     const int64_t r = r0 + rr;
@@ -405,6 +453,20 @@ k_sim_frames(Track trk, int64_t lo, int64_t n, int c, SimState st, pp_plans pl, 
         default: break;
       }
     }
+    if constexpr (kRec) {
+      const int s = s_slot[rr];
+      if (s >= 0 && field < 6) {
+        double *const d = rc.slot(s);
+        switch (field) {
+          case 0: d[r] = st.ego_x[r]; break;
+          case 1: d[rc.R + r] = st.ego_y[r]; break;
+          case 2: d[2 * rc.R + r] = st.ego_yaw[r]; break;
+          case 3: d[3 * rc.R + r] = st.ego_mph[r]; break;
+          case 4: rc.ints(s)[r] = st.path_n[r]; break;
+          default: rc.ints(s)[rc.R + r] = st.target_lane[r]; break;
+        }
+      }
+    }
   }
   // kept points: the unconsumed points of the last plan, behind path_off
   for (int e = threadIdx.x; e < nr * PP_PREV_KEEP; e += kB) {
@@ -412,8 +474,18 @@ k_sim_frames(Track trk, int64_t lo, int64_t n, int c, SimState st, pp_plans pl, 
     const int64_t r = r0 + rr;
     const bool have = i < st.path_n[r];
     const int64_t src = r * PP_PATH_LEN + st.path_off[r] + i;
-    const_cast<double *>(fr.prev_x)[r0 * PP_PREV_KEEP + e] = have ? pl.next_x[src] : 0.0;
-    const_cast<double *>(fr.prev_y)[r0 * PP_PREV_KEEP + e] = have ? pl.next_y[src] : 0.0;
+    const double px = have ? pl.next_x[src] : 0.0;
+    const_cast<double *>(fr.prev_x)[r0 * PP_PREV_KEEP + e] = px;
+    const double py = have ? pl.next_y[src] : 0.0;
+    const_cast<double *>(fr.prev_y)[r0 * PP_PREV_KEEP + e] = py;
+    if constexpr (kRec) {
+      const int s = s_slot[rr];
+      if (s >= 0) {
+        double *const d = rc.slot(s) + r0 * PP_PREV_KEEP + e;
+        d[4 * rc.R] = px;
+        d[14 * rc.R] = py;
+      }
+    }
   }
   for (int64_t q = r0 * c + threadIdx.x; q < r_end * c; q += kB) {
     double x, y, vx, vy;
@@ -423,6 +495,17 @@ k_sim_frames(Track trk, int64_t lo, int64_t n, int c, SimState st, pp_plans pl, 
     const_cast<double *>(fr.car_y)[q] = y;
     const_cast<double *>(fr.car_vx)[q] = vx;
     const_cast<double *>(fr.car_vy)[q] = vy;
+    if constexpr (kRec) {
+      const int s = s_slot[(int)(q - r0 * c) / c];
+      if (s >= 0) {
+        double *const d = rc.slot(s) + 24 * rc.R + q;
+        const int64_t cr = (int64_t)c * rc.R;
+        d[0] = x;
+        d[cr] = y;
+        d[2 * cr] = vx;
+        d[3 * cr] = vy;
+      }
+    }
   }
 }
 static_assert(kB >= 7 * 32 && kR == 32, "k_sim_frames: a warp per scalar field, a lane per rollout");
@@ -450,11 +533,15 @@ static_assert(kB >= 7 * 32 && kR == 32, "k_sim_frames: a warp per scalar field, 
 // different rollouts read different banks and those of one rollout read the same word) and
 // meet at a barrier of their own, while warps 0 and 1 go on; warp 1 also stores the ego's lane
 // state for the next tick.
-template <int kTraffic>
+//
+// kRec: the ego warp, which knows the kinds it counts in the tick (the kinematic ones in
+// monitor_points, the lateral ones and the collisions after the barrier), compares them and the
+// finiteness of distance_m against the recorder's mask and freezes the rollout's window.
+template <int kTraffic, bool kRec>
 __global__ void __launch_bounds__(kB)
 k_sim_advance(Track trk, int64_t lo, int64_t n, int c, uint64_t seed, int64_t first, int consume_k,
               SimState st, pp_plans pl, unsigned long long *stats_sum, int do_xsum, Monitor mo,
-              Traffic tf) {
+              Traffic tf, Recorder rc) {
   constexpr bool kIdm = kTraffic == PP_TRAFFIC_IDM;
   __shared__ unsigned s_coll[kR];  // per rollout: bit 0 a front, bit 1 a rear collision began
   __shared__ unsigned s_lat[kR];   // per rollout: out-of-lane / off-road condition bits
@@ -463,6 +550,7 @@ k_sim_advance(Track trk, int64_t lo, int64_t n, int c, uint64_t seed, int64_t fi
   if (r_end > lo + n) r_end = lo + n;
   const int nr = (int)(r_end - r0);
   unsigned act = 0, act0 = 0;  // the ego warp's edge bits of its rollout, before and after
+  unsigned fired = 0;          // kRec: the kinematic kinds the ego warp counted in this tick
   int64_t tick = 0;
   bool drove = false;
   if (threadIdx.x < 32) {
@@ -496,8 +584,8 @@ k_sim_advance(Track trk, int64_t lo, int64_t n, int c, uint64_t seed, int64_t fi
       fl = pl.flags[r];
     }
     if (k > 0)
-      act = monitor_points(mo, r, k, ox, oy, pl.next_x + r * PP_PATH_LEN, pl.next_y + r * PP_PATH_LEN,
-                           act0, tick);
+      act = monitor_points<kRec>(mo, r, k, ox, oy, pl.next_x + r * PP_PATH_LEN,
+                                 pl.next_y + r * PP_PATH_LEN, act0, tick, fired);
     // counters: lane i ends up holding entry i of the statistics vector
     const unsigned full = 0xffffffffu;
     unsigned long long mine = 0;
@@ -682,6 +770,15 @@ k_sim_advance(Track trk, int64_t lo, int64_t n, int c, uint64_t seed, int64_t fi
       if (cb & 2u) monitor_count(mo, r, PP_INC_COLLISION_REAR, tick);
       if (rise | (cb & 1u)) mo.clean[r] = 0;
     }
+    if constexpr (kRec) {
+      unsigned hit = fired | rise | cb;
+      if (!isfinite(mo.dist[r])) hit |= 1u << PP_REC_NONFINITE;
+      hit &= rc.mask;
+      if (hit && rc.trig_tick[r] < 0) {
+        rc.trig_tick[r] = tick;
+        rc.trig_bits[r] = hit;
+      }
+    }
     st.ticks[r] += 1;
   }
 }
@@ -719,6 +816,69 @@ __global__ void __launch_bounds__(kB) k_traffic_init(Track trk, const double *ex
   ppd::init_reference(mv, ex[r], ey[r], rs);
   const ppd::Match mt = ppd::lane_match(mv, rs, ex[r], ey[r]);
   if (i < tf.R) traffic_ego_state(trk, tf, r, 0, rs, mt);
+}
+
+// The staging buffer of pp_rollouts_get_recording: m rows of W frames in pp_frames layout (frame
+// (i, j) at i * W + j), then the trigger arrays of the m rows.
+struct RecOut {
+  double *d[10];  // ego_x, ego_y, ego_yaw_deg, ego_speed_mph, prev_x, prev_y, car_x, car_y, car_vx, car_vy
+  int32_t *i[2];  // prev_n, target_lane_in
+  int64_t *trig_tick;
+  uint32_t *trig_bits;
+};
+
+// Gathers the windows of m rollouts (rows[i], or i when rows is NULL), oldest frame first: row i
+// ends at its trigger tick, or at tick ticks_done - 1 when it is not frozen, and holds its last
+// min(end + 1, W) ticks; the slots after those are 0.  blockIdx.y is the field: 0 the trigger
+// arrays, 1..12 the frame fields in the order of RecOut.
+__global__ void __launch_bounds__(kB) k_rec_gather(Recorder rc, const int64_t *rows, int64_t m,
+                                                   int64_t ticks_done, RecOut out) {
+  const int fld = blockIdx.y;
+  const int W = rc.W, c = rc.c;
+  if (fld == 0) {
+    for (int64_t i = (int64_t)blockIdx.x * kB + threadIdx.x; i < m; i += (int64_t)gridDim.x * kB) {
+      const int64_t r = rows ? rows[i] : i;
+      out.trig_tick[i] = rc.trig_tick[r];
+      out.trig_bits[i] = rc.trig_bits[r];
+    }
+    return;
+  }
+  // words per frame and offset in a slot (units of R words) of the frame field
+  const int f = fld - 1;
+  const int inner = f == 4 || f == 5 ? PP_PREV_KEEP : (f >= 6 && f < 10 ? c : 1);
+  const int64_t off = f < 4 ? f : (f < 6 ? 4 + 10 * (f - 4) : 24 + (int64_t)c * (f - 6));
+  // the destination, picked by a switch: indexing the parameter's arrays by a runtime field
+  // number would copy RecOut to the stack
+  double *dd = nullptr;
+  int32_t *di = nullptr;
+  switch (f) {
+    case 0: dd = out.d[0]; break;
+    case 1: dd = out.d[1]; break;
+    case 2: dd = out.d[2]; break;
+    case 3: dd = out.d[3]; break;
+    case 4: dd = out.d[4]; break;
+    case 5: dd = out.d[5]; break;
+    case 6: dd = out.d[6]; break;
+    case 7: dd = out.d[7]; break;
+    case 8: dd = out.d[8]; break;
+    case 9: dd = out.d[9]; break;
+    case 10: di = out.i[0]; break;
+    default: di = out.i[1]; break;
+  }
+  const int64_t total = m * W * inner;
+  for (int64_t e = (int64_t)blockIdx.x * kB + threadIdx.x; e < total; e += (int64_t)gridDim.x * kB) {
+    const int64_t fi = e / inner, i = fi / W;
+    const int k = (int)(e - fi * inner), j = (int)(fi - i * W);
+    const int64_t r = rows ? rows[i] : i;
+    const int64_t tt = rc.trig_tick[r], end = tt >= 0 ? tt : ticks_done - 1;
+    const int64_t filled = end + 1 < W ? end + 1 : W;
+    const int s = j < filled ? (int)((end - filled + 1 + j) % W) : -1;
+    if (dd) {
+      dd[e] = s >= 0 ? rc.slot(s)[off * rc.R + r * inner + k] : 0.0;
+    } else {
+      di[e] = s >= 0 ? rc.ints(s)[(f - 10) * rc.R + r] : 0;
+    }
+  }
 }
 
 inline size_t al(size_t v) { return (v + 255) & ~(size_t)255; }
@@ -949,6 +1109,7 @@ extern "C" void pp_rollouts_destroy(pp_rollouts *r) {
   if (r->o_join) cudaEventDestroy(r->o_join);
   if (r->buf) cudaFree(r->buf);
   if (r->trf_buf) cudaFree(r->trf_buf);
+  if (r->rec_buf) cudaFree(r->rec_buf);
   delete r;
 }
 
@@ -957,6 +1118,10 @@ namespace {
 Traffic traffic_view(const pp_rollouts *r) {
   return Traffic{r->trf_v0, r->trf_acc, r->trf_cum, r->trf_ego_lanes, r->trf_ego_s,
                  r->fr.ego_speed_mph, r->n};
+}
+
+Recorder recorder_view(const pp_rollouts *r) {
+  return Recorder{r->rec_ring, r->rec_trig_tick, r->rec_trig_bits, r->n, r->c, r->rec_w, r->rec_mask};
 }
 
 // dynamic shared memory of the IDM k_sim_advance: S and v (double) and lane (int) per car slot
@@ -1003,7 +1168,11 @@ int issue_tick(pp_rollouts *r, const pp_config *cfg, int32_t consume_k, cudaStre
     const pp_plans pl = ppi::offset_plans(r->pl, lo, mc);
     const SimState sst{r->ego_x, r->ego_y, r->ego_yaw, r->ego_mph, r->path_n, r->path_off,
                        r->target_lane, r->car_lane, r->car_wp, r->car_ratio, r->car_speed, r->tick_dev};
-    k_sim_frames<<<grid, kB, 0, gs>>>(trk, lo, cnt, r->c, sst, r->pl, r->fr);
+    const Recorder rec = recorder_view(r);
+    if (r->rec_w)
+      k_sim_frames<true><<<grid, kB, 0, gs>>>(trk, lo, cnt, r->c, sst, r->pl, r->fr, rec);
+    else
+      k_sim_frames<false><<<grid, kB, 0, gs>>>(trk, lo, cnt, r->c, sst, r->pl, r->fr, rec);
     if (!r->scratch[g]) {
       const size_t need = ppi::plan_scratch_bytes(per, mc);
       if (need && cudaMalloc((void **)&r->scratch[g], need) != cudaSuccess)
@@ -1017,14 +1186,13 @@ int issue_tick(pp_rollouts *r, const pp_config *cfg, int32_t consume_k, cudaStre
                                      (unsigned long long *)r->stats_sum + PP_STAT_XSUM);
     if (rc != PP_OK) return rc;
     const Traffic tf = traffic_view(r);
-    if (r->traffic == PP_TRAFFIC_IDM)
-      k_sim_advance<PP_TRAFFIC_IDM><<<grid, kB, traffic_smem_bytes(r->c), gs>>>(
-          trk, lo, cnt, r->c, r->seed, r->first, consume_k, sst, r->pl,
-          (unsigned long long *)r->stats_sum, plan_sums ? 0 : 1, mo, tf);
-    else
-      k_sim_advance<PP_TRAFFIC_CONSTANT><<<grid, kB, 0, gs>>>(
-          trk, lo, cnt, r->c, r->seed, r->first, consume_k, sst, r->pl,
-          (unsigned long long *)r->stats_sum, plan_sums ? 0 : 1, mo, tf);
+    const bool idm = r->traffic == PP_TRAFFIC_IDM;
+    auto *advance = idm ? (r->rec_w ? k_sim_advance<PP_TRAFFIC_IDM, true> : k_sim_advance<PP_TRAFFIC_IDM, false>)
+                        : (r->rec_w ? k_sim_advance<PP_TRAFFIC_CONSTANT, true>
+                                    : k_sim_advance<PP_TRAFFIC_CONSTANT, false>);
+    advance<<<grid, kB, idm ? traffic_smem_bytes(r->c) : 0, gs>>>(
+        trk, lo, cnt, r->c, r->seed, r->first, consume_k, sst, r->pl,
+        (unsigned long long *)r->stats_sum, plan_sums ? 0 : 1, mo, tf, rec);
     ppi::count_launch(2);
   }
   r->launches_per_tick = pp_launch_count() - launches0;
@@ -1060,6 +1228,8 @@ extern "C" int pp_rollouts_run(pp_rollouts *r, const pp_config *cfg, int64_t n_t
     const int rc = ppi::check_map_device(r->map, "pp_rollouts_run");
     if (rc != PP_OK) return rc;
   }
+  if (r->rec_w && (r->rec_k.empty() || r->rec_k.back().second != consume_k))
+    r->rec_k.emplace_back(r->tick, consume_k);
   // A tick is ~36 short launches over 8 streams (4 groups, each with its side stream).  It can
   // be captured once and replayed as a CUDA graph (PP_ROLLOUT_GRAPH=1; the pipeline's scratch is
   // owned by the rollouts object, so the graph holds only kernels, memsets and event edges).
@@ -1330,5 +1500,123 @@ extern "C" int pp_rollouts_incident_totals(const pp_rollouts *r, int64_t *totals
   ppi::count_launch(1);
   e = cudaGetLastError();
   if (e != cudaSuccess) return cuda_fail("k_incident_totals", e);
+  return PP_OK;
+}
+
+extern "C" int pp_rollouts_set_recorder(pp_rollouts *r, int32_t window, uint32_t triggers) {
+  if (!r || r->tick != 0 || window < 0 || window > PP_REC_MAX_WINDOW ||
+      (triggers >> (PP_REC_NONFINITE + 1)) != 0)
+    return PP_E_ARG;
+  if (r->rec_buf) {
+    cudaFree(r->rec_buf);
+    r->rec_buf = nullptr;
+  }
+  r->rec_w = 0;
+  r->rec_mask = 0;
+  r->rec_k.clear();
+  if (window == 0) return PP_OK;
+  const size_t N = (size_t)r->n;
+  const size_t ring = N * (size_t)window * (size_t)(200 + 32 * r->c);
+  cudaError_t e = cudaMalloc((void **)&r->rec_buf, al(ring) + al(N * 8) + al(N * 4));
+  if (e != cudaSuccess) {
+    r->rec_buf = nullptr;
+    return cuda_fail("cudaMalloc(rollout recorder)", e);
+  }
+  r->rec_ring = (double *)r->rec_buf;
+  r->rec_trig_tick = (int64_t *)(r->rec_buf + al(ring));
+  r->rec_trig_bits = (uint32_t *)(r->rec_buf + al(ring) + al(N * 8));
+  e = cudaMemset(r->rec_trig_tick, 0xff, N * 8);  // -1: recording
+  if (e == cudaSuccess) e = cudaMemset(r->rec_trig_bits, 0, N * 4);
+  if (e != cudaSuccess) {
+    cudaFree(r->rec_buf);
+    r->rec_buf = nullptr;
+    return cuda_fail("pp_rollouts_set_recorder", e);
+  }
+  r->rec_w = window;
+  r->rec_mask = triggers;
+  return PP_OK;
+}
+
+extern "C" int pp_rollouts_get_recording(const pp_rollouts *r, const int64_t *rollouts, int64_t m,
+                                         pp_rollout_recording *h) {
+  if (!r || !h || !r->rec_w || m < 0 || (!rollouts && m != r->n)) return PP_E_ARG;
+  for (int64_t i = 0; rollouts && i < m; i++)
+    if (rollouts[i] < 0 || rollouts[i] >= r->n) return PP_E_ARG;
+  if (m == 0) return PP_OK;
+  {
+    const int rc = ppi::check_map_device(r->map, "pp_rollouts_get_recording");
+    if (rc != PP_OK) return rc;
+  }
+  cudaError_t e = cudaDeviceSynchronize();
+  if (e != cudaSuccess) return cuda_fail("pp_rollouts_get_recording", e);
+  const int W = r->rec_w, c = r->c;
+  const size_t M = (size_t)m, MW = M * (size_t)W, MWC = MW * (size_t)c;
+  double *const dst_d[10] = {h->ego_x, h->ego_y, h->ego_yaw_deg, h->ego_speed_mph, h->prev_x,
+                             h->prev_y, h->car_x, h->car_y, h->car_vx, h->car_vy};
+  int32_t *const dst_i[2] = {h->prev_n, h->target_lane_in};
+  const size_t words_d[10] = {MW, MW, MW, MW, MW * PP_PREV_KEEP, MW * PP_PREV_KEEP, MWC, MWC, MWC, MWC};
+  bool frames = dst_i[0] || dst_i[1];
+  for (int f = 0; f < 10; f++) frames = frames || dst_d[f];
+  // staging: the rows, the trigger arrays, then (frames only) every frame field
+  size_t off = 0;
+  auto take = [&](size_t bytes) {
+    const size_t o = off;
+    off += al(bytes);
+    return o;
+  };
+  const size_t o_rows = rollouts ? take(M * 8) : 0, o_tt = take(M * 8), o_tb = take(M * 4);
+  size_t o_d[10] = {}, o_i[2] = {};
+  if (frames) {
+    for (int f = 0; f < 10; f++) o_d[f] = take(words_d[f] * 8);
+    for (int f = 0; f < 2; f++) o_i[f] = take(MW * 4);
+  }
+  char *buf = nullptr;
+  e = cudaMalloc((void **)&buf, off);
+  if (e != cudaSuccess) return cuda_fail("cudaMalloc(recording staging)", e);
+  RecOut out;
+  for (int f = 0; f < 10; f++) out.d[f] = (double *)(buf + o_d[f]);
+  for (int f = 0; f < 2; f++) out.i[f] = (int32_t *)(buf + o_i[f]);
+  out.trig_tick = (int64_t *)(buf + o_tt);
+  out.trig_bits = (uint32_t *)(buf + o_tb);
+  const int64_t *rows_dev = rollouts ? (const int64_t *)(buf + o_rows) : nullptr;
+  if (rollouts) e = cudaMemcpy(buf + o_rows, rollouts, M * 8, cudaMemcpyHostToDevice);
+  if (e == cudaSuccess) {
+    const size_t most = frames ? (MWC > MW * PP_PREV_KEEP ? MWC : MW * PP_PREV_KEEP) : M;
+    const size_t blocks = (most + kB - 1) / kB;
+    const dim3 grid((unsigned)(blocks < 4096 ? (blocks ? blocks : 1) : 4096), frames ? 13 : 1);
+    k_rec_gather<<<grid, kB>>>(recorder_view(r), rows_dev, m, r->tick, out);
+    ppi::count_launch(1);
+    e = cudaGetLastError();
+    if (e == cudaSuccess) e = cudaDeviceSynchronize();
+  }
+  std::vector<int64_t> tt(M);
+  auto dn = [&](void *dst, const void *src, size_t bytes) {
+    if (e == cudaSuccess && dst && bytes) e = cudaMemcpy(dst, src, bytes, cudaMemcpyDeviceToHost);
+  };
+  dn(tt.data(), out.trig_tick, M * 8);
+  dn(h->trigger_bits, out.trig_bits, M * 4);
+  for (int f = 0; frames && f < 10; f++) dn(dst_d[f], out.d[f], words_d[f] * 8);
+  for (int f = 0; frames && f < 2; f++) dn(dst_i[f], out.i[f], MW * 4);
+  cudaFree(buf);
+  if (e != cudaSuccess) return cuda_fail("pp_rollouts_get_recording copy", e);
+  // what the host knows: each slot's tick and consume_k, and the constant frame fields
+  if (h->trigger_tick) std::memcpy(h->trigger_tick, tt.data(), M * 8);
+  for (size_t i = 0; i < M; i++) {
+    const int64_t end = tt[i] >= 0 ? tt[i] : r->tick - 1;
+    const int64_t filled = end + 1 < W ? end + 1 : W;
+    for (int j = 0; j < W; j++) {
+      const size_t fi = i * W + j;
+      const int64_t t = j < filled ? end - filled + 1 + j : -1;
+      if (h->tick) h->tick[fi] = t;
+      if (h->consume_k) {
+        int32_t k = 0;
+        for (const auto &run : r->rec_k)  // a handful of entries: one per change of consume_k
+          if (t >= 0 && run.first <= t) k = run.second;
+        h->consume_k[fi] = k;
+      }
+      if (h->n_cars) h->n_cars[fi] = t >= 0 ? c : 0;
+      for (int q = 0; h->car_id && q < c; q++) h->car_id[fi * c + q] = t >= 0 ? q : 0;
+    }
+  }
   return PP_OK;
 }

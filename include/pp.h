@@ -698,6 +698,51 @@ typedef struct pp_rollout_traffic { /* host arrays; any pointer may be NULL */
  * PP_E_ARG unless PP_TRAFFIC_IDM is selected. */
 int pp_rollouts_get_traffic(const pp_rollouts *r, pp_rollout_traffic *host_out);
 
+/* ---- flight recorder of the rollouts -----------------------------------------------------
+ * An opt-in observer that keeps, for every rollout, the planner frames of its last W ticks and
+ * stops writing them (freezes) at the first tick in which a chosen trigger fires, so that the
+ * frames a rollout was given before it failed can be read back and replanned as they are.
+ *
+ * What is recorded.  Tick t is the rollout's own tick counter before the tick.  Unless the
+ * rollout is frozen, tick t writes its frame (the frame the simulator builds for the planner)
+ * into slot t % W.  Only the fields that vary are stored: ego_x, ego_y, ego_yaw_deg,
+ * ego_speed_mph, prev_n, target_lane_in, prev_x[10], prev_y[10], car_x / car_y / car_vx /
+ * car_vy[C], 200 + 32 C bytes a frame; car_id[j] = j and n_cars = C are filled in on read-back.
+ * Triggers.  `triggers` is a bit mask.  Bit PP_INC_<kind> fires in tick t when the monitor
+ * COUNTS an incident of that kind in tick t (edge-triggered, exactly as it counts); bit
+ * PP_REC_NONFINITE fires when the rollout's distance_m is not finite after tick t.  At the end
+ * of the first tick t in which a bit of the mask fires, the rollout freezes: trigger_tick = t,
+ * trigger_bits = every bit of the mask that fired in tick t.  The window then holds ticks
+ * max(0, t - W + 1) .. t; its last frame is the frame whose plan the ego was driving when the
+ * trigger fired.  A rollout that never triggers keeps its last W ticks.
+ * The recorder is an observer: state, plans, statistics, the incident record and the traffic
+ * state do not depend on whether it is on, on W or on the mask.
+ * Device memory: R * W * (200 + 32 C) bytes; 65,536 rollouts with W = 256 take 9.8 GB at 12
+ * cars and 37.7 GB at 64 cars. */
+#define PP_REC_NONFINITE PP_INC_KINDS  /* trigger bit: distance_m is not finite */
+#define PP_REC_MAX_WINDOW 1024         /* ticks; out-of-lane needs 150 driven points */
+/* Before the first tick only (PP_E_ARG afterwards).  window 0 = off (the default), else
+ * 1..PP_REC_MAX_WINDOW; triggers: bits below (1u << (PP_REC_NONFINITE + 1)), else PP_E_ARG.
+ * If the allocation fails the recorder is left off and the error returned. */
+int pp_rollouts_set_recorder(pp_rollouts *r, int32_t window, uint32_t triggers);
+typedef struct pp_rollout_recording { /* host arrays, m rows; any pointer may be NULL */
+  int64_t *trigger_tick;              /* [m] tick the rollout froze in, -1: not frozen */
+  uint32_t *trigger_bits;             /* [m] bits of the mask that fired then, 0: not frozen */
+  int64_t *tick;                      /* [m][W] oldest first; -1: slot not filled */
+  int32_t *consume_k;                 /* [m][W] consume_k of that tick, 0: slot not filled */
+  /* [m * W] frames in pp_frames layout with max_cars = C: frame (i, j) at i * W + j; the
+   * frames of unfilled slots are all 0 */
+  double *ego_x, *ego_y, *ego_yaw_deg, *ego_speed_mph, *prev_x, *prev_y;
+  double *car_x, *car_y, *car_vx, *car_vy;
+  int32_t *prev_n, *target_lane_in, *n_cars, *car_id;
+} pp_rollout_recording;
+/* Read back the windows of m rollouts (synchronises the device).  rollouts: host, m indices in
+ * [0, R); NULL means m == R and row i = rollout i.  PP_E_ARG without a recorder or for an index out
+ * of range.  With every frame pointer NULL only the trigger arrays are copied (how a caller finds
+ * the rollouts worth fetching). */
+int pp_rollouts_get_recording(const pp_rollouts *r, const int64_t *rollouts, int64_t m,
+                              pp_rollout_recording *host_out);
+
 #ifdef __cplusplus
 }
 #endif

@@ -828,11 +828,63 @@ class Rollouts {
     check(pp_rollouts_get_traffic(h_, &h), "pp_rollouts_get_traffic");
     return t;
   }
+  // Flight recorder (pp.h, pp_rollouts_set_recorder), before the first tick only.
+  void set_recorder(int window, uint32_t triggers) {
+    check(pp_rollouts_set_recorder(h_, window, triggers), "pp_rollouts_set_recorder");
+    window_ = window;
+  }
+  // The recorded windows of `rows` (all rollouts when empty): m rows of window() slots, oldest
+  // first; the frame fields are in pp_frames layout with max_cars = n_cars (frame (i, j) at
+  // i * window() + j).
+  struct Recording {
+    std::vector<int64_t> trigger_tick, tick;
+    std::vector<uint32_t> trigger_bits;
+    std::vector<int32_t> consume_k, prev_n, target_lane_in, n_cars, car_id;
+    std::vector<double> ego_x, ego_y, ego_yaw_deg, ego_speed_mph, prev_x, prev_y, car_x, car_y,
+        car_vx, car_vy;
+  };
+  Recording recording(const std::vector<int64_t> &rows = std::vector<int64_t>()) const {
+    const size_t m = rows.empty() ? (size_t)n_ : rows.size(), mw = m * (size_t)window_,
+                 mwc = mw * (size_t)n_cars_;
+    Recording o;
+    o.trigger_tick.resize(m);
+    o.trigger_bits.resize(m);
+    o.tick.resize(mw);
+    for (auto *v : {&o.consume_k, &o.prev_n, &o.target_lane_in, &o.n_cars}) v->resize(mw);
+    for (auto *v : {&o.ego_x, &o.ego_y, &o.ego_yaw_deg, &o.ego_speed_mph}) v->resize(mw);
+    o.prev_x.resize(mw * PP_PREV_KEEP);
+    o.prev_y.resize(mw * PP_PREV_KEEP);
+    for (auto *v : {&o.car_x, &o.car_y, &o.car_vx, &o.car_vy}) v->resize(mwc);
+    o.car_id.resize(mwc);
+    pp_rollout_recording h;
+    h.trigger_tick = o.trigger_tick.data();
+    h.trigger_bits = o.trigger_bits.data();
+    h.tick = o.tick.data();
+    h.consume_k = o.consume_k.data();
+    h.ego_x = o.ego_x.data();
+    h.ego_y = o.ego_y.data();
+    h.ego_yaw_deg = o.ego_yaw_deg.data();
+    h.ego_speed_mph = o.ego_speed_mph.data();
+    h.prev_x = o.prev_x.data();
+    h.prev_y = o.prev_y.data();
+    h.car_x = o.car_x.data();
+    h.car_y = o.car_y.data();
+    h.car_vx = o.car_vx.data();
+    h.car_vy = o.car_vy.data();
+    h.prev_n = o.prev_n.data();
+    h.target_lane_in = o.target_lane_in.data();
+    h.n_cars = o.n_cars.data();
+    h.car_id = o.car_id.data();
+    check(pp_rollouts_get_recording(h_, rows.empty() ? nullptr : rows.data(), (int64_t)m, &h),
+          "pp_rollouts_get_recording");
+    return o;
+  }
 
  private:
   pp_rollouts *h_ = nullptr;
   int64_t n_;
   int n_cars_;
+  int window_ = 0;
   pp_config cfg_;
 };
 
