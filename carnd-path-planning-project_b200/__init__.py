@@ -47,6 +47,7 @@ EXPORTS = [
     "pp_rollouts_get_state", "pp_rollouts_stats", "pp_rollouts_set_lean", "pp_rollouts_set_groups",
     "pp_rollouts_get_incidents", "pp_rollouts_incident_totals", "pp_rollouts_set_traffic",
     "pp_rollouts_get_traffic", "pp_rollouts_set_recorder", "pp_rollouts_get_recording",
+    "pp_rollouts_set_surrogate", "pp_rollouts_get_surrogate", "pp_rollouts_surrogate_totals",
     "pp_sweep_batch",
     "pp_set_pipes", "pp_plan_stats_batch", "pp_synth_frames_dev", "pp_fstats_batch",
     "pp_comm_unique_id", "pp_comm_init_rank", "pp_comm_init_all", "pp_comm_destroy",
@@ -547,6 +548,35 @@ class Rollouts:
         _check(lib.pp_rollouts_get_recording(self._h, None if rows is None else C.c_void_p(rows.ctypes.data),
                                              C.c_int64(m), C.byref(s)), "pp_rollouts_get_recording")
         out["frames"] = fb
+        return out
+
+    def set_surrogate(self, on: bool = True):
+        """Switch the near-miss measures on (or off) before the first tick (include/pp.h): time to
+        collision ahead and behind, time headway, their minima and exposure histograms."""
+        _check(lib.pp_rollouts_set_surrogate(self._h, C.c_int(1 if on else 0)),
+               "pp_rollouts_set_surrogate")
+
+    def surrogate(self) -> dict:
+        """The near-miss record (include/pp.h, pp_rollout_surrogate) as numpy arrays:
+        min_ttc_front, min_ttc_rear, min_thw [n] (s, inf: never defined), min_ttc_front_tick [n]
+        (-1: never), time_hist [n][SSM_MEASURES][SSM_BINS] (ticks' weights in units of 0.02 s;
+        measures in the order of abi.SSM_NAMES, bins below abi.SSM_EDGES)."""
+        inner = {0: (), "hist": (abi.SSM_MEASURES, abi.SSM_BINS)}
+        out = {name: np.zeros((self.n,) + inner[kind], dtype=dt) for name, dt, kind in abi.SSM_FIELDS}
+        s = abi.RolloutSurrogate(*[a.ctypes.data for a in out.values()])
+        _check(lib.pp_rollouts_get_surrogate(self._h, C.byref(s)), "pp_rollouts_get_surrogate")
+        return out
+
+    def surrogate_totals(self, stream=None):
+        """pp_rollouts_surrogate_totals -> int64[SSM_TOTALS_LEN] device tensor: time_hist summed
+        over the rollouts (entry m * SSM_BINS + b), then the rollouts per bin of their minima
+        (entry SSM_TOTAL_MIN + m * SSM_BINS + b)."""
+        import torch
+        if stream is None:
+            stream = torch.cuda.current_stream().cuda_stream
+        out = torch.empty(abi.SSM_TOTALS_LEN, dtype=torch.int64, device="cuda")
+        _check(lib.pp_rollouts_surrogate_totals(self._h, C.c_void_p(out.data_ptr()),
+                                                C.c_void_p(stream)), "pp_rollouts_surrogate_totals")
         return out
 
     def incident_totals(self, stream=None):

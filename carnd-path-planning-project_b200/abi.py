@@ -215,6 +215,24 @@ class RolloutRecording(C.Structure):
     _fields_ = [(n, _dp) for n, _, _ in REC_FIELDS]
 
 
+# near-miss measures of the rollouts (pp_rollouts_set_surrogate), in the order of PP_SSM_*
+SSM_NAMES = ["ttc_front", "ttc_rear", "thw"]
+SSM = {name: i for i, name in enumerate(SSM_NAMES)}
+SSM_MEASURES = len(SSM_NAMES)
+SSM_EDGES = [0.5, 1.0, 1.5, 2.0, 3.0, 4.0, 6.0, 8.0]  # s, upper bin edges (PP_SSM_EDGES)
+SSM_BINS = len(SSM_EDGES)
+SSM_TOTAL_MIN = SSM_MEASURES * SSM_BINS  # pp_rollouts_surrogate_totals: rollouts per bin of the minima
+SSM_TOTALS_LEN = 2 * SSM_MEASURES * SSM_BINS
+SSM_FIELDS = [  # (name, dtype, inner) ; inner: 0 scalar, 'hist' [SSM_MEASURES][SSM_BINS]
+    ("min_ttc_front", np.float64, 0), ("min_ttc_rear", np.float64, 0), ("min_thw", np.float64, 0),
+    ("min_ttc_front_tick", np.int64, 0), ("time_hist", np.int32, "hist"),
+]
+
+
+class RolloutSurrogate(C.Structure):
+    _fields_ = [(n, _dp) for n, _, _ in SSM_FIELDS]
+
+
 def rec_mask(triggers) -> int:
     """Recorder trigger mask from an int or an iterable of names of REC_NAMES."""
     if isinstance(triggers, (int, np.integer)):

@@ -71,6 +71,12 @@ struct pp_rollouts {
   // (first tick, consume_k) of every stretch of ticks run with one consume_k.  All rollouts tick
   // together, so the host knows each tick's k; a window frozen long ago still finds its k here.
   std::vector<std::pair<int64_t, int32_t>> rec_k;
+  // near-miss measures (pp.h, pp_rollouts_set_surrogate); an allocation of its own, made only
+  // when they are switched on
+  char *ssm_buf = nullptr;
+  double *ssm_min = nullptr;
+  int64_t *ssm_tick = nullptr;
+  int32_t *ssm_hist = nullptr;
 };
 
 namespace {
@@ -199,6 +205,24 @@ struct Recorder {
 };
 static_assert(PP_INC_COLLISION_FRONT == 0 && PP_INC_COLLISION_REAR == 1,
               "k_sim_advance: the collision word's bits are the trigger bits");
+
+// The near-miss record on the device (pp.h, pp_rollouts_set_surrogate).
+struct Surrogate {
+  double *min;        // [PP_SSM_MEASURES][R]
+  int64_t *min_tick;  // [R] tick min_ttc_front was last lowered in
+  int32_t *hist;      // [PP_SSM_MEASURES][PP_SSM_BINS][R]
+  int64_t R;
+};
+constexpr unsigned long long kInfBits = 0x7FF0000000000000ull;  // +inf
+
+// Bin of a value >= +0: the number of edges at or below it (PP_SSM_BINS: not counted).
+__host__ __device__ inline int ssm_bin(double v) {
+  constexpr double e[PP_SSM_BINS] = PP_SSM_EDGES;
+  int b = 0;
+#pragma unroll
+  for (int i = 0; i < PP_SSM_BINS; i++) b += v < e[i] ? 0 : 1;
+  return b;
+}
 
 // The ego's lane state from its reference and lane match (pp.h, PP_TRAFFIC_IDM).
 __device__ __forceinline__ void traffic_ego_state(const Track &trk, const Traffic &tf, int64_t r,
@@ -416,6 +440,46 @@ struct SimState {
 // fifty over its trajectory row.  Eight threads per rollout make that two trips and seven.
 constexpr int kR = 32;  // rollouts per block (one warp's worth: the ego part is one warp)
 
+// One car's near-miss measures against the ego at P = (px, py) moving at U (pp.h), merged into
+// the rollout's three shared words.  Every defined value is >= +0, and non-negative doubles order
+// like their bits, so an unsigned 64-bit atomicMin is an order-independent minimum.
+__device__ __forceinline__ void ssm_car(double cx, double cy, double tx, double ty, double px,
+                                        double py, double ux, double uy, double v,
+                                        unsigned long long *s_min) {
+  const double dx = cx - px, dy = cy - py;
+  const double along = dx * tx + dy * ty;
+  const double across = dx * ty - dy * tx;
+  if (!(fabs(across) < PP_INC_CAR_HALF_WIDTH)) return;
+  const double ut = ux * tx + uy * ty;
+  if (along >= PP_INC_CAR_HALF_LEN) {
+    const double gap = along - PP_INC_CAR_HALF_LEN;
+    const double w = ut - v;
+    if (w > 0) atomicMin(&s_min[PP_SSM_TTC_FRONT * kR], (unsigned long long)__double_as_longlong(gap / w));
+    if (ut > 0) atomicMin(&s_min[PP_SSM_THW * kR], (unsigned long long)__double_as_longlong(gap / ut));
+  } else if (along <= -PP_INC_CAR_HALF_LEN) {
+    const double gap = -along - PP_INC_CAR_HALF_LEN;
+    const double w = v - ut;
+    if (w > 0) atomicMin(&s_min[PP_SSM_TTC_REAR * kR], (unsigned long long)__double_as_longlong(gap / w));
+  }
+}
+
+// The ego warp's merge of a rollout's tick values into its record (rare stores: a minimum is
+// lowered, or a value falls below the last edge).
+__device__ __forceinline__ void ssm_merge(const Surrogate &sg, int64_t r, int64_t tick, int k,
+                                          const unsigned long long *s_min) {
+  const int weight = k > 0 ? k : 1;
+#pragma unroll
+  for (int m = 0; m < PP_SSM_MEASURES; m++) {
+    const double v = __longlong_as_double((long long)s_min[m * kR]);
+    const int b = ssm_bin(v);
+    if (b < PP_SSM_BINS) sg.hist[((int64_t)m * PP_SSM_BINS + b) * sg.R + r] += weight;
+    if (v < sg.min[m * sg.R + r]) {
+      sg.min[m * sg.R + r] = v;
+      if (m == PP_SSM_TTC_FRONT) sg.min_tick[r] = tick;
+    }
+  }
+}
+
 // frame <- state.  The block's threads sweep the rollouts' scalars (a warp per field), their
 // kept points and their car slots, all coalesced.
 // kRec: the frame also goes to the recorder's slot tick % W of each rollout that is not frozen.
@@ -537,14 +601,24 @@ static_assert(kB >= 7 * 32 && kR == 32, "k_sim_frames: a warp per scalar field, 
 // kRec: the ego warp, which knows the kinds it counts in the tick (the kinematic ones in
 // monitor_points, the lateral ones and the collisions after the barrier), compares them and the
 // finiteness of distance_m against the recorder's mask and freezes the rollout's window.
-template <int kTraffic, bool kRec>
+//
+// kSsm: the near-miss measures (pp.h).  The car-slot threads, which hold each advanced car and
+// the ego's P and E for the collision test, take every car's measures and atomicMin them into
+// three shared words per rollout (set to +inf beside the s_coll clear); after the block barrier
+// the ego warp merges the words into the record.
+template <int kTraffic, bool kRec, bool kSsm>
 __global__ void __launch_bounds__(kB)
 k_sim_advance(Track trk, int64_t lo, int64_t n, int c, uint64_t seed, int64_t first, int consume_k,
               SimState st, pp_plans pl, unsigned long long *stats_sum, int do_xsum, Monitor mo,
-              Traffic tf, Recorder rc) {
+              Traffic tf, Recorder rc, Surrogate sg) {
   constexpr bool kIdm = kTraffic == PP_TRAFFIC_IDM;
   __shared__ unsigned s_coll[kR];  // per rollout: bit 0 a front, bit 1 a rear collision began
   __shared__ unsigned s_lat[kR];   // per rollout: out-of-lane / off-road condition bits
+  unsigned long long *s_ssm = nullptr;  // kSsm: [PP_SSM_MEASURES][kR] bits of the tick's minima
+  if constexpr (kSsm) {
+    __shared__ unsigned long long ssm_[PP_SSM_MEASURES * kR];
+    s_ssm = ssm_;
+  }
   const int64_t r0 = lo + (int64_t)blockIdx.x * kR;
   int64_t r_end = r0 + kR;
   if (r_end > lo + n) r_end = lo + n;
@@ -553,8 +627,13 @@ k_sim_advance(Track trk, int64_t lo, int64_t n, int c, uint64_t seed, int64_t fi
   unsigned fired = 0;          // kRec: the kinematic kinds the ego warp counted in this tick
   int64_t tick = 0;
   bool drove = false;
+  int k_ssm = 0;  // kSsm: the ego warp's k, kept for the merge after the barrier
   if (threadIdx.x < 32) {
     s_coll[threadIdx.x] = 0;
+    if constexpr (kSsm) {
+#pragma unroll
+      for (int m = 0; m < PP_SSM_MEASURES; m++) s_ssm[m * kR + threadIdx.x] = kInfBits;
+    }
     asm volatile("bar.arrive 1, %0;" ::"n"(kB - 32) : "memory");  // the car-slot threads may OR now
     // ---- the ego consumes k points of the new trajectory (one lane per rollout)
     const int ln = threadIdx.x;
@@ -566,6 +645,7 @@ k_sim_advance(Track trk, int64_t lo, int64_t n, int c, uint64_t seed, int64_t fi
     tick = st.ticks[r];
     act0 = act = mo.active[r];
     drove = k > 0;
+    if constexpr (kSsm) k_ssm = k;
     int tl = -1, el = -1;
     uint32_t fl = 0;
     if (live) {
@@ -737,6 +817,14 @@ k_sim_advance(Track trk, int64_t lo, int64_t n, int c, uint64_t seed, int64_t fi
         const double ey = k > 0 ? pl.next_y[r * PP_PATH_LEN + k - 1] : mo.ego0_y[r];
         const int now = car_overlap(cx, cy, tx, ty, ex, ey);
         if (now && !was) atomicOr(&s_coll[r - r0], (unsigned)now);
+        if constexpr (kSsm) {
+          double ux = 0.0, uy = 0.0;
+          if (k > 0) {
+            ux = (ex - mo.ego0_x[r]) * 50.0 / k;
+            uy = (ey - mo.ego0_y[r]) * 50.0 / k;
+          }
+          ssm_car(cx, cy, tx, ty, ex, ey, ux, uy, v, s_ssm + (r - r0));
+        }
       }
     }
   }
@@ -779,6 +867,7 @@ k_sim_advance(Track trk, int64_t lo, int64_t n, int c, uint64_t seed, int64_t fi
         rc.trig_bits[r] = hit;
       }
     }
+    if constexpr (kSsm) ssm_merge(sg, r, tick, k_ssm, s_ssm + threadIdx.x);
     st.ticks[r] += 1;
   }
 }
@@ -803,6 +892,33 @@ __global__ void __launch_bounds__(kB) k_incident_totals(Monitor mo, unsigned lon
   }
 }
 static_assert(PP_STATS_LEN <= 32, "k_sim_advance: a lane per statistics entry");
+
+// pp_rollouts_surrogate_totals: the histograms summed over the rollouts, then the rollouts per
+// bin of their minima.
+__global__ void __launch_bounds__(kB) k_surrogate_totals(Surrogate sg, unsigned long long *tot) {
+  constexpr int MB = PP_SSM_MEASURES * PP_SSM_BINS;
+  unsigned long long acc[PP_SSM_TOTALS_LEN];
+#pragma unroll
+  for (int e = 0; e < PP_SSM_TOTALS_LEN; e++) acc[e] = 0;
+  for (int64_t r = (int64_t)blockIdx.x * kB + threadIdx.x; r < sg.R; r += (int64_t)gridDim.x * kB) {
+#pragma unroll
+    for (int e = 0; e < MB; e++) acc[e] += (unsigned long long)sg.hist[e * sg.R + r];
+#pragma unroll
+    for (int m = 0; m < PP_SSM_MEASURES; m++) {
+      const int b = ssm_bin(sg.min[m * sg.R + r]);
+#pragma unroll
+      for (int i = 0; i < PP_SSM_BINS; i++) acc[MB + m * PP_SSM_BINS + i] += b == i ? 1u : 0u;
+    }
+  }
+#pragma unroll
+  for (int e = 0; e < PP_SSM_TOTALS_LEN; e++) {
+    unsigned long long v = acc[e];
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) v += __shfl_down_sync(0xffffffffu, v, o);
+    if ((threadIdx.x & 31) == 0 && v) atomicAdd(&tot[e], v);
+  }
+}
+static_assert(PP_SSM_TOTAL_MIN == PP_SSM_MEASURES * PP_SSM_BINS, "k_surrogate_totals: layout");
 
 // The ego's lane state before the first tick (pp.h, PP_TRAFFIC_IDM): the full reference search
 // of Map::init_reference_waypoint at the initial pose, then the lane match.  Whole warps run the
@@ -1110,6 +1226,7 @@ extern "C" void pp_rollouts_destroy(pp_rollouts *r) {
   if (r->buf) cudaFree(r->buf);
   if (r->trf_buf) cudaFree(r->trf_buf);
   if (r->rec_buf) cudaFree(r->rec_buf);
+  if (r->ssm_buf) cudaFree(r->ssm_buf);
   delete r;
 }
 
@@ -1122,6 +1239,17 @@ Traffic traffic_view(const pp_rollouts *r) {
 
 Recorder recorder_view(const pp_rollouts *r) {
   return Recorder{r->rec_ring, r->rec_trig_tick, r->rec_trig_bits, r->n, r->c, r->rec_w, r->rec_mask};
+}
+
+Surrogate surrogate_view(const pp_rollouts *r) {
+  return Surrogate{r->ssm_min, r->ssm_tick, r->ssm_hist, r->n};
+}
+
+// The k_sim_advance instantiation for (traffic model, recorder on, near-miss measures on).
+template <int kTraffic>
+auto advance_kernel(bool rec, bool ssm) {
+  return rec ? (ssm ? k_sim_advance<kTraffic, true, true> : k_sim_advance<kTraffic, true, false>)
+             : (ssm ? k_sim_advance<kTraffic, false, true> : k_sim_advance<kTraffic, false, false>);
 }
 
 // dynamic shared memory of the IDM k_sim_advance: S and v (double) and lane (int) per car slot
@@ -1187,12 +1315,12 @@ int issue_tick(pp_rollouts *r, const pp_config *cfg, int32_t consume_k, cudaStre
     if (rc != PP_OK) return rc;
     const Traffic tf = traffic_view(r);
     const bool idm = r->traffic == PP_TRAFFIC_IDM;
-    auto *advance = idm ? (r->rec_w ? k_sim_advance<PP_TRAFFIC_IDM, true> : k_sim_advance<PP_TRAFFIC_IDM, false>)
-                        : (r->rec_w ? k_sim_advance<PP_TRAFFIC_CONSTANT, true>
-                                    : k_sim_advance<PP_TRAFFIC_CONSTANT, false>);
+    const bool ssm = r->ssm_buf != nullptr;
+    auto *advance = idm ? advance_kernel<PP_TRAFFIC_IDM>(r->rec_w != 0, ssm)
+                        : advance_kernel<PP_TRAFFIC_CONSTANT>(r->rec_w != 0, ssm);
     advance<<<grid, kB, idm ? traffic_smem_bytes(r->c) : 0, gs>>>(
         trk, lo, cnt, r->c, r->seed, r->first, consume_k, sst, r->pl,
-        (unsigned long long *)r->stats_sum, plan_sums ? 0 : 1, mo, tf, rec);
+        (unsigned long long *)r->stats_sum, plan_sums ? 0 : 1, mo, tf, rec, surrogate_view(r));
     ppi::count_launch(2);
   }
   r->launches_per_tick = pp_launch_count() - launches0;
@@ -1618,5 +1746,79 @@ extern "C" int pp_rollouts_get_recording(const pp_rollouts *r, const int64_t *ro
       for (int q = 0; h->car_id && q < c; q++) h->car_id[fi * c + q] = t >= 0 ? q : 0;
     }
   }
+  return PP_OK;
+}
+
+extern "C" int pp_rollouts_set_surrogate(pp_rollouts *r, int on) {
+  if (!r || r->tick != 0) return PP_E_ARG;
+  if (r->ssm_buf) {
+    cudaFree(r->ssm_buf);
+    r->ssm_buf = nullptr;
+    r->ssm_min = nullptr;
+    r->ssm_tick = nullptr;
+    r->ssm_hist = nullptr;
+  }
+  if (!on) return PP_OK;
+  const size_t N = (size_t)r->n, M = PP_SSM_MEASURES;
+  char *b = nullptr;
+  cudaError_t e = cudaMalloc((void **)&b, al(M * N * 8) + al(N * 8) + al(M * PP_SSM_BINS * N * 4));
+  if (e != cudaSuccess) return cuda_fail("cudaMalloc(rollout surrogate)", e);
+  double *mins = (double *)b;
+  int64_t *tick = (int64_t *)(b + al(M * N * 8));
+  int32_t *hist = (int32_t *)(b + al(M * N * 8) + al(N * 8));
+  const std::vector<double> inf(M * N, INFINITY);
+  e = cudaMemcpy(mins, inf.data(), M * N * 8, cudaMemcpyHostToDevice);
+  if (e == cudaSuccess) e = cudaMemset(tick, 0xff, N * 8);  // -1: never lowered
+  if (e == cudaSuccess) e = cudaMemset(hist, 0, M * PP_SSM_BINS * N * 4);
+  if (e != cudaSuccess) {
+    cudaFree(b);
+    return cuda_fail("pp_rollouts_set_surrogate", e);
+  }
+  r->ssm_buf = b;
+  r->ssm_min = mins;
+  r->ssm_tick = tick;
+  r->ssm_hist = hist;
+  return PP_OK;
+}
+
+extern "C" int pp_rollouts_get_surrogate(const pp_rollouts *r, pp_rollout_surrogate *h) {
+  if (!r || !h || !r->ssm_buf) return PP_E_ARG;
+  cudaError_t e = cudaDeviceSynchronize();
+  if (e != cudaSuccess) return cuda_fail("pp_rollouts_get_surrogate", e);
+  const size_t N = (size_t)r->n;
+  bool ok = true;
+  auto dn = [&](void *dst, const void *src, size_t bytes) {
+    if (dst && cudaMemcpy(dst, src, bytes, cudaMemcpyDeviceToHost) != cudaSuccess) ok = false;
+  };
+  double *const mins[PP_SSM_MEASURES] = {h->min_ttc_front, h->min_ttc_rear, h->min_thw};
+  for (int m = 0; m < PP_SSM_MEASURES; m++) dn(mins[m], r->ssm_min + m * N, N * 8);
+  dn(h->min_ttc_front_tick, r->ssm_tick, N * 8);
+  if (h->time_hist) {  // [measure][bin][R] on the device, [R][measure][bin] for the caller
+    constexpr int MB = PP_SSM_MEASURES * PP_SSM_BINS;
+    std::vector<int32_t> hist(N * MB);
+    dn(hist.data(), r->ssm_hist, N * MB * 4);
+    for (size_t i = 0; i < N; i++)
+      for (int e2 = 0; e2 < MB; e2++) h->time_hist[i * MB + e2] = hist[e2 * N + i];
+  }
+  if (!ok) return cuda_fail("pp_rollouts_get_surrogate copy", cudaGetLastError());
+  return PP_OK;
+}
+
+extern "C" int pp_rollouts_surrogate_totals(const pp_rollouts *r, int64_t *totals_dev,
+                                            void *cuda_stream) {
+  if (!r || !totals_dev || !r->ssm_buf) return PP_E_ARG;
+  {
+    const int rc = ppi::check_map_device(r->map, "pp_rollouts_surrogate_totals");
+    if (rc != PP_OK) return rc;
+  }
+  cudaStream_t st = (cudaStream_t)cuda_stream;
+  cudaError_t e = cudaMemsetAsync(totals_dev, 0, PP_SSM_TOTALS_LEN * sizeof(int64_t), st);
+  if (e != cudaSuccess) return cuda_fail("pp_rollouts_surrogate_totals", e);
+  const int64_t blocks = (r->n + kB - 1) / kB;
+  k_surrogate_totals<<<(int)(blocks < 1184 ? blocks : 1184), kB, 0, st>>>(
+      surrogate_view(r), (unsigned long long *)totals_dev);
+  ppi::count_launch(1);
+  e = cudaGetLastError();
+  if (e != cudaSuccess) return cuda_fail("k_surrogate_totals", e);
   return PP_OK;
 }

@@ -743,6 +743,65 @@ typedef struct pp_rollout_recording { /* host arrays, m rows; any pointer may be
 int pp_rollouts_get_recording(const pp_rollouts *r, const int64_t *rollouts, int64_t m,
                               pp_rollout_recording *host_out);
 
+/* ---- near-miss (surrogate safety) measures of the rollouts --------------------------------
+ * An opt-in observer that measures how close each ego comes to a collision, not only whether it
+ * has one: time to collision with the car ahead and the car behind (TTC, Hayward 1972), time
+ * headway to the car ahead, their running minima and how long each rollout spends below a set of
+ * thresholds (time-exposed TTC, Minderhoud & Bovy 2001).  Evaluated once per tick at the
+ * collision check's instant.  Every operation is IEEE double + - * /, left to right, without fused
+ * multiply-add, so the CPU restatement is bit-identical.
+ *
+ * Inputs of a tick.  E = the ego before the tick (this tick's frame); k = the points driven this
+ * tick; P = the last driven point, or E when k = 0; the ego's velocity U = (P - E) * 50 / k per
+ * component, left to right (U = 0 when k = 0).  Every car j after the advance (a respawned car at
+ * its new place): its position C and unit lane tangent t as the collision check takes them, and
+ * its speed v after the advance (velocity v t).
+ * Geometry per car, with the collision check's expressions:
+ *   dx = cx - px;  dy = cy - py;  along = dx*tx + dy*ty;  across = dx*ty - dy*tx;  ut = ux*tx + uy*ty
+ * The car is in the ego's path when fabs(across) < PP_INC_CAR_HALF_WIDTH.  A measure is defined
+ * only when its condition is true (every comparison with a NaN is false: a non-finite ego defines
+ * none):
+ *   ahead   in path and along >= PP_INC_CAR_HALF_LEN; gap = along - PP_INC_CAR_HALF_LEN
+ *             TTC ahead = gap / w with w = ut - v, when w > 0
+ *             time headway = gap / ut, when ut > 0
+ *   behind  in path and along <= -PP_INC_CAR_HALF_LEN; gap = -along - PP_INC_CAR_HALF_LEN
+ *             TTC behind = gap / w with w = v - ut, when w > 0
+ * (an overlapping car is the collision check's business and never a near miss).  The tick's value
+ * of each measure is its minimum over the cars, +inf when no car defines it.  Every defined value
+ * is >= +0.
+ * Record per rollout.  min_ttc_front, min_ttc_rear, min_thw: running minima of the tick values
+ * (+inf until first defined); min_ttc_front_tick: the rollout's tick counter at which
+ * min_ttc_front was last lowered (strict <), -1 never.  time_hist[m][b]: the tick's weight
+ * (k > 0 ? k : 1, in units of 0.02 s, the car model's dt) is added to bin b of measure m when the
+ * tick's value lies in [e_{b-1}, e_b), with e = PP_SSM_EDGES and e_{-1} = 0; values >= 8 s and
+ * +inf are not counted.  Binning uses comparisons only.
+ * The observer changes nothing else: state, plans, statistics, the incident record, the traffic
+ * state and the recorder are bit-identical with it on or off.  Device memory: 128 R bytes. */
+#define PP_SSM_TTC_FRONT 0
+#define PP_SSM_TTC_REAR 1
+#define PP_SSM_THW 2
+#define PP_SSM_MEASURES 3
+#define PP_SSM_BINS 8
+#define PP_SSM_EDGES {0.5, 1.0, 1.5, 2.0, 3.0, 4.0, 6.0, 8.0} /* s, upper bin edges */
+/* Before the first tick only (PP_E_ARG afterwards).  on != 0 allocates and clears the record;
+ * on == 0 (the default) frees it.  If the allocation fails the observer is left off. */
+int pp_rollouts_set_surrogate(pp_rollouts *r, int on);
+typedef struct pp_rollout_surrogate { /* host arrays, R rollouts; any pointer may be NULL */
+  double *min_ttc_front, *min_ttc_rear, *min_thw; /* [R] s, +inf: never defined */
+  int64_t *min_ttc_front_tick;                    /* [R] -1: never defined */
+  int32_t *time_hist;                             /* [R][PP_SSM_MEASURES][PP_SSM_BINS] */
+} pp_rollout_surrogate;
+/* Copy the record out (synchronises the device).  PP_E_ARG when the observer is off. */
+int pp_rollouts_get_surrogate(const pp_rollouts *r, pp_rollout_surrogate *host_out);
+/* totals_dev[PP_SSM_TOTALS_LEN] (device, int64, overwritten; asynchronous on cuda_stream):
+ * entry m * PP_SSM_BINS + b is time_hist[.][m][b] summed over the rollouts; entry
+ * PP_SSM_TOTAL_MIN + m * PP_SSM_BINS + b is the number of rollouts whose minimum of measure m lies
+ * in bin b (binned as above).  All int64, so a multi-GPU job all-reduces it with ncclSum.
+ * PP_E_ARG when the observer is off. */
+#define PP_SSM_TOTAL_MIN (PP_SSM_MEASURES * PP_SSM_BINS)
+#define PP_SSM_TOTALS_LEN (2 * PP_SSM_MEASURES * PP_SSM_BINS)
+int pp_rollouts_surrogate_totals(const pp_rollouts *r, int64_t *totals_dev, void *cuda_stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -879,6 +879,37 @@ class Rollouts {
           "pp_rollouts_get_recording");
     return o;
   }
+  // Near-miss measures (pp.h, pp_rollouts_set_surrogate), before the first tick only.
+  void set_surrogate(bool on = true) {
+    check(pp_rollouts_set_surrogate(h_, on ? 1 : 0), "pp_rollouts_set_surrogate");
+  }
+  // The near-miss record; time_hist is [n][PP_SSM_MEASURES][PP_SSM_BINS].
+  struct Surrogate {
+    std::vector<double> min_ttc_front, min_ttc_rear, min_thw;
+    std::vector<int64_t> min_ttc_front_tick;
+    std::vector<int32_t> time_hist;
+  };
+  Surrogate surrogate() const {
+    Surrogate o;
+    for (auto *v : {&o.min_ttc_front, &o.min_ttc_rear, &o.min_thw}) v->resize(n_);
+    o.min_ttc_front_tick.resize(n_);
+    o.time_hist.resize((size_t)n_ * PP_SSM_MEASURES * PP_SSM_BINS);
+    pp_rollout_surrogate h;
+    h.min_ttc_front = o.min_ttc_front.data();
+    h.min_ttc_rear = o.min_ttc_rear.data();
+    h.min_thw = o.min_thw.data();
+    h.min_ttc_front_tick = o.min_ttc_front_tick.data();
+    h.time_hist = o.time_hist.data();
+    check(pp_rollouts_get_surrogate(h_, &h), "pp_rollouts_get_surrogate");
+    return o;
+  }
+  // The totals (pp.h, pp_rollouts_surrogate_totals), copied to the host.
+  std::vector<int64_t> surrogate_totals() const {
+    detail::Dev<int64_t> dev(PP_SSM_TOTALS_LEN);
+    check(pp_rollouts_surrogate_totals(h_, dev.get(), nullptr), "pp_rollouts_surrogate_totals");
+    check(pp_dev_sync(), "pp_dev_sync");
+    return dev.to_host();
+  }
 
  private:
   pp_rollouts *h_ = nullptr;
