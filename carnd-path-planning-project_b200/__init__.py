@@ -484,9 +484,7 @@ class Rollouts:
         """The incident monitor's record (include/pp.h, pp_rollout_incidents) as numpy arrays:
         count [n][INC_KINDS] (columns in the order of abi.INC_NAMES), first_tick / first_kind [n]
         (-1: none), distance_m, clean_m, best_clean_m, max_speed, max_acc, max_jerk [n]."""
-        out = {name: np.zeros((self.n, abi.INC_KINDS) if kind else (self.n,), dtype=dt)
-               for name, dt, kind in abi.INC_FIELDS}
-        s = abi.RolloutIncidents(*[a.ctypes.data for a in out.values()])
+        out, s = abi.host_record(abi.INC_FIELDS, abi.RolloutIncidents, self.n)
         _check(lib.pp_rollouts_get_incidents(self._h, C.byref(s)), "pp_rollouts_get_incidents")
         return out
 
@@ -501,10 +499,7 @@ class Rollouts:
         """The IDM traffic state (only under abi.TRAFFIC_IDM) as numpy arrays: car_v0, car_acc
         [n][n_cars], and the ego's lane state the next tick reads, ego_lanes [n] (bit L: the ego
         leads lane L) and ego_s [n][3]."""
-        inner = {"cars": (self.n_cars,), 0: (), "lanes": (3,)}
-        out = {name: np.zeros((self.n,) + inner[kind], dtype=dt)
-               for name, dt, kind in abi.TRAFFIC_FIELDS}
-        s = abi.RolloutTraffic(*[a.ctypes.data for a in out.values()])
+        out, s = abi.host_record(abi.TRAFFIC_FIELDS, abi.RolloutTraffic, self.n, self.n_cars)
         _check(lib.pp_rollouts_get_traffic(self._h, C.byref(s)), "pp_rollouts_get_traffic")
         return out
 
@@ -561,9 +556,7 @@ class Rollouts:
         min_ttc_front, min_ttc_rear, min_thw [n] (s, inf: never defined), min_ttc_front_tick [n]
         (-1: never), time_hist [n][SSM_MEASURES][SSM_BINS] (ticks' weights in units of 0.02 s;
         measures in the order of abi.SSM_NAMES, bins below abi.SSM_EDGES)."""
-        inner = {0: (), "hist": (abi.SSM_MEASURES, abi.SSM_BINS)}
-        out = {name: np.zeros((self.n,) + inner[kind], dtype=dt) for name, dt, kind in abi.SSM_FIELDS}
-        s = abi.RolloutSurrogate(*[a.ctypes.data for a in out.values()])
+        out, s = abi.host_record(abi.SSM_FIELDS, abi.RolloutSurrogate, self.n)
         _check(lib.pp_rollouts_get_surrogate(self._h, C.byref(s)), "pp_rollouts_get_surrogate")
         return out
 

@@ -252,7 +252,15 @@ def default_config() -> Config:
 
 
 def _inner(kind, max_cars):
-    return {0: (), "prev": (PREV_KEEP,), "path": (PATH_LEN,), "cars": (max_cars,)}[kind]
+    return {0: (), "prev": (PREV_KEEP,), "path": (PATH_LEN,), "cars": (max_cars,),
+            "kinds": (INC_KINDS,), "lanes": (NUM_LANES,), "hist": (SSM_MEASURES, SSM_BINS)}[kind]
+
+
+def host_record(fields, struct, n: int, max_cars: int = 0):
+    """Zeroed host arrays of a record of n rollouts, one [n] + inner shape per (name, dtype, kind)
+    of `fields` (INC_FIELDS, TRAFFIC_FIELDS, SSM_FIELDS), and the `struct` pointing at them."""
+    arrays = {name: np.zeros((n,) + _inner(kind, max_cars), dtype=dt) for name, dt, kind in fields}
+    return arrays, struct(*[a.ctypes.data for a in arrays.values()])
 
 
 class FrameBatch:

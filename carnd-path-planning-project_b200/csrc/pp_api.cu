@@ -389,7 +389,7 @@ struct Staging {
 
 thread_local Staging t_stage;
 
-inline size_t align256(size_t v) { return (v + 255) & ~(size_t)255; }
+using ppi::align256;
 
 #define CK(call)                                                    \
   do {                                                              \

@@ -1,5 +1,6 @@
 // Internal declarations shared by the translation units of libpp_b200.so.
 #pragma once
+#include <cstddef>
 #include <cstdint>
 #include <vector>
 
@@ -35,6 +36,23 @@ void set_cuda_error(const char *what, int cuda_err, const char *text);
 // device table, PP_E_ARG when it was created on another device (using it would dereference a
 // foreign device pointer inside a kernel and poison the context).
 int check_map_device(const pp_map *map, const char *who);
+
+// Device buffers are carved into sub-buffers that start on 256-byte boundaries.
+inline size_t align256(size_t v) { return (v + 255) & ~(size_t)255; }
+
+// Typed sub-buffers of one allocation.  A layout is one block of take() calls run twice: on a
+// Carve without a base it only adds up the size (and hands out nullptr), on the allocated base
+// it binds the pointers at the same offsets.
+struct Carve {
+  char *base = nullptr;
+  size_t size = 0;  // bytes taken so far, a multiple of 256
+  explicit Carve(char *b = nullptr) : base(b) {}
+  template <class T>
+  void take(T *&p, size_t count) {
+    p = base ? (T *)(base + size) : nullptr;
+    size += align256(count * sizeof(T));
+  }
+};
 
 // pp_plan.cu: the pipeline with caller-owned scratch (see there)
 size_t plan_scratch_bytes(int64_t n_frames, int max_cars);

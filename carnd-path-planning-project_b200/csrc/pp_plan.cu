@@ -540,47 +540,33 @@ constexpr int kEstRows = kEstHead + 5 * PPD_TAILK;
 constexpr int kEstPartial = 1 << 8;
 constexpr int kEstFallback = 1 << 9;  // e_nk = kEstFallback | ncp: state for k_fallback, not k_emit
 
-size_t scratch_bytes(int64_t n, int mc) {
-  const size_t per_frame = 11 * 8 + 4 * 4 + (size_t)kEstRows * 8 + 3 * 4;
-  const size_t per_car = 4 * 8 + 4;
-  return (size_t)n * (per_frame + (size_t)mc * per_car) + 64 * 256;
-}
-
-Scratch carve_scratch(char *base, int64_t n, int mc) {
-  Scratch s;
-  size_t off = 0;
-  auto take = [&](size_t bytes) {
-    char *p = base + off;
-    off += (bytes + 255) & ~(size_t)255;
-    return p;
-  };
+// The scratch of one chunk of n frames, carved by `cv` (see ppi::Carve).
+Scratch carve_scratch(ppi::Carve &cv, int64_t n, int mc) {
+  Scratch s = {};
   const size_t N = (size_t)n, NC = (size_t)n * (size_t)mc;
-  s.x = (double *)take(N * 8);
-  s.y = (double *)take(N * 8);
-  s.speed = (double *)take(N * 8);
-  s.acc = (double *)take(N * 8);
-  s.s = (double *)take(N * 8);
-  s.d = (double *)take(N * 8);
-  s.vs = (double *)take(N * 8);
-  s.vd = (double *)take(N * 8);
-  s.ratio = (double *)take(3 * N * 8);
-  s.wp = (int32_t *)take(N * 4);
-  s.lane = (int32_t *)take(N * 4);
-  s.nprev = (int32_t *)take(N * 4);
-  s.flags = (uint32_t *)take(N * 4);
-  s.car_s = (double *)take(NC * 8);
-  s.car_d = (double *)take(NC * 8);
-  s.car_vs = (double *)take(NC * 8);
-  s.car_vd = (double *)take(NC * 8);
-  s.car_lane = (int32_t *)take(NC * 4);
-  s.est = (double *)take((size_t)kEstRows * N * 8);
-  s.e_np = (int32_t *)take(N * 4);
-  s.e_nk = (int32_t *)take(N * 4);
-  s.e_flags = (uint32_t *)take(N * 4);
-  s.slow_qa = s.slow_qb = s.slow_na = s.slow_nb = s.dbg = nullptr;  // set per chunk by the caller
-  s.xsum = nullptr;
-  s.bh_d = nullptr;
-  s.bh_i = nullptr;
+  cv.take(s.x, N);
+  cv.take(s.y, N);
+  cv.take(s.speed, N);
+  cv.take(s.acc, N);
+  cv.take(s.s, N);
+  cv.take(s.d, N);
+  cv.take(s.vs, N);
+  cv.take(s.vd, N);
+  cv.take(s.ratio, 3 * N);
+  cv.take(s.wp, N);
+  cv.take(s.lane, N);
+  cv.take(s.nprev, N);
+  cv.take(s.flags, N);
+  cv.take(s.car_s, NC);
+  cv.take(s.car_d, NC);
+  cv.take(s.car_vs, NC);
+  cv.take(s.car_vd, NC);
+  cv.take(s.car_lane, NC);
+  cv.take(s.est, (size_t)kEstRows * N);
+  cv.take(s.e_np, N);
+  cv.take(s.e_nk, N);
+  cv.take(s.e_flags, N);
+  // slow_qa / slow_qb / slow_na / slow_nb / dbg / xsum are set per chunk by the caller
   s.n = n;
   return s;
 }
@@ -590,40 +576,37 @@ Scratch carve_scratch(char *base, int64_t n, int mc) {
 // multiple of 32 frames.
 constexpr int kBehavDoubles = 10, kBehavInts = 10;
 int64_t scratch3_stride(int64_t n) { return (n + 31) / 32 * 32; }
-size_t scratch3_bytes(int64_t n) {
-  const size_t N = (size_t)scratch3_stride(n);
-  return N * (11 * 8 + 4 * 4 + kBehavDoubles * 8 + kBehavInts * 4 + (size_t)kEstRows * 8 + 3 * 4) +
-         40 * 256;
-}
-Scratch carve_scratch3(char *base, int64_t n) {
+Scratch carve_scratch3(ppi::Carve &cv, int64_t n) {
   Scratch s = {};
-  size_t off = 0;
-  auto take = [&](size_t bytes) {
-    char *p = base + off;
-    off += (bytes + 255) & ~(size_t)255;
-    return p;
-  };
   const size_t N = (size_t)scratch3_stride(n);
-  s.x = (double *)take(N * 8);
-  s.y = (double *)take(N * 8);
-  s.speed = (double *)take(N * 8);
-  s.acc = (double *)take(N * 8);
-  s.s = (double *)take(N * 8);
-  s.d = (double *)take(N * 8);
-  s.vs = (double *)take(N * 8);
-  s.vd = (double *)take(N * 8);
-  s.ratio = (double *)take(3 * N * 8);
-  s.wp = (int32_t *)take(N * 4);
-  s.lane = (int32_t *)take(N * 4);
-  s.nprev = (int32_t *)take(N * 4);
-  s.flags = (uint32_t *)take(N * 4);
-  s.bh_d = (double *)take((size_t)kBehavDoubles * N * 8);
-  s.bh_i = (int32_t *)take((size_t)kBehavInts * N * 4);
-  s.est = (double *)take((size_t)kEstRows * N * 8);
-  s.e_np = (int32_t *)take(N * 4);
-  s.e_nk = (int32_t *)take(N * 4);
-  s.e_flags = (uint32_t *)take(N * 4);
+  cv.take(s.x, N);
+  cv.take(s.y, N);
+  cv.take(s.speed, N);
+  cv.take(s.acc, N);
+  cv.take(s.s, N);
+  cv.take(s.d, N);
+  cv.take(s.vs, N);
+  cv.take(s.vd, N);
+  cv.take(s.ratio, 3 * N);
+  cv.take(s.wp, N);
+  cv.take(s.lane, N);
+  cv.take(s.nprev, N);
+  cv.take(s.flags, N);
+  cv.take(s.bh_d, (size_t)kBehavDoubles * N);
+  cv.take(s.bh_i, (size_t)kBehavInts * N);
+  cv.take(s.est, (size_t)kEstRows * N);
+  cv.take(s.e_np, N);
+  cv.take(s.e_nk, N);
+  cv.take(s.e_flags, N);
   s.n = (int64_t)N;
+  return s;
+}
+
+// One chunk's scratch at `base` (variant 3: the tiled pipeline's); a null base only sizes it.
+Scratch carve_chunk(char *base, bool tiled, int64_t n, int mc, size_t *bytes = nullptr) {
+  ppi::Carve cv(base);
+  const Scratch s = tiled ? carve_scratch3(cv, n) : carve_scratch(cv, n, mc);
+  if (bytes) *bytes = cv.size;
   return s;
 }
 
@@ -1881,8 +1864,8 @@ size_t ppi::plan_scratch_bytes(int64_t n_frames, int max_cars) {
   const int64_t chunk = chunk_for(n_frames, 1);
   const int64_t n_chunks = (n_frames + chunk - 1) / chunk;
   const int n_buf = 1;
-  const size_t scratch =
-      ((variant == 3 ? scratch3_bytes(chunk) : scratch_bytes(chunk, max_cars)) + 255) & ~(size_t)255;
+  size_t scratch = 0;
+  carve_chunk(nullptr, variant == 3, chunk, max_cars, &scratch);
   return n_buf * scratch + (size_t)n_frames * 2 * sizeof(int32_t) +
          (size_t)n_chunks * 2 * sizeof(int32_t) + 256;
 }
@@ -2017,8 +2000,8 @@ int ppi::plan_batch_scratch(const pp_map *map, const pp_config *cfg, const pp_fr
     lane_side[k] = &side_for(lane_st[k]);
     if ((rc = lane_side[k]->ensure()) != PP_OK) return rc;
   }
-  const size_t scratch =
-      ((tiled ? scratch3_bytes(chunk) : scratch_bytes(chunk, mc)) + 255) & ~(size_t)255;
+  size_t scratch = 0;
+  carve_chunk(nullptr, tiled, chunk, mc, &scratch);
   const size_t queues = (size_t)n_frames * 2 * sizeof(int32_t);
   const size_t counters = (size_t)n_chunks * 2 * sizeof(int32_t);
   char *buf = caller_scratch;
@@ -2032,7 +2015,7 @@ int ppi::plan_batch_scratch(const pp_map *map, const pp_config *cfg, const pp_fr
   }
   Scratch scs[kMaxPipes];
   for (int k = 0; k < pipes; k++)
-    scs[k] = tiled ? carve_scratch3(buf + k * scratch, chunk) : carve_scratch(buf + k * scratch, chunk, mc);
+    scs[k] = carve_chunk(buf + k * scratch, tiled, chunk, mc);
   static const int cars_items = env_int("PP_CARS_ITEMS", 256, 32, 256);
   static const int cars_threads = env_int("PP_CARS_THREADS", 0, 0, 1024);
   const CarsGeom cg = cars_geom(mc, *in, cars_items);

@@ -14,71 +14,6 @@
 #include "pp_device.cuh"
 #include "pp_internal.h"
 
-struct pp_rollouts {
-  const pp_map *map = nullptr;
-  int64_t n = 0;   // rollouts
-  int32_t c = 0;   // cars per rollout
-  uint64_t seed = 0;
-  int64_t first = 0;
-  int64_t tick = 0;
-  char *buf = nullptr;  // one device allocation
-  // simulator state
-  double *ego_x, *ego_y, *ego_yaw, *ego_mph, *car_ratio, *car_speed;
-  int32_t *path_n, *path_off, *target_lane, *car_lane, *car_wp;
-  bool lean = false;  // plans without the per-frame diagnostics and unused per-car outputs
-  pp_plans full_pl;   // the complete set of output pointers (restored when lean is switched off)
-  // per-tick frames and plans
-  pp_frames fr;
-  pp_plans pl;
-  int64_t *stats_sum;  // running sum of the per-tick statistics over all ticks
-  // Rollouts are independent, so they are cut into kGroups ranges that tick on their own
-  // streams: one group's short kernels and side-stream tail overlap the other groups' work.
-  static constexpr int kGroups = 8;  // streams that exist; PP_ROLLOUT_GROUPS of them are used
-  cudaStream_t gs[kGroups] = {};
-  cudaEvent_t g_done[kGroups] = {};
-  cudaEvent_t fork = nullptr;
-  cudaStream_t origin = nullptr;  // graph capture / replay stream (the caller's may be the
-                                  // legacy default stream, which cannot be captured)
-  cudaEvent_t o_fork = nullptr, o_join = nullptr;
-  int64_t *tick_dev = nullptr;  // [R] ticks done per rollout (device side of `tick`)
-  char *scratch[kGroups] = {};  // the planning pipeline's scratch, one per group
-  // one tick of every group, captured once and replayed (a tick is ~50 small launches)
-  cudaGraphExec_t graph = nullptr;
-  int32_t graph_k = 0;
-  pp_config graph_cfg;
-  int64_t launches_per_tick = 0;
-  int groups_wanted = 0;  // pp_rollouts_set_groups: 0 = automatic
-  // incident monitor (pp.h, pp_rollout_incidents); device arrays in `buf`
-  double2 *inc_ring, *inc_ring_acc;
-  int64_t *inc_pts, *inc_first_tick;
-  uint32_t *inc_active;
-  int32_t *inc_off, *inc_count, *inc_first_kind;
-  double *inc_d[6];  // distance_m, clean_m, best_clean_m, max_speed, max_acc, max_jerk
-  // traffic model (pp.h, pp_rollouts_set_traffic); the IDM state has an allocation of its own,
-  // made only when that model is selected
-  int traffic = PP_TRAFFIC_CONSTANT;
-  char *trf_buf = nullptr;
-  double *trf_v0 = nullptr, *trf_acc = nullptr, *trf_cum = nullptr, *trf_ego_s = nullptr;
-  int32_t *trf_ego_lanes = nullptr;
-  // flight recorder (pp.h, pp_rollouts_set_recorder); an allocation of its own, made only when
-  // it is switched on
-  int rec_w = 0;  // window W, 0 = off
-  uint32_t rec_mask = 0;
-  char *rec_buf = nullptr;
-  double *rec_ring = nullptr;
-  int64_t *rec_trig_tick = nullptr;
-  uint32_t *rec_trig_bits = nullptr;
-  // (first tick, consume_k) of every stretch of ticks run with one consume_k.  All rollouts tick
-  // together, so the host knows each tick's k; a window frozen long ago still finds its k here.
-  std::vector<std::pair<int64_t, int32_t>> rec_k;
-  // near-miss measures (pp.h, pp_rollouts_set_surrogate); an allocation of its own, made only
-  // when they are switched on
-  char *ssm_buf = nullptr;
-  double *ssm_min = nullptr;
-  int64_t *ssm_tick = nullptr;
-  int32_t *ssm_hist = nullptr;
-};
-
 namespace {
 
 constexpr int kB = 256;
@@ -997,13 +932,194 @@ __global__ void __launch_bounds__(kB) k_rec_gather(Recorder rc, const int64_t *r
   }
 }
 
-inline size_t al(size_t v) { return (v + 255) & ~(size_t)255; }
-
 int cuda_fail(const char *what, cudaError_t e) {
   ppi::set_cuda_error(what, (int)e, cudaGetErrorString(e));
   cudaGetLastError();
   return PP_E_CUDA;
 }
+
+// Blocking copies of the getters and of pp_rollouts_create's upload.  A null destination or an
+// empty copy is skipped; after the first CUDA error nothing more is copied and `e` keeps it.
+struct Copy {
+  cudaMemcpyKind kind;
+  cudaError_t e = cudaSuccess;
+  void operator()(void *dst, const void *src, size_t bytes) {
+    if (e == cudaSuccess && dst && bytes) e = cudaMemcpy(dst, src, bytes, kind);
+  }
+  // [K][R] on the device -> [R][K] for the caller
+  template <class T>
+  void transpose(T *dst, const T *src, size_t R, size_t K) {
+    if (!dst) return;
+    std::vector<T> t(R * K);
+    (*this)(t.data(), src, R * K * sizeof(T));
+    for (size_t i = 0; i < R; i++)
+      for (size_t k = 0; k < K; k++) dst[i * K + k] = t[k * R + i];
+  }
+};
+
+}  // namespace
+
+struct pp_rollouts {
+  const pp_map *map = nullptr;
+  int64_t n = 0;   // rollouts
+  int32_t c = 0;   // cars per rollout
+  uint64_t seed = 0;
+  int64_t first = 0;
+  int64_t tick = 0;
+  // one device allocation (rollouts_layout): the simulator state, the per-tick frames and plans,
+  // the statistics and the incident monitor
+  char *buf = nullptr;
+  SimState st;
+  bool lean = false;  // plans without the per-frame diagnostics and unused per-car outputs
+  pp_plans full_pl;   // the complete set of output pointers (restored when lean is switched off)
+  // per-tick frames and plans
+  pp_frames fr;
+  pp_plans pl;
+  int64_t *stats_sum;  // running sum of the per-tick statistics over all ticks
+  // Rollouts are independent, so they are cut into kGroups ranges that tick on their own
+  // streams: one group's short kernels and side-stream tail overlap the other groups' work.
+  static constexpr int kGroups = 8;  // streams that exist; PP_ROLLOUT_GROUPS of them are used
+  cudaStream_t gs[kGroups] = {};
+  cudaEvent_t g_done[kGroups] = {};
+  cudaEvent_t fork = nullptr;
+  cudaStream_t origin = nullptr;  // graph capture / replay stream (the caller's may be the
+                                  // legacy default stream, which cannot be captured)
+  cudaEvent_t o_fork = nullptr, o_join = nullptr;
+  char *scratch[kGroups] = {};  // the planning pipeline's scratch, one per group
+  // one tick of every group, captured once and replayed (a tick is ~50 small launches)
+  cudaGraphExec_t graph = nullptr;
+  int32_t graph_k = 0;
+  pp_config graph_cfg;
+  int64_t launches_per_tick = 0;
+  int groups_wanted = 0;  // pp_rollouts_set_groups: 0 = automatic
+  Monitor mo;  // incident monitor (pp.h, pp_rollout_incidents), in `buf`
+  // Each observer below owns one allocation of its own, made only when it is switched on; its
+  // view's pointers are null until then.
+  int traffic = PP_TRAFFIC_CONSTANT;  // traffic model (pp.h, pp_rollouts_set_traffic)
+  char *tf_buf = nullptr;             // the IDM state
+  Traffic tf;
+  char *rc_buf = nullptr;  // flight recorder (pp.h, pp_rollouts_set_recorder): on while rc.W > 0
+  Recorder rc;
+  // (first tick, consume_k) of every stretch of ticks run with one consume_k.  All rollouts tick
+  // together, so the host knows each tick's k; a window frozen long ago still finds its k here.
+  std::vector<std::pair<int64_t, int32_t>> rec_k;
+  char *sg_buf = nullptr;  // near-miss measures (pp.h, pp_rollouts_set_surrogate): on while allocated
+  Surrogate sg;
+};
+
+namespace {
+
+// The layout of pp_rollouts::buf (ppi::Carve).  Plans get all outputs: tests compare them tick by
+// tick.
+size_t rollouts_layout(pp_rollouts *r, char *base) {
+  const size_t N = (size_t)r->n, NC = (size_t)r->n * (size_t)(r->c > 0 ? r->c : 1);
+  ppi::Carve cv(base);
+  SimState &s = r->st;
+  cv.take(s.ego_x, N);
+  cv.take(s.ego_y, N);
+  cv.take(s.ego_yaw, N);
+  cv.take(s.ego_mph, N);
+  cv.take(s.path_n, N);
+  cv.take(s.path_off, N);
+  cv.take(s.target_lane, N);
+  cv.take(s.car_lane, NC);
+  cv.take(s.car_wp, NC);
+  cv.take(s.car_ratio, NC);
+  cv.take(s.car_speed, NC);
+  pp_frames &f = r->fr;
+  cv.take(f.ego_x, N);
+  cv.take(f.ego_y, N);
+  cv.take(f.ego_yaw_deg, N);
+  cv.take(f.ego_speed_mph, N);
+  cv.take(f.prev_n, N);
+  cv.take(f.prev_x, N * PP_PREV_KEEP);
+  cv.take(f.prev_y, N * PP_PREV_KEEP);
+  cv.take(f.target_lane_in, N);
+  cv.take(f.n_cars, N);
+  cv.take(f.car_id, NC);
+  cv.take(f.car_x, NC);
+  cv.take(f.car_y, NC);
+  cv.take(f.car_vx, NC);
+  cv.take(f.car_vy, NC);
+  pp_plans &p = r->pl;
+  cv.take(p.next_x, N * PP_PATH_LEN);
+  cv.take(p.next_y, N * PP_PATH_LEN);
+  cv.take(p.n_points, N);
+  cv.take(p.ego_lane, N);
+  cv.take(p.ref_wp, N);
+  cv.take(p.target_lane, N);
+  cv.take(p.flags, N);
+  cv.take(p.ego_s, N);
+  cv.take(p.ego_d, N);
+  cv.take(p.ego_vs, N);
+  cv.take(p.ego_vd, N);
+  cv.take(p.ego_speed, N);
+  cv.take(p.ego_acc, N);
+  cv.take(p.target_speed, N);
+  cv.take(p.target_time, N);
+  cv.take(p.next_car_id, N);
+  cv.take(p.next_car_in_target_lane, N);
+  cv.take(p.car_s, NC);
+  cv.take(p.car_d, NC);
+  cv.take(p.car_vs, NC);
+  cv.take(p.car_vd, NC);
+  cv.take(p.car_lane, NC);
+  cv.take(p.car_next_wp, NC);
+  cv.take(r->stats_sum, PP_STATS_LEN);
+  cv.take(s.ticks, N);
+  Monitor &m = r->mo;
+  cv.take(m.ring, N * PP_INC_HISTORY);
+  cv.take(m.ring_acc, N * PP_INC_HISTORY);
+  cv.take(m.pts, N);
+  cv.take(m.first_tick, N);
+  cv.take(m.active, N);
+  cv.take(m.off_pts, N);
+  cv.take(m.count, N * PP_INC_KINDS);
+  cv.take(m.first_kind, N);
+  for (double **d : {&m.dist, &m.clean, &m.best, &m.vmax, &m.amax, &m.jmax}) cv.take(*d, N);
+  return cv.size;
+}
+
+// An observer's own block for `layout`, a ppi::Carve layout that binds the observer's view and
+// returns its size.  The block stays null when the allocation fails.
+template <class Layout>
+cudaError_t observer_alloc(char *&block, Layout layout) {
+  const cudaError_t e = cudaMalloc((void **)&block, layout(nullptr));
+  if (e != cudaSuccess) {
+    block = nullptr;
+    return e;
+  }
+  layout(block);
+  return cudaSuccess;
+}
+
+// Frees an observer's block; its layout run without a base leaves the view's pointers null.
+template <class Layout>
+void observer_free(char *&block, Layout layout) {
+  cudaFree(block);
+  block = nullptr;
+  layout(nullptr);
+}
+
+// The totals entry points: zero `len` totals on the caller's stream, then `kernel` adds every
+// rollout's record into them.
+template <class View>
+int record_totals(const pp_rollouts *r, const char *who, void (*kernel)(View, unsigned long long *),
+                  const char *kernel_name, const View &view, int len, int64_t *totals_dev,
+                  void *cuda_stream) {
+  const int rc = ppi::check_map_device(r->map, who);
+  if (rc != PP_OK) return rc;
+  cudaStream_t st = (cudaStream_t)cuda_stream;
+  cudaError_t e = cudaMemsetAsync(totals_dev, 0, len * sizeof(int64_t), st);
+  if (e != cudaSuccess) return cuda_fail(who, e);
+  const int64_t blocks = (r->n + kB - 1) / kB;
+  kernel<<<(int)(blocks < 1184 ? blocks : 1184), kB, 0, st>>>(view, (unsigned long long *)totals_dev);
+  ppi::count_launch(1);
+  e = cudaGetLastError();
+  if (e != cudaSuccess) return cuda_fail(kernel_name, e);
+  return PP_OK;
+}
+
 
 }  // namespace
 
@@ -1024,110 +1140,24 @@ extern "C" int pp_rollouts_create(const pp_map *map, int64_t n, int32_t c, uint6
   r->seed = seed;
   r->first = first;
   const size_t N = (size_t)n, NC = (size_t)n * (size_t)(c > 0 ? c : 1);
-  // carve one allocation
-  size_t off = 0;
-  auto take = [&](size_t bytes) {
-    const size_t o = off;
-    off += al(bytes);
-    return o;
-  };
-  const size_t o_ex = take(N * 8), o_ey = take(N * 8), o_yaw = take(N * 8), o_mph = take(N * 8);
-  const size_t o_pn = take(N * 4), o_po = take(N * 4);
-  const size_t o_tl = take(N * 4), o_cl = take(NC * 4), o_cw = take(NC * 4), o_cr = take(NC * 8),
-               o_cs = take(NC * 8);
-  // frames
-  const size_t f_ex = take(N * 8), f_ey = take(N * 8), f_yaw = take(N * 8), f_mph = take(N * 8),
-               f_pn = take(N * 4), f_px = take(N * PP_PREV_KEEP * 8), f_py = take(N * PP_PREV_KEEP * 8),
-               f_tl = take(N * 4), f_nc = take(N * 4), f_id = take(NC * 4), f_cx = take(NC * 8),
-               f_cy = take(NC * 8), f_vx = take(NC * 8), f_vy = take(NC * 8);
-  // plans (all outputs: tests compare them tick by tick)
-  const size_t p_nx = take(N * PP_PATH_LEN * 8), p_ny = take(N * PP_PATH_LEN * 8), p_np = take(N * 4),
-               p_el = take(N * 4), p_rw = take(N * 4), p_tl = take(N * 4), p_fl = take(N * 4);
-  size_t p_d[8];
-  for (int i = 0; i < 8; i++) p_d[i] = take(N * 8);
-  const size_t p_i0 = take(N * 4), p_i1 = take(N * 4);
-  const size_t p_cs = take(NC * 8), p_cd = take(NC * 8), p_cvs = take(NC * 8), p_cvd = take(NC * 8),
-               p_cl = take(NC * 4), p_cw = take(NC * 4);
-  const size_t o_ss = take(PP_STATS_LEN * 8);
-  const size_t o_tk = take(N * 8);
-  // incident monitor
-  const size_t m_ring = take(N * PP_INC_HISTORY * 16), m_racc = take(N * PP_INC_HISTORY * 16), m_pts = take(N * 8), m_ft = take(N * 8),
-               m_act = take(N * 4), m_off = take(N * 4), m_cnt = take(N * PP_INC_KINDS * 4),
-               m_fk = take(N * 4);
-  size_t m_d[6];
-  for (int i = 0; i < 6; i++) m_d[i] = take(N * 8);
-  cudaError_t e = cudaMalloc((void **)&r->buf, off);
+  const size_t bytes = rollouts_layout(r, nullptr);
+  cudaError_t e = cudaMalloc((void **)&r->buf, bytes);
   if (e != cudaSuccess) {
     delete r;
     return cuda_fail("cudaMalloc(rollouts)", e);
   }
-  cudaMemset(r->buf, 0, off);
-  char *b = r->buf;
-  r->ego_x = (double *)(b + o_ex);
-  r->ego_y = (double *)(b + o_ey);
-  r->ego_yaw = (double *)(b + o_yaw);
-  r->ego_mph = (double *)(b + o_mph);
-  r->path_n = (int32_t *)(b + o_pn);
-  r->path_off = (int32_t *)(b + o_po);
-  r->target_lane = (int32_t *)(b + o_tl);
-  r->car_lane = (int32_t *)(b + o_cl);
-  r->car_wp = (int32_t *)(b + o_cw);
-  r->car_ratio = (double *)(b + o_cr);
-  r->car_speed = (double *)(b + o_cs);
-  pp_frames &f = r->fr;
-  f.ego_x = (double *)(b + f_ex);
-  f.ego_y = (double *)(b + f_ey);
-  f.ego_yaw_deg = (double *)(b + f_yaw);
-  f.ego_speed_mph = (double *)(b + f_mph);
-  f.prev_n = (int32_t *)(b + f_pn);
-  f.prev_x = (double *)(b + f_px);
-  f.prev_y = (double *)(b + f_py);
-  f.target_lane_in = (int32_t *)(b + f_tl);
-  f.n_cars = (int32_t *)(b + f_nc);
-  f.car_id = (int32_t *)(b + f_id);
-  f.car_x = (double *)(b + f_cx);
-  f.car_y = (double *)(b + f_cy);
-  f.car_vx = (double *)(b + f_vx);
-  f.car_vy = (double *)(b + f_vy);
-  f.max_cars = c > 0 ? c : 1;
-  f.reserved = 0;
-  pp_plans &p = r->pl;
-  p.next_x = (double *)(b + p_nx);
-  p.next_y = (double *)(b + p_ny);
-  p.n_points = (int32_t *)(b + p_np);
-  p.ego_lane = (int32_t *)(b + p_el);
-  p.ref_wp = (int32_t *)(b + p_rw);
-  p.target_lane = (int32_t *)(b + p_tl);
-  p.flags = (uint32_t *)(b + p_fl);
-  p.ego_s = (double *)(b + p_d[0]);
-  p.ego_d = (double *)(b + p_d[1]);
-  p.ego_vs = (double *)(b + p_d[2]);
-  p.ego_vd = (double *)(b + p_d[3]);
-  p.ego_speed = (double *)(b + p_d[4]);
-  p.ego_acc = (double *)(b + p_d[5]);
-  p.target_speed = (double *)(b + p_d[6]);
-  p.target_time = (double *)(b + p_d[7]);
-  p.next_car_id = (int32_t *)(b + p_i0);
-  p.next_car_in_target_lane = (int32_t *)(b + p_i1);
-  p.car_s = (double *)(b + p_cs);
-  p.car_d = (double *)(b + p_cd);
-  p.car_vs = (double *)(b + p_cvs);
-  p.car_vd = (double *)(b + p_cvd);
-  p.car_lane = (int32_t *)(b + p_cl);
-  p.car_next_wp = (int32_t *)(b + p_cw);
-  r->stats_sum = (int64_t *)(b + o_ss);
-  r->tick_dev = (int64_t *)(b + o_tk);
-  r->inc_ring = (double2 *)(b + m_ring);
-  r->inc_ring_acc = (double2 *)(b + m_racc);
-  r->inc_pts = (int64_t *)(b + m_pts);
-  r->inc_first_tick = (int64_t *)(b + m_ft);
-  r->inc_active = (uint32_t *)(b + m_act);
-  r->inc_off = (int32_t *)(b + m_off);
-  r->inc_count = (int32_t *)(b + m_cnt);
-  r->inc_first_kind = (int32_t *)(b + m_fk);
-  for (int i = 0; i < 6; i++) r->inc_d[i] = (double *)(b + m_d[i]);
-  cudaMemset(r->inc_first_tick, 0xff, N * 8);  // -1: no incident yet
-  cudaMemset(r->inc_first_kind, 0xff, N * 4);
+  cudaMemset(r->buf, 0, bytes);
+  rollouts_layout(r, r->buf);
+  r->fr.max_cars = c > 0 ? c : 1;
+  r->fr.reserved = 0;
+  r->mo.ego0_x = r->fr.ego_x;
+  r->mo.ego0_y = r->fr.ego_y;
+  r->mo.R = n;
+  r->tf = Traffic{nullptr, nullptr, nullptr, nullptr, nullptr, r->fr.ego_speed_mph, n};
+  r->rc = Recorder{nullptr, nullptr, nullptr, n, c, 0, 0};
+  r->sg = Surrogate{nullptr, nullptr, nullptr, n};
+  cudaMemset(r->mo.first_tick, 0xff, N * 8);  // -1: no incident yet
+  cudaMemset(r->mo.first_kind, 0xff, N * 4);
 
   // ---- initial state on the host: a pure function of (seed, first + r)
   std::vector<double> ex(N), ey(N), yaw(N), mph(N), cr(NC), cs(NC);
@@ -1163,35 +1193,32 @@ extern "C" int pp_rollouts_create(const pp_map *map, int64_t n, int32_t c, uint6
       cs[i * c + j] = sp;
     }
   }
-  bool ok = true;
-  auto up = [&](void *dst, const void *src, size_t bytes) {
-    if (bytes && cudaMemcpy(dst, src, bytes, cudaMemcpyHostToDevice) != cudaSuccess) ok = false;
-  };
-  up(r->ego_x, ex.data(), N * 8);
-  up(r->ego_y, ey.data(), N * 8);
-  up(r->ego_yaw, yaw.data(), N * 8);
-  up(r->ego_mph, mph.data(), N * 8);
-  up(r->target_lane, tl.data(), N * 4);
+  Copy up{cudaMemcpyHostToDevice};
+  up(r->st.ego_x, ex.data(), N * 8);
+  up(r->st.ego_y, ey.data(), N * 8);
+  up(r->st.ego_yaw, yaw.data(), N * 8);
+  up(r->st.ego_mph, mph.data(), N * 8);
+  up(r->st.target_lane, tl.data(), N * 4);
   {  // D_0, the initial pose, in row 0 of the monitor's history
     std::vector<double> d0(2 * N);
     for (size_t i = 0; i < N; i++) {
       d0[2 * i] = ex[i];
       d0[2 * i + 1] = ey[i];
     }
-    up(r->inc_ring, d0.data(), N * 16);
+    up(r->mo.ring, d0.data(), N * 16);
   }
   if (c > 0) {
-    up(r->car_lane, cl.data(), NC * 4);
-    up(r->car_wp, cw.data(), NC * 4);
-    up(r->car_ratio, cr.data(), NC * 8);
-    up(r->car_speed, cs.data(), NC * 8);
+    up(r->st.car_lane, cl.data(), NC * 4);
+    up(r->st.car_wp, cw.data(), NC * 4);
+    up(r->st.car_ratio, cr.data(), NC * 8);
+    up(r->st.car_speed, cs.data(), NC * 8);
   }
-  if (!ok) {
-    cudaError_t e2 = cudaGetLastError();
+  if (up.e != cudaSuccess) {
     cudaFree(r->buf);
     delete r;
-    return cuda_fail("cudaMemcpy(rollouts init)", e2);
+    return cuda_fail("cudaMemcpy(rollouts init)", up.e);
   }
+  bool ok = true;
   for (int g = 0; g < pp_rollouts::kGroups; g++) {
     if (cudaStreamCreateWithFlags(&r->gs[g], cudaStreamNonBlocking) != cudaSuccess ||
         cudaEventCreateWithFlags(&r->g_done[g], cudaEventDisableTiming) != cudaSuccess)
@@ -1224,26 +1251,13 @@ extern "C" void pp_rollouts_destroy(pp_rollouts *r) {
   if (r->o_fork) cudaEventDestroy(r->o_fork);
   if (r->o_join) cudaEventDestroy(r->o_join);
   if (r->buf) cudaFree(r->buf);
-  if (r->trf_buf) cudaFree(r->trf_buf);
-  if (r->rec_buf) cudaFree(r->rec_buf);
-  if (r->ssm_buf) cudaFree(r->ssm_buf);
+  if (r->tf_buf) cudaFree(r->tf_buf);
+  if (r->rc_buf) cudaFree(r->rc_buf);
+  if (r->sg_buf) cudaFree(r->sg_buf);
   delete r;
 }
 
 namespace {
-
-Traffic traffic_view(const pp_rollouts *r) {
-  return Traffic{r->trf_v0, r->trf_acc, r->trf_cum, r->trf_ego_lanes, r->trf_ego_s,
-                 r->fr.ego_speed_mph, r->n};
-}
-
-Recorder recorder_view(const pp_rollouts *r) {
-  return Recorder{r->rec_ring, r->rec_trig_tick, r->rec_trig_bits, r->n, r->c, r->rec_w, r->rec_mask};
-}
-
-Surrogate surrogate_view(const pp_rollouts *r) {
-  return Surrogate{r->ssm_min, r->ssm_tick, r->ssm_hist, r->n};
-}
 
 // The k_sim_advance instantiation for (traffic model, recorder on, near-miss measures on).
 template <int kTraffic>
@@ -1294,33 +1308,27 @@ int issue_tick(pp_rollouts *r, const pp_config *cfg, int32_t consume_k, cudaStre
     const int grid = (int)((cnt + kR - 1) / kR);
     const pp_frames fr = ppi::offset_frames(r->fr, lo);
     const pp_plans pl = ppi::offset_plans(r->pl, lo, mc);
-    const SimState sst{r->ego_x, r->ego_y, r->ego_yaw, r->ego_mph, r->path_n, r->path_off,
-                       r->target_lane, r->car_lane, r->car_wp, r->car_ratio, r->car_speed, r->tick_dev};
-    const Recorder rec = recorder_view(r);
-    if (r->rec_w)
-      k_sim_frames<true><<<grid, kB, 0, gs>>>(trk, lo, cnt, r->c, sst, r->pl, r->fr, rec);
+    const bool rec = r->rc.W != 0;
+    if (rec)
+      k_sim_frames<true><<<grid, kB, 0, gs>>>(trk, lo, cnt, r->c, r->st, r->pl, r->fr, r->rc);
     else
-      k_sim_frames<false><<<grid, kB, 0, gs>>>(trk, lo, cnt, r->c, sst, r->pl, r->fr, rec);
+      k_sim_frames<false><<<grid, kB, 0, gs>>>(trk, lo, cnt, r->c, r->st, r->pl, r->fr, r->rc);
     if (!r->scratch[g]) {
       const size_t need = ppi::plan_scratch_bytes(per, mc);
       if (need && cudaMalloc((void **)&r->scratch[g], need) != cudaSuccess)
         return cuda_fail("cudaMalloc(rollout scratch)", cudaGetLastError());
     }
-    const Monitor mo{r->inc_ring, r->inc_ring_acc, r->inc_pts, r->inc_active, r->inc_off, r->inc_count,
-                     r->inc_first_tick, r->inc_first_kind, r->inc_d[0], r->inc_d[1], r->inc_d[2],
-                     r->inc_d[3], r->inc_d[4], r->inc_d[5], r->fr.ego_x, r->fr.ego_y, r->n};
     const bool plan_sums = ppi::plan_adds_checksum(cnt);
     int rc = ppi::plan_batch_scratch(r->map, cfg, &fr, &pl, cnt, gs, r->scratch[g], nullptr,
                                      (unsigned long long *)r->stats_sum + PP_STAT_XSUM);
     if (rc != PP_OK) return rc;
-    const Traffic tf = traffic_view(r);
     const bool idm = r->traffic == PP_TRAFFIC_IDM;
-    const bool ssm = r->ssm_buf != nullptr;
-    auto *advance = idm ? advance_kernel<PP_TRAFFIC_IDM>(r->rec_w != 0, ssm)
-                        : advance_kernel<PP_TRAFFIC_CONSTANT>(r->rec_w != 0, ssm);
+    const bool ssm = r->sg_buf != nullptr;
+    auto *advance = idm ? advance_kernel<PP_TRAFFIC_IDM>(rec, ssm)
+                        : advance_kernel<PP_TRAFFIC_CONSTANT>(rec, ssm);
     advance<<<grid, kB, idm ? traffic_smem_bytes(r->c) : 0, gs>>>(
-        trk, lo, cnt, r->c, r->seed, r->first, consume_k, sst, r->pl,
-        (unsigned long long *)r->stats_sum, plan_sums ? 0 : 1, mo, tf, rec, surrogate_view(r));
+        trk, lo, cnt, r->c, r->seed, r->first, consume_k, r->st, r->pl,
+        (unsigned long long *)r->stats_sum, plan_sums ? 0 : 1, r->mo, r->tf, r->rc, r->sg);
     ppi::count_launch(2);
   }
   r->launches_per_tick = pp_launch_count() - launches0;
@@ -1356,7 +1364,7 @@ extern "C" int pp_rollouts_run(pp_rollouts *r, const pp_config *cfg, int64_t n_t
     const int rc = ppi::check_map_device(r->map, "pp_rollouts_run");
     if (rc != PP_OK) return rc;
   }
-  if (r->rec_w && (r->rec_k.empty() || r->rec_k.back().second != consume_k))
+  if (r->rc.W && (r->rec_k.empty() || r->rec_k.back().second != consume_k))
     r->rec_k.emplace_back(r->tick, consume_k);
   // A tick is ~36 short launches over 8 streams (4 groups, each with its side stream).  It can
   // be captured once and replayed as a CUDA graph (PP_ROLLOUT_GRAPH=1; the pipeline's scratch is
@@ -1462,20 +1470,18 @@ extern "C" int pp_rollouts_get_state(const pp_rollouts *r, pp_rollout_state *h) 
   cudaError_t e = cudaDeviceSynchronize();
   if (e != cudaSuccess) return cuda_fail("pp_rollouts_get_state", e);
   const size_t N = (size_t)r->n, NC = (size_t)r->n * (size_t)r->c;
-  bool ok = true;
-  auto dn = [&](void *dst, const void *src, size_t bytes) {
-    if (dst && bytes && cudaMemcpy(dst, src, bytes, cudaMemcpyDeviceToHost) != cudaSuccess) ok = false;
-  };
-  dn(h->ego_x, r->ego_x, N * 8);
-  dn(h->ego_y, r->ego_y, N * 8);
-  dn(h->ego_yaw_deg, r->ego_yaw, N * 8);
-  dn(h->ego_speed_mph, r->ego_mph, N * 8);
-  dn(h->path_n, r->path_n, N * 4);
+  const SimState &s = r->st;
+  Copy dn{cudaMemcpyDeviceToHost};
+  dn(h->ego_x, s.ego_x, N * 8);
+  dn(h->ego_y, s.ego_y, N * 8);
+  dn(h->ego_yaw_deg, s.ego_yaw, N * 8);
+  dn(h->ego_speed_mph, s.ego_mph, N * 8);
+  dn(h->path_n, s.path_n, N * 4);
   if (h->path_x || h->path_y) {  // the unconsumed points live in the plan buffer at path_off
     std::vector<int32_t> pn(N), po(N);
     std::vector<double> buf(N * PP_PATH_LEN);
-    dn(pn.data(), r->path_n, N * 4);
-    dn(po.data(), r->path_off, N * 4);
+    dn(pn.data(), s.path_n, N * 4);
+    dn(po.data(), s.path_off, N * 4);
     for (int axis = 0; axis < 2; axis++) {
       double *dst = axis ? h->path_y : h->path_x;
       if (!dst) continue;
@@ -1485,13 +1491,13 @@ extern "C" int pp_rollouts_get_state(const pp_rollouts *r, pp_rollout_state *h) 
           dst[i * PP_PATH_LEN + k] = k < pn[i] ? buf[i * PP_PATH_LEN + po[i] + k] : 0.0;
     }
   }
-  dn(h->target_lane, r->target_lane, N * 4);
-  dn(h->car_lane, r->car_lane, NC * 4);
-  dn(h->car_wp, r->car_wp, NC * 4);
-  dn(h->car_ratio, r->car_ratio, NC * 8);
-  dn(h->car_speed, r->car_speed, NC * 8);
+  dn(h->target_lane, s.target_lane, N * 4);
+  dn(h->car_lane, s.car_lane, NC * 4);
+  dn(h->car_wp, s.car_wp, NC * 4);
+  dn(h->car_ratio, s.car_ratio, NC * 8);
+  dn(h->car_speed, s.car_speed, NC * 8);
   h->tick = r->tick;
-  if (!ok) return cuda_fail("pp_rollouts_get_state copy", cudaGetLastError());
+  if (dn.e != cudaSuccess) return cuda_fail("pp_rollouts_get_state copy", dn.e);
   return PP_OK;
 }
 
@@ -1514,23 +1520,21 @@ extern "C" int pp_rollouts_set_traffic(pp_rollouts *r, int model) {
   }
   const int nw = r->map->n;
   const size_t N = (size_t)r->n, NC = (size_t)r->n * (size_t)r->c;
-  if (!r->trf_buf) {
-    const size_t bytes = al(NC * 8) * 2 + al(3 * (size_t)(nw + 1) * 8) + al(2 * N * 4) + al(6 * N * 8);
-    cudaError_t e = cudaMalloc((void **)&r->trf_buf, bytes);
+  Traffic &tf = r->tf;
+  if (!r->tf_buf) {
+    cudaError_t e = observer_alloc(r->tf_buf, [&](char *base) {
+      ppi::Carve cv(base);
+      cv.take(tf.v0, NC);
+      cv.take(tf.acc, NC);
+      cv.take(tf.cum, 3 * (size_t)(nw + 1));
+      cv.take(tf.ego_lanes, 2 * N);
+      cv.take(tf.ego_s, 6 * N);
+      return cv.size;
+    });
     if (e != cudaSuccess) {
       r->traffic = PP_TRAFFIC_CONSTANT;
       return cuda_fail("cudaMalloc(rollout traffic)", e);
     }
-    char *b = r->trf_buf;
-    r->trf_v0 = (double *)b;
-    b += al(NC * 8);
-    r->trf_acc = (double *)b;
-    b += al(NC * 8);
-    r->trf_cum = (double *)b;
-    b += al(3 * (size_t)(nw + 1) * 8);
-    r->trf_ego_lanes = (int32_t *)b;
-    b += al(2 * N * 4);
-    r->trf_ego_s = (double *)b;
   }
   // cum(L, w), summed on the host in ascending w
   std::vector<double> cum(3 * (size_t)(nw + 1));
@@ -1542,16 +1546,15 @@ extern "C" int pp_rollouts_set_traffic(pp_rollouts *r, int model) {
       cum[(size_t)L * (nw + 1) + w + 1] = acc;
     }
   }
-  cudaError_t e = cudaMemcpy(r->trf_cum, cum.data(), cum.size() * 8, cudaMemcpyHostToDevice);
-  if (e == cudaSuccess && NC)
-    e = cudaMemcpy(r->trf_v0, r->car_speed, NC * 8, cudaMemcpyDeviceToDevice);
-  if (e == cudaSuccess && NC) e = cudaMemset(r->trf_acc, 0, NC * 8);
+  cudaError_t e = cudaMemcpy((double *)tf.cum, cum.data(), cum.size() * 8, cudaMemcpyHostToDevice);
+  if (e == cudaSuccess && NC) e = cudaMemcpy(tf.v0, r->st.car_speed, NC * 8, cudaMemcpyDeviceToDevice);
+  if (e == cudaSuccess && NC) e = cudaMemset(tf.acc, 0, NC * 8);
   if (e != cudaSuccess) {
     r->traffic = PP_TRAFFIC_CONSTANT;
     return cuda_fail("pp_rollouts_set_traffic", e);
   }
   const Track trk{r->map->dev_table + (size_t)PPD_PAD_ROWS * PP_MAP_STRIDE, nw, PP_MAP_STRIDE};
-  k_traffic_init<<<(int)((r->n + kB - 1) / kB), kB>>>(trk, r->ego_x, r->ego_y, traffic_view(r));
+  k_traffic_init<<<(int)((r->n + kB - 1) / kB), kB>>>(trk, r->st.ego_x, r->st.ego_y, tf);
   ppi::count_launch(1);
   e = cudaDeviceSynchronize();
   if (e == cudaSuccess) e = cudaGetLastError();
@@ -1568,20 +1571,12 @@ extern "C" int pp_rollouts_get_traffic(const pp_rollouts *r, pp_rollout_traffic 
   if (e != cudaSuccess) return cuda_fail("pp_rollouts_get_traffic", e);
   const size_t N = (size_t)r->n, NC = (size_t)r->n * (size_t)r->c;
   const int buf = (int)(r->tick & 1);  // the copy the next tick reads
-  bool ok = true;
-  auto dn = [&](void *dst, const void *src, size_t bytes) {
-    if (dst && bytes && cudaMemcpy(dst, src, bytes, cudaMemcpyDeviceToHost) != cudaSuccess) ok = false;
-  };
-  dn(h->car_v0, r->trf_v0, NC * 8);
-  dn(h->car_acc, r->trf_acc, NC * 8);
-  dn(h->ego_lanes, r->trf_ego_lanes + buf * N, N * 4);
-  if (h->ego_s) {  // [L][R] on the device, [R][L] for the caller
-    std::vector<double> s(3 * N);
-    dn(s.data(), r->trf_ego_s + buf * 3 * N, 3 * N * 8);
-    for (size_t i = 0; i < N; i++)
-      for (int L = 0; L < 3; L++) h->ego_s[i * 3 + L] = s[L * N + i];
-  }
-  if (!ok) return cuda_fail("pp_rollouts_get_traffic copy", cudaGetLastError());
+  Copy dn{cudaMemcpyDeviceToHost};
+  dn(h->car_v0, r->tf.v0, NC * 8);
+  dn(h->car_acc, r->tf.acc, NC * 8);
+  dn(h->ego_lanes, r->tf.ego_lanes + buf * N, N * 4);
+  dn.transpose(h->ego_s, r->tf.ego_s + buf * 3 * N, N, 3);
+  if (dn.e != cudaSuccess) return cuda_fail("pp_rollouts_get_traffic copy", dn.e);
   return PP_OK;
 }
 
@@ -1590,84 +1585,62 @@ extern "C" int pp_rollouts_get_incidents(const pp_rollouts *r, pp_rollout_incide
   cudaError_t e = cudaDeviceSynchronize();
   if (e != cudaSuccess) return cuda_fail("pp_rollouts_get_incidents", e);
   const size_t N = (size_t)r->n;
-  bool ok = true;
-  auto dn = [&](void *dst, const void *src, size_t bytes) {
-    if (dst && cudaMemcpy(dst, src, bytes, cudaMemcpyDeviceToHost) != cudaSuccess) ok = false;
-  };
-  if (h->count) {  // [kind][R] on the device, [R][kind] for the caller
-    std::vector<int32_t> cnt(N * PP_INC_KINDS);
-    dn(cnt.data(), r->inc_count, N * PP_INC_KINDS * 4);
-    for (size_t i = 0; i < N; i++)
-      for (int k = 0; k < PP_INC_KINDS; k++) h->count[i * PP_INC_KINDS + k] = cnt[k * N + i];
-  }
-  dn(h->first_tick, r->inc_first_tick, N * 8);
-  dn(h->first_kind, r->inc_first_kind, N * 4);
-  double *const outs[6] = {h->distance_m, h->clean_m, h->best_clean_m, h->max_speed, h->max_acc,
-                           h->max_jerk};
-  for (int i = 0; i < 6; i++) dn(outs[i], r->inc_d[i], N * 8);
-  if (!ok) return cuda_fail("pp_rollouts_get_incidents copy", cudaGetLastError());
+  const Monitor &mo = r->mo;
+  Copy dn{cudaMemcpyDeviceToHost};
+  dn.transpose(h->count, mo.count, N, PP_INC_KINDS);
+  dn(h->first_tick, mo.first_tick, N * 8);
+  dn(h->first_kind, mo.first_kind, N * 4);
+  dn(h->distance_m, mo.dist, N * 8);
+  dn(h->clean_m, mo.clean, N * 8);
+  dn(h->best_clean_m, mo.best, N * 8);
+  dn(h->max_speed, mo.vmax, N * 8);
+  dn(h->max_acc, mo.amax, N * 8);
+  dn(h->max_jerk, mo.jmax, N * 8);
+  if (dn.e != cudaSuccess) return cuda_fail("pp_rollouts_get_incidents copy", dn.e);
   return PP_OK;
 }
 
 extern "C" int pp_rollouts_incident_totals(const pp_rollouts *r, int64_t *totals_dev,
                                            void *cuda_stream) {
   if (!r || !totals_dev) return PP_E_ARG;
-  {
-    const int rc = ppi::check_map_device(r->map, "pp_rollouts_incident_totals");
-    if (rc != PP_OK) return rc;
-  }
-  cudaStream_t st = (cudaStream_t)cuda_stream;
-  cudaError_t e = cudaMemsetAsync(totals_dev, 0, PP_INC_TOTALS_LEN * sizeof(int64_t), st);
-  if (e != cudaSuccess) return cuda_fail("pp_rollouts_incident_totals", e);
-  const Monitor mo{r->inc_ring, r->inc_ring_acc, r->inc_pts, r->inc_active, r->inc_off, r->inc_count,
-                   r->inc_first_tick, r->inc_first_kind, r->inc_d[0], r->inc_d[1], r->inc_d[2],
-                   r->inc_d[3], r->inc_d[4], r->inc_d[5], r->fr.ego_x, r->fr.ego_y, r->n};
-  const int64_t blocks = (r->n + kB - 1) / kB;
-  k_incident_totals<<<(int)(blocks < 1184 ? blocks : 1184), kB, 0, st>>>(
-      mo, (unsigned long long *)totals_dev);
-  ppi::count_launch(1);
-  e = cudaGetLastError();
-  if (e != cudaSuccess) return cuda_fail("k_incident_totals", e);
-  return PP_OK;
+  return record_totals(r, "pp_rollouts_incident_totals", k_incident_totals, "k_incident_totals",
+                       r->mo, PP_INC_TOTALS_LEN, totals_dev, cuda_stream);
 }
 
 extern "C" int pp_rollouts_set_recorder(pp_rollouts *r, int32_t window, uint32_t triggers) {
   if (!r || r->tick != 0 || window < 0 || window > PP_REC_MAX_WINDOW ||
       (triggers >> (PP_REC_NONFINITE + 1)) != 0)
     return PP_E_ARG;
-  if (r->rec_buf) {
-    cudaFree(r->rec_buf);
-    r->rec_buf = nullptr;
-  }
-  r->rec_w = 0;
-  r->rec_mask = 0;
+  const size_t N = (size_t)r->n;
+  Recorder &rc = r->rc;
+  auto layout = [&](char *base) {
+    ppi::Carve cv(base);
+    cv.take(rc.ring, (size_t)window * (size_t)rc.slot_words());
+    cv.take(rc.trig_tick, N);
+    cv.take(rc.trig_bits, N);
+    return cv.size;
+  };
+  observer_free(r->rc_buf, layout);
+  rc.W = 0;
+  rc.mask = 0;
   r->rec_k.clear();
   if (window == 0) return PP_OK;
-  const size_t N = (size_t)r->n;
-  const size_t ring = N * (size_t)window * (size_t)(200 + 32 * r->c);
-  cudaError_t e = cudaMalloc((void **)&r->rec_buf, al(ring) + al(N * 8) + al(N * 4));
+  cudaError_t e = observer_alloc(r->rc_buf, layout);
+  if (e != cudaSuccess) return cuda_fail("cudaMalloc(rollout recorder)", e);
+  e = cudaMemset(rc.trig_tick, 0xff, N * 8);  // -1: recording
+  if (e == cudaSuccess) e = cudaMemset(rc.trig_bits, 0, N * 4);
   if (e != cudaSuccess) {
-    r->rec_buf = nullptr;
-    return cuda_fail("cudaMalloc(rollout recorder)", e);
-  }
-  r->rec_ring = (double *)r->rec_buf;
-  r->rec_trig_tick = (int64_t *)(r->rec_buf + al(ring));
-  r->rec_trig_bits = (uint32_t *)(r->rec_buf + al(ring) + al(N * 8));
-  e = cudaMemset(r->rec_trig_tick, 0xff, N * 8);  // -1: recording
-  if (e == cudaSuccess) e = cudaMemset(r->rec_trig_bits, 0, N * 4);
-  if (e != cudaSuccess) {
-    cudaFree(r->rec_buf);
-    r->rec_buf = nullptr;
+    observer_free(r->rc_buf, layout);
     return cuda_fail("pp_rollouts_set_recorder", e);
   }
-  r->rec_w = window;
-  r->rec_mask = triggers;
+  rc.W = window;
+  rc.mask = triggers;
   return PP_OK;
 }
 
 extern "C" int pp_rollouts_get_recording(const pp_rollouts *r, const int64_t *rollouts, int64_t m,
                                          pp_rollout_recording *h) {
-  if (!r || !h || !r->rec_w || m < 0 || (!rollouts && m != r->n)) return PP_E_ARG;
+  if (!r || !h || !r->rc.W || m < 0 || (!rollouts && m != r->n)) return PP_E_ARG;
   for (int64_t i = 0; rollouts && i < m; i++)
     if (rollouts[i] < 0 || rollouts[i] >= r->n) return PP_E_ARG;
   if (m == 0) return PP_OK;
@@ -1677,7 +1650,7 @@ extern "C" int pp_rollouts_get_recording(const pp_rollouts *r, const int64_t *ro
   }
   cudaError_t e = cudaDeviceSynchronize();
   if (e != cudaSuccess) return cuda_fail("pp_rollouts_get_recording", e);
-  const int W = r->rec_w, c = r->c;
+  const int W = r->rc.W, c = r->c;
   const size_t M = (size_t)m, MW = M * (size_t)W, MWC = MW * (size_t)c;
   double *const dst_d[10] = {h->ego_x, h->ego_y, h->ego_yaw_deg, h->ego_speed_mph, h->prev_x,
                              h->prev_y, h->car_x, h->car_y, h->car_vx, h->car_vy};
@@ -1686,47 +1659,39 @@ extern "C" int pp_rollouts_get_recording(const pp_rollouts *r, const int64_t *ro
   bool frames = dst_i[0] || dst_i[1];
   for (int f = 0; f < 10; f++) frames = frames || dst_d[f];
   // staging: the rows, the trigger arrays, then (frames only) every frame field
-  size_t off = 0;
-  auto take = [&](size_t bytes) {
-    const size_t o = off;
-    off += al(bytes);
-    return o;
+  RecOut out = {};
+  int64_t *rows_dev = nullptr;
+  auto layout = [&](char *base) {
+    ppi::Carve cv(base);
+    if (rollouts) cv.take(rows_dev, M);
+    cv.take(out.trig_tick, M);
+    cv.take(out.trig_bits, M);
+    for (int f = 0; frames && f < 10; f++) cv.take(out.d[f], words_d[f]);
+    for (int f = 0; frames && f < 2; f++) cv.take(out.i[f], MW);
+    return cv.size;
   };
-  const size_t o_rows = rollouts ? take(M * 8) : 0, o_tt = take(M * 8), o_tb = take(M * 4);
-  size_t o_d[10] = {}, o_i[2] = {};
-  if (frames) {
-    for (int f = 0; f < 10; f++) o_d[f] = take(words_d[f] * 8);
-    for (int f = 0; f < 2; f++) o_i[f] = take(MW * 4);
-  }
   char *buf = nullptr;
-  e = cudaMalloc((void **)&buf, off);
+  e = cudaMalloc((void **)&buf, layout(nullptr));
   if (e != cudaSuccess) return cuda_fail("cudaMalloc(recording staging)", e);
-  RecOut out;
-  for (int f = 0; f < 10; f++) out.d[f] = (double *)(buf + o_d[f]);
-  for (int f = 0; f < 2; f++) out.i[f] = (int32_t *)(buf + o_i[f]);
-  out.trig_tick = (int64_t *)(buf + o_tt);
-  out.trig_bits = (uint32_t *)(buf + o_tb);
-  const int64_t *rows_dev = rollouts ? (const int64_t *)(buf + o_rows) : nullptr;
-  if (rollouts) e = cudaMemcpy(buf + o_rows, rollouts, M * 8, cudaMemcpyHostToDevice);
+  layout(buf);
+  if (rollouts) e = cudaMemcpy(rows_dev, rollouts, M * 8, cudaMemcpyHostToDevice);
   if (e == cudaSuccess) {
     const size_t most = frames ? (MWC > MW * PP_PREV_KEEP ? MWC : MW * PP_PREV_KEEP) : M;
     const size_t blocks = (most + kB - 1) / kB;
     const dim3 grid((unsigned)(blocks < 4096 ? (blocks ? blocks : 1) : 4096), frames ? 13 : 1);
-    k_rec_gather<<<grid, kB>>>(recorder_view(r), rows_dev, m, r->tick, out);
+    k_rec_gather<<<grid, kB>>>(r->rc, rows_dev, m, r->tick, out);
     ppi::count_launch(1);
     e = cudaGetLastError();
     if (e == cudaSuccess) e = cudaDeviceSynchronize();
   }
   std::vector<int64_t> tt(M);
-  auto dn = [&](void *dst, const void *src, size_t bytes) {
-    if (e == cudaSuccess && dst && bytes) e = cudaMemcpy(dst, src, bytes, cudaMemcpyDeviceToHost);
-  };
+  Copy dn{cudaMemcpyDeviceToHost, e};
   dn(tt.data(), out.trig_tick, M * 8);
   dn(h->trigger_bits, out.trig_bits, M * 4);
   for (int f = 0; frames && f < 10; f++) dn(dst_d[f], out.d[f], words_d[f] * 8);
   for (int f = 0; frames && f < 2; f++) dn(dst_i[f], out.i[f], MW * 4);
   cudaFree(buf);
-  if (e != cudaSuccess) return cuda_fail("pp_rollouts_get_recording copy", e);
+  if (dn.e != cudaSuccess) return cuda_fail("pp_rollouts_get_recording copy", dn.e);
   // what the host knows: each slot's tick and consume_k, and the constant frame fields
   if (h->trigger_tick) std::memcpy(h->trigger_tick, tt.data(), M * 8);
   for (size_t i = 0; i < M; i++) {
@@ -1751,74 +1716,47 @@ extern "C" int pp_rollouts_get_recording(const pp_rollouts *r, const int64_t *ro
 
 extern "C" int pp_rollouts_set_surrogate(pp_rollouts *r, int on) {
   if (!r || r->tick != 0) return PP_E_ARG;
-  if (r->ssm_buf) {
-    cudaFree(r->ssm_buf);
-    r->ssm_buf = nullptr;
-    r->ssm_min = nullptr;
-    r->ssm_tick = nullptr;
-    r->ssm_hist = nullptr;
-  }
-  if (!on) return PP_OK;
   const size_t N = (size_t)r->n, M = PP_SSM_MEASURES;
-  char *b = nullptr;
-  cudaError_t e = cudaMalloc((void **)&b, al(M * N * 8) + al(N * 8) + al(M * PP_SSM_BINS * N * 4));
+  Surrogate &sg = r->sg;
+  auto layout = [&](char *base) {
+    ppi::Carve cv(base);
+    cv.take(sg.min, M * N);
+    cv.take(sg.min_tick, N);
+    cv.take(sg.hist, M * PP_SSM_BINS * N);
+    return cv.size;
+  };
+  observer_free(r->sg_buf, layout);
+  if (!on) return PP_OK;
+  cudaError_t e = observer_alloc(r->sg_buf, layout);
   if (e != cudaSuccess) return cuda_fail("cudaMalloc(rollout surrogate)", e);
-  double *mins = (double *)b;
-  int64_t *tick = (int64_t *)(b + al(M * N * 8));
-  int32_t *hist = (int32_t *)(b + al(M * N * 8) + al(N * 8));
   const std::vector<double> inf(M * N, INFINITY);
-  e = cudaMemcpy(mins, inf.data(), M * N * 8, cudaMemcpyHostToDevice);
-  if (e == cudaSuccess) e = cudaMemset(tick, 0xff, N * 8);  // -1: never lowered
-  if (e == cudaSuccess) e = cudaMemset(hist, 0, M * PP_SSM_BINS * N * 4);
+  e = cudaMemcpy(sg.min, inf.data(), M * N * 8, cudaMemcpyHostToDevice);
+  if (e == cudaSuccess) e = cudaMemset(sg.min_tick, 0xff, N * 8);  // -1: never lowered
+  if (e == cudaSuccess) e = cudaMemset(sg.hist, 0, M * PP_SSM_BINS * N * 4);
   if (e != cudaSuccess) {
-    cudaFree(b);
+    observer_free(r->sg_buf, layout);
     return cuda_fail("pp_rollouts_set_surrogate", e);
   }
-  r->ssm_buf = b;
-  r->ssm_min = mins;
-  r->ssm_tick = tick;
-  r->ssm_hist = hist;
   return PP_OK;
 }
 
 extern "C" int pp_rollouts_get_surrogate(const pp_rollouts *r, pp_rollout_surrogate *h) {
-  if (!r || !h || !r->ssm_buf) return PP_E_ARG;
+  if (!r || !h || !r->sg_buf) return PP_E_ARG;
   cudaError_t e = cudaDeviceSynchronize();
   if (e != cudaSuccess) return cuda_fail("pp_rollouts_get_surrogate", e);
   const size_t N = (size_t)r->n;
-  bool ok = true;
-  auto dn = [&](void *dst, const void *src, size_t bytes) {
-    if (dst && cudaMemcpy(dst, src, bytes, cudaMemcpyDeviceToHost) != cudaSuccess) ok = false;
-  };
+  Copy dn{cudaMemcpyDeviceToHost};
   double *const mins[PP_SSM_MEASURES] = {h->min_ttc_front, h->min_ttc_rear, h->min_thw};
-  for (int m = 0; m < PP_SSM_MEASURES; m++) dn(mins[m], r->ssm_min + m * N, N * 8);
-  dn(h->min_ttc_front_tick, r->ssm_tick, N * 8);
-  if (h->time_hist) {  // [measure][bin][R] on the device, [R][measure][bin] for the caller
-    constexpr int MB = PP_SSM_MEASURES * PP_SSM_BINS;
-    std::vector<int32_t> hist(N * MB);
-    dn(hist.data(), r->ssm_hist, N * MB * 4);
-    for (size_t i = 0; i < N; i++)
-      for (int e2 = 0; e2 < MB; e2++) h->time_hist[i * MB + e2] = hist[e2 * N + i];
-  }
-  if (!ok) return cuda_fail("pp_rollouts_get_surrogate copy", cudaGetLastError());
+  for (int m = 0; m < PP_SSM_MEASURES; m++) dn(mins[m], r->sg.min + m * N, N * 8);
+  dn(h->min_ttc_front_tick, r->sg.min_tick, N * 8);
+  dn.transpose(h->time_hist, r->sg.hist, N, PP_SSM_MEASURES * PP_SSM_BINS);
+  if (dn.e != cudaSuccess) return cuda_fail("pp_rollouts_get_surrogate copy", dn.e);
   return PP_OK;
 }
 
 extern "C" int pp_rollouts_surrogate_totals(const pp_rollouts *r, int64_t *totals_dev,
                                             void *cuda_stream) {
-  if (!r || !totals_dev || !r->ssm_buf) return PP_E_ARG;
-  {
-    const int rc = ppi::check_map_device(r->map, "pp_rollouts_surrogate_totals");
-    if (rc != PP_OK) return rc;
-  }
-  cudaStream_t st = (cudaStream_t)cuda_stream;
-  cudaError_t e = cudaMemsetAsync(totals_dev, 0, PP_SSM_TOTALS_LEN * sizeof(int64_t), st);
-  if (e != cudaSuccess) return cuda_fail("pp_rollouts_surrogate_totals", e);
-  const int64_t blocks = (r->n + kB - 1) / kB;
-  k_surrogate_totals<<<(int)(blocks < 1184 ? blocks : 1184), kB, 0, st>>>(
-      surrogate_view(r), (unsigned long long *)totals_dev);
-  ppi::count_launch(1);
-  e = cudaGetLastError();
-  if (e != cudaSuccess) return cuda_fail("k_surrogate_totals", e);
-  return PP_OK;
+  if (!r || !totals_dev || !r->sg_buf) return PP_E_ARG;
+  return record_totals(r, "pp_rollouts_surrogate_totals", k_surrogate_totals, "k_surrogate_totals",
+                       r->sg, PP_SSM_TOTALS_LEN, totals_dev, cuda_stream);
 }

@@ -256,8 +256,6 @@ k_sweep_select(const __grid_constant__ pp_config cfg, const __grid_constant__ pp
   out.n_points[f] = np;
 }
 
-inline size_t al(size_t v) { return (v + 255) & ~(size_t)255; }
-
 }  // namespace
 
 extern "C" int pp_sweep_batch(const pp_map *map, const pp_config *cfg, const pp_frames *in,
@@ -273,43 +271,37 @@ extern "C" int pp_sweep_batch(const pp_map *map, const pp_config *cfg, const pp_
   cudaStream_t st = (cudaStream_t)cuda_stream;
   const size_t N = (size_t)n;
   // scratch: plans of the ordinary step (for ego_d, ego_vd, ego_speed, target_lane) + sweep state
-  size_t off = 0;
-  auto take = [&](size_t bytes) {
-    const size_t o = off;
-    off += al(bytes);
-    return o;
+  pp_plans pl = {};
+  SweepScratch sw;
+  auto carve = [&](char *base) {
+    ppi::Carve cv(base);
+    cv.take(pl.next_x, N * PP_PATH_LEN);
+    cv.take(pl.next_y, N * PP_PATH_LEN);
+    cv.take(pl.n_points, N);
+    cv.take(pl.ego_lane, N);
+    cv.take(pl.ref_wp, N);
+    cv.take(pl.target_lane, N);
+    cv.take(pl.flags, N);
+    cv.take(pl.ego_d, N);
+    cv.take(pl.ego_vd, N);
+    cv.take(pl.ego_speed, N);
+    cv.take(sw.est, (size_t)kRows * 3 * N);
+    cv.take(sw.np, 3 * N);
+    cv.take(sw.code, 3 * N);
+    cv.take(sw.scores, N * PP_SWEEP_CANDS);
+    return cv.size;
   };
-  const size_t o_nx = take(N * PP_PATH_LEN * 8), o_ny = take(N * PP_PATH_LEN * 8);
-  const size_t o_i[5] = {take(N * 4), take(N * 4), take(N * 4), take(N * 4), take(N * 4)};
-  const size_t o_d[3] = {take(N * 8), take(N * 8), take(N * 8)};
-  const size_t o_est = take((size_t)kRows * 3 * N * 8), o_np = take(3 * N * 4), o_code = take(3 * N * 4);
-  const size_t o_sc = take(N * PP_SWEEP_CANDS * 8);
   char *buf = nullptr;
-  cudaError_t e = cudaMallocAsync((void **)&buf, off, st);
+  cudaError_t e = cudaMallocAsync((void **)&buf, carve(nullptr), st);
   if (e != cudaSuccess) {
     ppi::set_cuda_error("cudaMallocAsync(sweep)", (int)e, cudaGetErrorString(e));
     cudaGetLastError();
     return PP_E_CUDA;
   }
-  pp_plans pl = {};
-  pl.next_x = (double *)(buf + o_nx);
-  pl.next_y = (double *)(buf + o_ny);
-  pl.n_points = (int32_t *)(buf + o_i[0]);
-  pl.ego_lane = (int32_t *)(buf + o_i[1]);
-  pl.ref_wp = (int32_t *)(buf + o_i[2]);
-  pl.target_lane = (int32_t *)(buf + o_i[3]);
-  pl.flags = (uint32_t *)(buf + o_i[4]);
-  pl.ego_d = (double *)(buf + o_d[0]);
-  pl.ego_vd = (double *)(buf + o_d[1]);
-  pl.ego_speed = (double *)(buf + o_d[2]);
+  carve(buf);
+  sw.n3 = 3 * n;
   int rc = pp_plan_batch(map, cfg, in, &pl, n, st);
   if (rc == PP_OK) {
-    SweepScratch sw;
-    sw.est = (double *)(buf + o_est);
-    sw.np = (int32_t *)(buf + o_np);
-    sw.code = (int32_t *)(buf + o_code);
-    sw.scores = (double *)(buf + o_sc);
-    sw.n3 = 3 * n;
     const size_t smem_setup = (size_t)PPD_SWEEP_ROWS * PPD_TAILK * 128 * sizeof(double);
     static bool attr_done = false;
     if (!attr_done) {

@@ -1,34 +1,16 @@
 """Test-side binding of tests/incident_oracle.c (TEST INFRASTRUCTURE): the CPU restatement of
-the rollouts' incident monitor, built on oracle/pp_oracle.c.  The library is compiled on first
-use into a temporary directory (the tree may be read-only), with the oracle's flags."""
+the rollouts' incident monitor, built on oracle/pp_oracle.c
+(compiled by sim_oracle.load)."""
 from __future__ import annotations
 
 import ctypes as C
-import os
-import subprocess
-import tempfile
 
 import numpy as np
 
 import checkers
+import sim_oracle
 
 abi = checkers.abi
-HERE = os.path.dirname(os.path.abspath(__file__))
-SRC = os.path.join(HERE, "incident_oracle.c")
-_lib = None
-
-
-def _load():
-    global _lib
-    if _lib is None:
-        out = os.path.join(tempfile.mkdtemp(prefix="pp_incident_oracle_"), "libppincident.so")
-        cc = os.environ.get("CC", "gcc")
-        subprocess.run([cc, "-O2", "-ffp-contract=off", "-fPIC", "-std=gnu99", "-shared", "-o", out,
-                        SRC, "-lm", "-lpthread"], check=True, capture_output=True)
-        _lib = C.CDLL(out)
-        _lib.ppo_map_create.restype = C.c_void_p
-        _lib.ppo_map_create_from_csv.restype = C.c_void_p
-    return _lib
 
 
 class _MonitorStruct(C.Structure):
@@ -47,26 +29,17 @@ class MonitorState:
         self.pts = np.zeros(n, np.int64)
         self.active = np.zeros(n, np.uint32)
         self.off_pts = np.zeros(n, np.int32)
-        self.rec = {name: np.zeros((n, abi.INC_KINDS) if kind else (n,), dtype=dt)
-                    for name, dt, kind in abi.INC_FIELDS}
+        self.rec, rec = abi.host_record(abi.INC_FIELDS, abi.RolloutIncidents, n)
         self.struct = _MonitorStruct(self.ring.ctypes.data, self.pts.ctypes.data,
-                                     self.active.ctypes.data, self.off_pts.ctypes.data,
-                                     abi.RolloutIncidents(*[a.ctypes.data for a in self.rec.values()]))
+                                     self.active.ctypes.data, self.off_pts.ctypes.data, rec)
 
 
 class IncidentOracle:
     """The monitor on the highway map (default) or on a map made of the given waypoints."""
 
     def __init__(self, points=None):
-        self.lib = _load()
-        if points is None:
-            self.map = C.c_void_p(self.lib.ppo_map_create_from_csv(checkers.MAP_CSV.encode()))
-        else:
-            wx = np.ascontiguousarray(points[0], dtype=np.float64)
-            wy = np.ascontiguousarray(points[1], dtype=np.float64)
-            self.map = C.c_void_p(self.lib.ppo_map_create(C.c_void_p(wx.ctypes.data),
-                                                          C.c_void_p(wy.ctypes.data), C.c_int(len(wx))))
-        assert self.map.value, "map creation failed"
+        self.lib = sim_oracle.load("incident")
+        self.map = sim_oracle.make_map(self.lib, points)
 
     def init(self, ego_x, ego_y) -> MonitorState:
         """A fresh monitor state for len(ego_x) rollouts starting at (ego_x, ego_y)."""
