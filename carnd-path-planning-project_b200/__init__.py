@@ -48,6 +48,7 @@ EXPORTS = [
     "pp_rollouts_get_incidents", "pp_rollouts_incident_totals", "pp_rollouts_set_traffic",
     "pp_rollouts_get_traffic", "pp_rollouts_set_recorder", "pp_rollouts_get_recording",
     "pp_rollouts_set_surrogate", "pp_rollouts_get_surrogate", "pp_rollouts_surrogate_totals",
+    "pp_rollouts_set_restart", "pp_rollouts_get_restarts", "pp_rollouts_restart_totals",
     "pp_sweep_batch",
     "pp_set_pipes", "pp_plan_stats_batch", "pp_synth_frames_dev", "pp_fstats_batch",
     "pp_comm_unique_id", "pp_comm_init_rank", "pp_comm_init_all", "pp_comm_destroy",
@@ -570,6 +571,34 @@ class Rollouts:
         out = torch.empty(abi.SSM_TOTALS_LEN, dtype=torch.int64, device="cuda")
         _check(lib.pp_rollouts_surrogate_totals(self._h, C.c_void_p(out.data_ptr()),
                                                 C.c_void_p(stream)), "pp_rollouts_surrogate_totals")
+        return out
+
+    def set_restart(self, triggers):
+        """Switch episode restarts on before the first tick (include/pp.h): a rollout in which a
+        trigger fires starts over from a fresh draw at the end of that tick.  `triggers` is a bit
+        mask or an iterable of names of abi.REC_NAMES, as for set_recorder; 0 = off."""
+        mask = abi.rec_mask(triggers)
+        if not 0 <= mask < 1 << 32:
+            raise PPError(f"pp_rollouts_set_restart failed: mask {mask:#x}")
+        _check(lib.pp_rollouts_set_restart(self._h, C.c_uint32(mask)), "pp_rollouts_set_restart")
+
+    def restarts(self) -> dict:
+        """The restart record (include/pp.h, pp_rollout_restarts) as numpy arrays: episodes [n],
+        by_bit [n][RST_BITS] (restarts per ending bit, in the order of abi.REC_NAMES),
+        episode_tick, episode_m, ended_m, ended_lap [n]."""
+        out, s = abi.host_record(abi.RST_FIELDS, abi.RolloutRestarts, self.n)
+        _check(lib.pp_rollouts_get_restarts(self._h, C.byref(s)), "pp_rollouts_get_restarts")
+        return out
+
+    def restart_totals(self, stream=None):
+        """pp_rollouts_restart_totals -> int64[RST_TOTALS_LEN] device tensor: restarts per ending
+        bit, ended laps (entry RST_TOTAL_LAPS), ended millimetres (entry RST_TOTAL_MM)."""
+        import torch
+        if stream is None:
+            stream = torch.cuda.current_stream().cuda_stream
+        out = torch.empty(abi.RST_TOTALS_LEN, dtype=torch.int64, device="cuda")
+        _check(lib.pp_rollouts_restart_totals(self._h, C.c_void_p(out.data_ptr()),
+                                              C.c_void_p(stream)), "pp_rollouts_restart_totals")
         return out
 
     def incident_totals(self, stream=None):

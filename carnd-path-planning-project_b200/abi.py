@@ -233,6 +233,22 @@ class RolloutSurrogate(C.Structure):
     _fields_ = [(n, _dp) for n, _, _ in SSM_FIELDS]
 
 
+# episode restarts of the rollouts (pp_rollouts_set_restart): triggers as the recorder's (REC_NAMES)
+RST_RUBRIC_M = 4.32 * 1609.344      # m: an ended episode this long counts in ended_lap
+RST_BITS = INC_KINDS + 1            # ending bits: the kinds, then REC_NONFINITE
+RST_TOTAL_LAPS = INC_KINDS + 1      # pp_rollouts_restart_totals: ended laps
+RST_TOTAL_MM = INC_KINDS + 2        # ... ended distance in millimetres
+RST_TOTALS_LEN = INC_KINDS + 3
+RST_FIELDS = [  # (name, dtype, inner) ; inner: 0 scalar, 'bits' [RST_BITS]
+    ("episodes", np.int64, 0), ("by_bit", np.int64, "bits"), ("episode_tick", np.int64, 0),
+    ("episode_m", np.float64, 0), ("ended_m", np.float64, 0), ("ended_lap", np.int64, 0),
+]
+
+
+class RolloutRestarts(C.Structure):
+    _fields_ = [(n, _dp) for n, _, _ in RST_FIELDS]
+
+
 def rec_mask(triggers) -> int:
     """Recorder trigger mask from an int or an iterable of names of REC_NAMES."""
     if isinstance(triggers, (int, np.integer)):
@@ -253,12 +269,14 @@ def default_config() -> Config:
 
 def _inner(kind, max_cars):
     return {0: (), "prev": (PREV_KEEP,), "path": (PATH_LEN,), "cars": (max_cars,),
-            "kinds": (INC_KINDS,), "lanes": (NUM_LANES,), "hist": (SSM_MEASURES, SSM_BINS)}[kind]
+            "kinds": (INC_KINDS,), "lanes": (NUM_LANES,), "hist": (SSM_MEASURES, SSM_BINS),
+            "bits": (RST_BITS,)}[kind]
 
 
 def host_record(fields, struct, n: int, max_cars: int = 0):
     """Zeroed host arrays of a record of n rollouts, one [n] + inner shape per (name, dtype, kind)
-    of `fields` (INC_FIELDS, TRAFFIC_FIELDS, SSM_FIELDS), and the `struct` pointing at them."""
+    of `fields` (INC_FIELDS, TRAFFIC_FIELDS, SSM_FIELDS, RST_FIELDS), and the `struct` pointing
+    at them."""
     arrays = {name: np.zeros((n,) + _inner(kind, max_cars), dtype=dt) for name, dt, kind in fields}
     return arrays, struct(*[a.ctypes.data for a in arrays.values()])
 

@@ -93,6 +93,54 @@ struct Track {
   }
 };
 
+// The key of episode e of rollout `rollout` (pp.h, pp_rollouts_set_restart); episode 0's is the
+// key pp_rollouts_create draws with.
+__host__ __device__ inline uint64_t episode_key(uint64_t seed, int64_t rollout, int64_t e) {
+  const uint64_t k0 = mix64(mix64(seed ^ 0x1417ull) ^ ((uint64_t)rollout * 0xD1B54A32D192ED03ull));
+  return e == 0 ? k0 : mix64(k0 + (uint64_t)e * 0xA0761D6478BD642Full);
+}
+
+// The ego of a draw: at rest at the centre of `lane` on segment w, and its lane direction
+// (vx, vy) at unit speed, which the host turns into the yaw.
+struct EgoDraw {
+  double x, y, vx, vy;
+  int lane, w;
+};
+
+// One rollout's initial state from its key (pp.h, pp_rollouts_create): the ego, then c cars into
+// the rollout's car rows cl / cw / cr / cs.
+__host__ __device__ inline EgoDraw draw_rollout(const Track &trk, uint64_t key, int c, int32_t *cl,
+                                                int32_t *cw, double *cr, double *cs) {
+  uint64_t ctr = 0;
+  auto uni = [&]() { return u01(mix64(key + (ctr++) * 0x9E3779B97F4A7C15ull)); };
+  EgoDraw eg;
+  int w = (int)(uni() * trk.n);
+  if (w >= trk.n) w = trk.n - 1;
+  const double u = uni();
+  int lane = (int)(uni() * 3);
+  if (lane > 2) lane = 2;
+  trk.car(lane, w, u, 1.0, eg.x, eg.y, eg.vx, eg.vy);
+  eg.lane = lane;
+  eg.w = w;
+  for (int j = 0; j < c; j++) {
+    int l = (int)(uni() * 3);
+    if (l > 2) l = 2;
+    const double ds = -100.0 + 400.0 * uni();
+    const double sp = 17.88 + 8.94 * uni();
+    int ww = w;
+    double uu = u;
+    trk.walk(ww, uu, l, ds);
+    cl[j] = l;
+    cw[j] = ww;
+    cr[j] = uu;
+    cs[j] = sp;
+  }
+  return eg;
+}
+
+// The ego's yaw from its lane direction, on the host (device atan2 need not give the same bits).
+inline double ego_yaw_deg(double vx, double vy) { return std::atan2(vy, vx) * 180 / M_PI; }
+
 // Incident monitor state on the device (definitions: pp.h, pp_rollout_incidents).  Per-rollout
 // arrays are indexed by the absolute rollout; [x][R] arrays are row-major in x, so the ego warp's
 // lanes (consecutive rollouts) touch consecutive words.
@@ -149,6 +197,20 @@ struct Surrogate {
   int64_t R;
 };
 constexpr unsigned long long kInfBits = 0x7FF0000000000000ull;  // +inf
+
+// The episode-restart mode on the device (pp.h, pp_rollouts_set_restart).
+struct Restart {
+  int32_t *count0;        // [PP_INC_KINDS][R] the monitor's counts after the last tick
+  double *dist0;          // [R] distance_m after the last tick (the restore of a non-finite one)
+  int64_t *episodes;      // [R]
+  int64_t *by_bit;        // [PP_INC_KINDS + 1][R]
+  int64_t *ep_tick;       // [R]
+  double *ep_m, *ended_m; // [R]
+  int64_t *ended_lap;     // [R]
+  const double *yaw;      // [3][n] the ego's yaw at the centre of lane L on segment w (host atan2)
+  int64_t R;
+  unsigned mask;
+};
 
 // Bin of a value >= +0: the number of edges at or below it (PP_SSM_BINS: not counted).
 __host__ __device__ inline int ssm_bin(double v) {
@@ -869,6 +931,97 @@ __global__ void __launch_bounds__(kB) k_traffic_init(Track trk, const double *ex
   if (i < tf.R) traffic_ego_state(trk, tf, r, 0, rs, mt);
 }
 
+// The episode restarts of rollouts lo .. lo+n-1 at the end of a tick (pp.h,
+// pp_rollouts_set_restart), a thread per rollout, after k_sim_advance has counted the tick.  The
+// fired bits are the kinds whose count rose since the last tick and a non-finite distance_m.
+// Restarts are rare, so a restarting thread draws its c cars serially; under IDM it also runs
+// k_traffic_init's search at the new pose (lane_match votes among the lanes that enter it).
+template <int kTraffic>
+__global__ void __launch_bounds__(kB) k_restart(Track trk, int64_t lo, int64_t n, int c,
+                                                uint64_t seed, int64_t first, SimState st,
+                                                Monitor mo, Traffic tf, Restart rt) {
+  const int64_t i = (int64_t)blockIdx.x * kB + threadIdx.x;
+  if (i >= n) return;
+  const int64_t r = lo + i, R = rt.R;
+  unsigned fired = 0;
+#pragma unroll
+  for (int kind = 0; kind < PP_INC_KINDS; kind++) {
+    const int32_t now = mo.count[kind * R + r];
+    if (now != rt.count0[kind * R + r]) {
+      fired |= 1u << kind;
+      rt.count0[kind * R + r] = now;
+    }
+  }
+  double d = mo.dist[r];
+  if (!isfinite(d)) fired |= 1u << PP_REC_NONFINITE;
+  const unsigned hit = fired & rt.mask;
+  if (!hit) {
+    rt.dist0[r] = d;
+    return;
+  }
+  if (!isfinite(d)) {
+    d = rt.dist0[r];
+    mo.dist[r] = d;
+  }
+  const double ended = d - rt.ep_m[r];
+  rt.ended_m[r] += ended;
+  if (ended >= PP_RST_RUBRIC_M) rt.ended_lap[r] += 1;
+  rt.by_bit[(__ffs(hit) - 1) * R + r] += 1;
+  const int64_t e = rt.episodes[r] + 1;
+  rt.episodes[r] = e;
+  const int64_t tick = st.ticks[r];  // t + 1
+  rt.ep_tick[r] = tick;
+  rt.ep_m[r] = d;
+  rt.dist0[r] = d;
+  const int64_t q = r * c;
+  const EgoDraw eg = draw_rollout(trk, episode_key(seed, first + r, e), c, st.car_lane + q,
+                                  st.car_wp + q, st.car_ratio + q, st.car_speed + q);
+  st.ego_x[r] = eg.x;
+  st.ego_y[r] = eg.y;
+  st.ego_yaw[r] = rt.yaw[eg.lane * trk.n + eg.w];
+  st.ego_mph[r] = 0.0;
+  st.path_n[r] = 0;
+  st.path_off[r] = 0;
+  st.target_lane[r] = eg.lane;
+  mo.ring[r] = make_double2(eg.x, eg.y);  // D_0 in row 0
+  mo.ring_acc[r] = make_double2(0.0, 0.0);
+  mo.pts[r] = 0;
+  mo.active[r] = 0;
+  mo.off_pts[r] = 0;
+  mo.clean[r] = 0.0;
+  if constexpr (kTraffic == PP_TRAFFIC_IDM) {
+    for (int j = 0; j < c; j++) {
+      tf.v0[q + j] = st.car_speed[q + j];
+      tf.acc[q + j] = 0.0;
+    }
+    const ppd::MapView mv{trk.t, trk.n, trk.n < PPD_PAD ? trk.n : PPD_PAD};
+    ppd::RefState rs;
+    ppd::init_reference(mv, eg.x, eg.y, rs);
+    const ppd::Match mt = ppd::lane_match(mv, rs, eg.x, eg.y);
+    traffic_ego_state(trk, tf, r, (int)(tick & 1), rs, mt);
+  }
+}
+
+// pp_rollouts_restart_totals: restarts per ending bit, ended laps, ended millimetres.
+__global__ void __launch_bounds__(kB) k_restart_totals(Restart rt, unsigned long long *tot) {
+  unsigned long long acc[PP_RST_TOTALS_LEN];
+#pragma unroll
+  for (int e = 0; e < PP_RST_TOTALS_LEN; e++) acc[e] = 0;
+  for (int64_t r = (int64_t)blockIdx.x * kB + threadIdx.x; r < rt.R; r += (int64_t)gridDim.x * kB) {
+#pragma unroll
+    for (int b = 0; b <= PP_INC_KINDS; b++) acc[b] += (unsigned long long)rt.by_bit[b * rt.R + r];
+    acc[PP_RST_TOTAL_LAPS] += (unsigned long long)rt.ended_lap[r];
+    acc[PP_RST_TOTAL_MM] += (unsigned long long)llround(rt.ended_m[r] * 1000.0);
+  }
+#pragma unroll
+  for (int e = 0; e < PP_RST_TOTALS_LEN; e++) {
+    unsigned long long v = acc[e];
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) v += __shfl_down_sync(0xffffffffu, v, o);
+    if ((threadIdx.x & 31) == 0 && v) atomicAdd(&tot[e], v);
+  }
+}
+
 // The staging buffer of pp_rollouts_get_recording: m rows of W frames in pp_frames layout (frame
 // (i, j) at i * W + j), then the trigger arrays of the m rows.
 struct RecOut {
@@ -1005,6 +1158,8 @@ struct pp_rollouts {
   std::vector<std::pair<int64_t, int32_t>> rec_k;
   char *sg_buf = nullptr;  // near-miss measures (pp.h, pp_rollouts_set_surrogate): on while allocated
   Surrogate sg;
+  char *rt_buf = nullptr;  // episode restarts (pp.h, pp_rollouts_set_restart): on while allocated
+  Restart rt;
 };
 
 namespace {
@@ -1156,6 +1311,8 @@ extern "C" int pp_rollouts_create(const pp_map *map, int64_t n, int32_t c, uint6
   r->tf = Traffic{nullptr, nullptr, nullptr, nullptr, nullptr, r->fr.ego_speed_mph, n};
   r->rc = Recorder{nullptr, nullptr, nullptr, n, c, 0, 0};
   r->sg = Surrogate{nullptr, nullptr, nullptr, n};
+  r->rt = Restart{};
+  r->rt.R = n;
   cudaMemset(r->mo.first_tick, 0xff, N * 8);  // -1: no incident yet
   cudaMemset(r->mo.first_kind, 0xff, N * 4);
 
@@ -1164,34 +1321,14 @@ extern "C" int pp_rollouts_create(const pp_map *map, int64_t n, int32_t c, uint6
   std::vector<int32_t> tl(N), cl(NC), cw(NC);
   Track trk{map->table.data(), map->n, PP_MAP_STRIDE};
   for (int64_t i = 0; i < n; i++) {
-    uint64_t key = mix64(mix64(seed ^ 0x1417ull) ^ ((uint64_t)(first + i) * 0xD1B54A32D192ED03ull));
-    uint64_t ctr = 0;
-    auto uni = [&]() { return u01(mix64(key + (ctr++) * 0x9E3779B97F4A7C15ull)); };
-    int w = (int)(uni() * map->n);
-    if (w >= map->n) w = map->n - 1;
-    double u = uni();
-    int lane = (int)(uni() * 3);
-    if (lane > 2) lane = 2;
-    double x, y, vx, vy;
-    trk.car(lane, w, u, 1.0, x, y, vx, vy);
-    ex[i] = x;
-    ey[i] = y;
-    yaw[i] = std::atan2(vy, vx) * 180 / M_PI;
+    const size_t q = (size_t)i * c;
+    const EgoDraw eg = draw_rollout(trk, episode_key(seed, first + i, 0), c, cl.data() + q,
+                                    cw.data() + q, cr.data() + q, cs.data() + q);
+    ex[i] = eg.x;
+    ey[i] = eg.y;
+    yaw[i] = ego_yaw_deg(eg.vx, eg.vy);
     mph[i] = 0.0;
-    tl[i] = lane;
-    for (int j = 0; j < c; j++) {
-      int l = (int)(uni() * 3);
-      if (l > 2) l = 2;
-      const double ds = -100.0 + 400.0 * uni();
-      const double sp = 17.88 + 8.94 * uni();
-      int ww = w;
-      double uu = u;
-      trk.walk(ww, uu, l, ds);
-      cl[i * c + j] = l;
-      cw[i * c + j] = ww;
-      cr[i * c + j] = uu;
-      cs[i * c + j] = sp;
-    }
+    tl[i] = eg.lane;
   }
   Copy up{cudaMemcpyHostToDevice};
   up(r->st.ego_x, ex.data(), N * 8);
@@ -1254,6 +1391,7 @@ extern "C" void pp_rollouts_destroy(pp_rollouts *r) {
   if (r->tf_buf) cudaFree(r->tf_buf);
   if (r->rc_buf) cudaFree(r->rc_buf);
   if (r->sg_buf) cudaFree(r->sg_buf);
+  if (r->rt_buf) cudaFree(r->rt_buf);
   delete r;
 }
 
@@ -1330,6 +1468,12 @@ int issue_tick(pp_rollouts *r, const pp_config *cfg, int32_t consume_k, cudaStre
         trk, lo, cnt, r->c, r->seed, r->first, consume_k, r->st, r->pl,
         (unsigned long long *)r->stats_sum, plan_sums ? 0 : 1, r->mo, r->tf, r->rc, r->sg);
     ppi::count_launch(2);
+    if (r->rt_buf) {
+      auto *restart = idm ? k_restart<PP_TRAFFIC_IDM> : k_restart<PP_TRAFFIC_CONSTANT>;
+      restart<<<(int)((cnt + kB - 1) / kB), kB, 0, gs>>>(trk, lo, cnt, r->c, r->seed, r->first,
+                                                          r->st, r->mo, r->tf, r->rt);
+      ppi::count_launch(1);
+    }
   }
   r->launches_per_tick = pp_launch_count() - launches0;
   if (join) {
@@ -1759,4 +1903,74 @@ extern "C" int pp_rollouts_surrogate_totals(const pp_rollouts *r, int64_t *total
   if (!r || !totals_dev || !r->sg_buf) return PP_E_ARG;
   return record_totals(r, "pp_rollouts_surrogate_totals", k_surrogate_totals, "k_surrogate_totals",
                        r->sg, PP_SSM_TOTALS_LEN, totals_dev, cuda_stream);
+}
+
+extern "C" int pp_rollouts_set_restart(pp_rollouts *r, uint32_t triggers) {
+  if (!r || r->tick != 0 || (triggers >> (PP_REC_NONFINITE + 1)) != 0) return PP_E_ARG;
+  const size_t N = (size_t)r->n, K = PP_INC_KINDS, nw = (size_t)r->map->n;
+  Restart &rt = r->rt;
+  auto layout = [&](char *base) {
+    ppi::Carve cv(base);
+    cv.take(rt.count0, K * N);
+    cv.take(rt.dist0, N);
+    cv.take(rt.episodes, N);
+    cv.take(rt.by_bit, (K + 1) * N);
+    cv.take(rt.ep_tick, N);
+    cv.take(rt.ep_m, N);
+    cv.take(rt.ended_m, N);
+    cv.take(rt.ended_lap, N);
+    cv.take(rt.yaw, 3 * nw);
+    return cv.size;
+  };
+  observer_free(r->rt_buf, layout);
+  rt.mask = 0;
+  if (triggers == 0) return PP_OK;
+  {
+    const int rc = ppi::check_map_device(r->map, "pp_rollouts_set_restart");
+    if (rc != PP_OK) return rc;
+  }
+  const size_t bytes = layout(nullptr);
+  cudaError_t e = observer_alloc(r->rt_buf, layout);
+  if (e != cudaSuccess) return cuda_fail("cudaMalloc(rollout restarts)", e);
+  // the yaw of a cold start at the centre of lane L on segment w, with create's expression
+  const Track trk{r->map->table.data(), r->map->n, PP_MAP_STRIDE};
+  std::vector<double> yaw(3 * nw);
+  for (int L = 0; L < 3; L++)
+    for (int w = 0; w < r->map->n; w++) {
+      double x, y, vx, vy;
+      trk.car(L, w, 0.0, 1.0, x, y, vx, vy);
+      yaw[L * nw + w] = ego_yaw_deg(vx, vy);
+    }
+  e = cudaMemset(r->rt_buf, 0, bytes);
+  if (e == cudaSuccess) e = cudaMemcpy((double *)rt.yaw, yaw.data(), yaw.size() * 8, cudaMemcpyHostToDevice);
+  if (e != cudaSuccess) {
+    observer_free(r->rt_buf, layout);
+    return cuda_fail("pp_rollouts_set_restart", e);
+  }
+  rt.mask = triggers;
+  return PP_OK;
+}
+
+extern "C" int pp_rollouts_get_restarts(const pp_rollouts *r, pp_rollout_restarts *h) {
+  if (!r || !h || !r->rt_buf) return PP_E_ARG;
+  cudaError_t e = cudaDeviceSynchronize();
+  if (e != cudaSuccess) return cuda_fail("pp_rollouts_get_restarts", e);
+  const size_t N = (size_t)r->n;
+  const Restart &rt = r->rt;
+  Copy dn{cudaMemcpyDeviceToHost};
+  dn(h->episodes, rt.episodes, N * 8);
+  dn.transpose(h->by_bit, rt.by_bit, N, PP_INC_KINDS + 1);
+  dn(h->episode_tick, rt.ep_tick, N * 8);
+  dn(h->episode_m, rt.ep_m, N * 8);
+  dn(h->ended_m, rt.ended_m, N * 8);
+  dn(h->ended_lap, rt.ended_lap, N * 8);
+  if (dn.e != cudaSuccess) return cuda_fail("pp_rollouts_get_restarts copy", dn.e);
+  return PP_OK;
+}
+
+extern "C" int pp_rollouts_restart_totals(const pp_rollouts *r, int64_t *totals_dev,
+                                          void *cuda_stream) {
+  if (!r || !totals_dev || !r->rt_buf) return PP_E_ARG;
+  return record_totals(r, "pp_rollouts_restart_totals", k_restart_totals, "k_restart_totals",
+                       r->rt, PP_RST_TOTALS_LEN, totals_dev, cuda_stream);
 }

@@ -743,6 +743,64 @@ typedef struct pp_rollout_recording { /* host arrays, m rows; any pointer may be
 int pp_rollouts_get_recording(const pp_rollouts *r, const int64_t *rollouts, int64_t m,
                               pp_rollout_recording *host_out);
 
+/* ---- episode restarts of the rollouts ----------------------------------------------------
+ * An opt-in mode in which a rollout that fails starts over from a fresh draw, so that every tick
+ * of a long run is spent driving and the rubric's "4.32 miles without incident" can be measured
+ * per episode.  Every operation is IEEE double + - * /, left to right, without fused multiply-add,
+ * so the CPU restatement is bit-identical.
+ *
+ * Triggers.  The mask is the recorder's: bit PP_INC_<kind> fires in tick t when the monitor COUNTS
+ * an incident of that kind in tick t (its count rises); bit PP_REC_NONFINITE fires when distance_m
+ * is not finite after tick t.  A rollout restarts at the end of tick t when fired & mask != 0;
+ * its ending bit is the lowest such bit.
+ * Order.  The tick runs as without the mode (frames, plan, advance, then the monitor, traffic,
+ * recorder and near-miss updates); only after all of them is the restart applied, so every
+ * observer sees the failing tick as it happened and a frozen recorder window stays frozen.
+ * pp_rollouts_get_state after a run returns the post-restart state.
+ * Episode draw.  Episode e of rollout i is drawn exactly as pp_rollouts_create draws the rollout,
+ * with key_e in place of key_0 = mix64(mix64(seed ^ 0x1417) ^ ((first + i) * 0xD1B54A32D192ED03)):
+ *   key_e = mix64(key_0 + e * 0xA0761D6478BD642F)   (e >= 1; uint64 arithmetic, mix64 = splitmix64)
+ * so episode 0 is the create draw bit for bit: the ego at rest on a random lane centre (yaw from
+ * the segment direction, computed on the host as create computes it, 0 mph, target_lane = that
+ * lane, no kept path: a cold start) and C cars within [-100, 300] m.
+ * What a restart resets: the rollout's simulator state; the monitor's ego history (D_0 = the new
+ * pose, point index 0, the active edge bits and the off-centre count cleared, so the kinematics
+ * are undefined again until 10 / 20 / 70 points have been driven; the jump to the new pose is not
+ * driven distance); clean_m = 0; under PP_TRAFFIC_IDM every car's v0 = its drawn speed and acc = 0,
+ * and the ego's lane state the next tick reads comes from Map::init_reference_waypoint's full
+ * search at the new pose, as before the first tick.
+ * What it keeps: the rollout's tick counter (respawn draws and first_tick stay keyed by the
+ * lifetime tick, so episodes never reuse respawn draws), the incident counts, first_tick /
+ * first_kind, best_clean_m, the maxima, the near-miss record and the recorder.
+ * Distance.  At a restart, a distance_m that is not finite is set back to its value after tick
+ * t-1 (so the failing tick adds nothing).  The ended episode's distance is distance_m (after that
+ * restore) minus the episode's episode_m.
+ * Device memory: 140 R bytes, and 24 bytes per waypoint for the yaw table. */
+#define PP_RST_RUBRIC_M (4.32 * 1609.344) /* m: the Udacity rubric's 4.32 miles */
+/* Before the first tick only (PP_E_ARG afterwards).  triggers: bits below
+ * (1u << (PP_REC_NONFINITE + 1)), else PP_E_ARG; 0 = off (the default: no launch, nothing
+ * changes).  May be called before or after pp_rollouts_set_traffic.  If the allocation fails the
+ * mode is left off. */
+int pp_rollouts_set_restart(pp_rollouts *r, uint32_t triggers);
+typedef struct pp_rollout_restarts { /* host arrays, R rollouts; any pointer may be NULL */
+  int64_t *episodes;                 /* [R] restarts so far */
+  int64_t *by_bit;                   /* [R][PP_INC_KINDS + 1] restarts per ending bit */
+  int64_t *episode_tick;             /* [R] tick the current episode began at: 0, or t + 1 */
+  double *episode_m;                 /* [R] distance_m when it began */
+  double *ended_m;                   /* [R] sum of the ended episodes' distances, in episode order */
+  int64_t *ended_lap;                /* [R] ended episodes with distance >= PP_RST_RUBRIC_M */
+} pp_rollout_restarts;
+/* Copy the record out (synchronises the device).  PP_E_ARG when the mode is off. */
+int pp_rollouts_get_restarts(const pp_rollouts *r, pp_rollout_restarts *host_out);
+/* totals_dev[PP_RST_TOTALS_LEN] (device, int64, overwritten; asynchronous on cuda_stream): by_bit
+ * summed over the rollouts, then the sum of ended_lap, then the ended distance in millimetres, sum
+ * of llround(ended_m * 1000).  All int64, so a multi-GPU job all-reduces it with ncclSum.
+ * PP_E_ARG when the mode is off. */
+#define PP_RST_TOTAL_LAPS (PP_INC_KINDS + 1)
+#define PP_RST_TOTAL_MM (PP_INC_KINDS + 2)
+#define PP_RST_TOTALS_LEN (PP_INC_KINDS + 3)
+int pp_rollouts_restart_totals(const pp_rollouts *r, int64_t *totals_dev, void *cuda_stream);
+
 /* ---- near-miss (surrogate safety) measures of the rollouts --------------------------------
  * An opt-in observer that measures how close each ego comes to a collision, not only whether it
  * has one: time to collision with the car ahead and the car behind (TTC, Hayward 1972), time

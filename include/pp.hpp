@@ -910,6 +910,38 @@ class Rollouts {
     check(pp_dev_sync(), "pp_dev_sync");
     return dev.to_host();
   }
+  // Episode restarts (pp.h, pp_rollouts_set_restart), before the first tick only; 0 = off.
+  void set_restart(uint32_t triggers) {
+    check(pp_rollouts_set_restart(h_, triggers), "pp_rollouts_set_restart");
+  }
+  // The restart record; by_bit is [n][PP_INC_KINDS + 1].
+  struct Restarts {
+    std::vector<int64_t> episodes, by_bit, episode_tick, ended_lap;
+    std::vector<double> episode_m, ended_m;
+  };
+  Restarts restarts() const {
+    Restarts o;
+    for (auto *v : {&o.episodes, &o.episode_tick, &o.ended_lap}) v->resize(n_);
+    o.by_bit.resize((size_t)n_ * (PP_INC_KINDS + 1));
+    o.episode_m.resize(n_);
+    o.ended_m.resize(n_);
+    pp_rollout_restarts h;
+    h.episodes = o.episodes.data();
+    h.by_bit = o.by_bit.data();
+    h.episode_tick = o.episode_tick.data();
+    h.episode_m = o.episode_m.data();
+    h.ended_m = o.ended_m.data();
+    h.ended_lap = o.ended_lap.data();
+    check(pp_rollouts_get_restarts(h_, &h), "pp_rollouts_get_restarts");
+    return o;
+  }
+  // The totals (pp.h, pp_rollouts_restart_totals), copied to the host.
+  std::vector<int64_t> restart_totals() const {
+    detail::Dev<int64_t> dev(PP_RST_TOTALS_LEN);
+    check(pp_rollouts_restart_totals(h_, dev.get(), nullptr), "pp_rollouts_restart_totals");
+    check(pp_dev_sync(), "pp_dev_sync");
+    return dev.to_host();
+  }
 
  private:
   pp_rollouts *h_ = nullptr;
