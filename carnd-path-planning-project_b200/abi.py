@@ -321,6 +321,9 @@ class FrameBatch:
         out.max_cars = self.max_cars
         for name, _, _ in FRAME_FIELDS:
             setattr(out, name, np.ascontiguousarray(getattr(self, name)[lo:hi]))
+        if getattr(self, "car_frozen_lane", None) is not None:
+            for name, _ in FROZEN_FIELDS:
+                setattr(out, name, np.ascontiguousarray(getattr(self, name)[lo:hi]))
         return out
 
     @staticmethod

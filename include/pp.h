@@ -133,7 +133,11 @@ typedef struct pp_frames {
    * the Frenet values of its last sighting, which the reference never recomputes:
    * car_frozen_lane[f*max_cars + j] >= 0 marks slot j as frozen (lane = that value, s / d / vs /
    * vd from the arrays below; its car_x / car_y are not matched, car_vx / car_vy still give its
-   * Cartesian speed to LimitSpeed, :1080); -1 = an ordinary car of the current message.
+   * Cartesian speed to LimitSpeed, :1080); -1 = an ordinary car of the current message.  A frozen
+   * lane must be 0..2, the values lane matching gives (it is not validated).  A frozen slot is
+   * never matched and never dropped; its per-car outputs are car_lane = the frozen lane,
+   * car_next_wp = 0 and car_s / car_d / car_vs / car_vd = the frozen values.  It takes its place
+   * in the ascending-id order like any other car.
    * include/pp_wire.hpp (pp::wire::Session) maintains this state for replayed sessions. */
   const int32_t *car_frozen_lane; /* [N][max_cars] */
   const double *car_frozen_s;     /* [N][max_cars] */

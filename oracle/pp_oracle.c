@@ -26,15 +26,20 @@
 
 #define EPS 1e-5 /* src/main.cpp:24 EPSILON */
 
-/* tunables, src/main.cpp:39-49 */
-static const double relaxed_acc = 5;
-static const double min_relaxed_acc_while_braking = 4;
-static const double maximum_acc = 8;
-static const double max_speed = 22.2;
-static const double car_length = 4.5;
-static const double safety_distance = 2;
-static const double keep_distance = 10;
-static const double keep_distance_leeway = 0.5;
+/* tunables, src/main.cpp:30,39-49: the reference's literals.  Every planning function takes
+ * the tunables as a pp_config; the ppo_* entry points without the _cfg suffix plan with these. */
+static const pp_config default_cfg = {
+    5,    /* relaxed_acc */
+    4,    /* min_relaxed_acc_while_braking */
+    8,    /* maximum_acc */
+    22.2, /* max_speed */
+    4.5,  /* car_length */
+    2,    /* safety_distance */
+    10,   /* keep_distance */
+    0.5,  /* keep_distance_leeway */
+    0,    /* test_fast_lane_change */
+    0,
+};
 
 typedef struct {
   double x, y;
@@ -332,8 +337,10 @@ typedef struct {
 
 /* src/main.cpp:364-485 LaneChangePlanner::calculate_target_lane.
  * cars[] must be in ascending id order (std::map iteration order). */
-static int choose_lane(const car_t *cars, int nc, int ego_lane, int target_lane, double ego_s,
-                       double ego_vs, double dt0, int fast_lane_change, uint32_t *flags) {
+static int choose_lane(const pp_config *cfg, const car_t *cars, int nc, int ego_lane,
+                       int target_lane, double ego_s, double ego_vs, double dt0, uint32_t *flags) {
+  const double max_speed = cfg->max_speed, car_length = cfg->car_length;
+  const double safety_distance = cfg->safety_distance, relaxed_acc = cfg->relaxed_acc;
   double lane_speed[3], next_s[3];
   int open[3];
   for (int i = 0; i < 3; i++) {
@@ -396,7 +403,7 @@ static int choose_lane(const car_t *cars, int nc, int ego_lane, int target_lane,
     double distance_score = 1 - fabs((double)(target_lane - lane)) / 2;
     double fr = next_s[lane] / 100;
     double free_score = (fr < 1.0) ? fr : 1.0; /* std::min(1.0, fr) */
-    if (fast_lane_change) distance_score = 0;
+    if (cfg->test_fast_lane_change) distance_score = 0;
     double total = speed_score + distance_score / 2 + free_score;
     if (total > best) {
       best = total;
@@ -417,11 +424,11 @@ typedef struct {
   double start, target, time, shift;
 } speedctl;
 
-static void sc_init(speedctl *c, double ego_speed) {
+static void sc_init(const pp_config *cfg, speedctl *c, double ego_speed) {
   c->shift = 0;
   c->start = ego_speed;
-  c->target = max_speed;
-  c->time = fabs(ego_speed - max_speed) / relaxed_acc;
+  c->target = cfg->max_speed;
+  c->time = fabs(ego_speed - cfg->max_speed) / cfg->relaxed_acc;
 }
 static double sc_speed(const speedctl *c, double t) {
   t -= c->shift;
@@ -450,9 +457,12 @@ static void sc_override(speedctl *c, double t, double speed) {
 }
 
 /* src/main.cpp:1052-1151 LimitSpeed (one fresh instance per call, as in the glue) */
-static void limit_speed(double car_vx, double car_vy, double next_s, double ego_s, double ego_speed,
-                        double ego_acc, int in_lane, double *t_speed, double *t_time,
-                        uint32_t *flags) {
+static void limit_speed(const pp_config *cfg, double car_vx, double car_vy, double next_s,
+                        double ego_s, double ego_speed, double ego_acc, int in_lane,
+                        double *t_speed, double *t_time, uint32_t *flags) {
+  const double relaxed_acc = cfg->relaxed_acc, maximum_acc = cfg->maximum_acc;
+  const double max_speed = cfg->max_speed, car_length = cfg->car_length;
+  const double safety_distance = cfg->safety_distance, keep_distance = cfg->keep_distance;
   double target_speed = max_speed;
   double target_time = fabs(ego_speed - max_speed) / relaxed_acc;
   int can_accelerate = 1;
@@ -464,7 +474,7 @@ static void limit_speed(double car_vx, double car_vy, double next_s, double ego_
   double car_speed = sqrt(car_vx * car_vx + car_vy * car_vy);
   if (ego_speed > car_speed) {
     double acc = relaxed_acc;
-    if (ego_acc < 0) acc = min_relaxed_acc_while_braking;
+    if (ego_acc < 0) acc = cfg->min_relaxed_acc_while_braking;
     double dv = ego_speed - car_speed;
     double dt = dv / acc;
     double dd = ego_speed * dt - dv / 2 * dt;
@@ -492,7 +502,7 @@ static void limit_speed(double car_vx, double car_vy, double next_s, double ego_
         if (target_time < mt) target_time = mt;
       }
       *flags |= PP_F_ADJUST;
-    } else if (ego_s + car_length + keep_distance + keep_distance_leeway > next_s) {
+    } else if (ego_s + car_length + keep_distance + cfg->keep_distance_leeway > next_s) {
       target_speed = car_speed;
       target_time = 1.0;
       {
@@ -593,11 +603,12 @@ static double spline_eval(const spline_t *sp, double x) {
 
 /* src/main.cpp:565-1049 TrajectoryBuilder::build.  prev has nprev (0 or 10)
  * points.  Returns the number of points written to ox/oy. */
-static int build_trajectory(const ppo_map *m, const refstate *rs, const vec2 *prev, int nprev,
-                            double ego_x, double ego_y, double yaw_deg, int target_lane,
-                            double ego_d, double ego_vd, speedctl *sc, double *ox, double *oy,
-                            uint32_t *flags) {
+static int build_trajectory(const ppo_map *m, const pp_config *cfg, const refstate *rs,
+                            const vec2 *prev, int nprev, double ego_x, double ego_y, double yaw_deg,
+                            int target_lane, double ego_d, double ego_vd, speedctl *sc, double *ox,
+                            double *oy, uint32_t *flags) {
   const double PI = M_PI;
+  const double maximum_acc = cfg->maximum_acc;
   int np = 0;
   for (int i = 0; i < nprev; i++) {
     ox[np] = prev[i].x;
@@ -807,7 +818,8 @@ static int build_trajectory(const ppo_map *m, const refstate *rs, const vec2 *pr
 }
 
 /* One frame: glue of main::onMessage, src/main.cpp:1254-1457. */
-static void plan_frame(const ppo_map *m, const pp_frames *in, const pp_plans *out, int64_t f) {
+static void plan_frame(const ppo_map *m, const pp_config *cfg, const pp_frames *in,
+                       const pp_plans *out, int64_t f) {
   const int K = PP_PREV_KEEP;
   uint32_t flags = 0;
   double ex = in->ego_x[f], ey = in->ego_y[f];
@@ -848,8 +860,8 @@ static void plan_frame(const ppo_map *m, const pp_frames *in, const pp_plans *ou
   }
   double evs, evd;
   project_speed(m, svx, svy, rs.wp, &evs, &evd); /* :1313 */
-  if (acc > maximum_acc) acc = maximum_acc;
-  if (acc < -maximum_acc) acc = -maximum_acc;
+  if (acc > cfg->maximum_acc) acc = cfg->maximum_acc;
+  if (acc < -cfg->maximum_acc) acc = -cfg->maximum_acc;
 
   /* sensor fusion (:1325-1350), kept in ascending id order like std::map */
   car_t cars[PP_MAX_CARS];
@@ -864,9 +876,21 @@ static void plan_frame(const ppo_map *m, const pp_frames *in, const pp_plans *ou
     c.vy = in->car_vy[f * mc + j];
     c.s = c.d = c.vs = c.vd = 0;
     c.lane = 0;
-    int nwp = 0;
-    int ok = lane_match(m, &rs, cx, cy, &c.s, &c.d, &c.lane, &nwp);
-    if (ok) project_speed(m, c.vx, c.vy, nwp, &c.vs, &c.vd);
+    int nwp = 0, ok;
+    const int frozen_lane = in->car_frozen_lane ? in->car_frozen_lane[f * mc + j] : -1;
+    if (frozen_lane >= 0) {
+      /* a car held over from an earlier message (pp_frames::car_frozen_*): the Frenet values of
+       * its last sighting, never matched and never dropped; car_vx / car_vy still feed LimitSpeed */
+      ok = 1;
+      c.lane = frozen_lane;
+      c.s = in->car_frozen_s[f * mc + j];
+      c.d = in->car_frozen_d[f * mc + j];
+      c.vs = in->car_frozen_vs[f * mc + j];
+      c.vd = in->car_frozen_vd[f * mc + j];
+    } else {
+      ok = lane_match(m, &rs, cx, cy, &c.s, &c.d, &c.lane, &nwp);
+      if (ok) project_speed(m, c.vx, c.vy, nwp, &c.vs, &c.vd);
+    }
     if (out->car_lane) out->car_lane[f * mc + j] = ok ? c.lane : -1;
     if (out->car_next_wp) out->car_next_wp[f * mc + j] = ok ? nwp : 0;
     if (out->car_s) out->car_s[f * mc + j] = ok ? c.s : 0;
@@ -892,7 +916,7 @@ static void plan_frame(const ppo_map *m, const pp_frames *in, const pp_plans *ou
     cars[pos] = c;
   }
 
-  target_lane = choose_lane(cars, nc, elane, target_lane, es, evs, dt0, 0, &flags); /* :1355 */
+  target_lane = choose_lane(cfg, cars, nc, elane, target_lane, es, evs, dt0, &flags); /* :1355 */
   if (target_lane != elane) { /* :1358-1369 */
     double dtl = lane_center_offset(target_lane);
     double diff = fabs(evd * 1.0 + ed - dtl);
@@ -914,7 +938,7 @@ static void plan_frame(const ppo_map *m, const pp_frames *in, const pp_plans *ou
         ns = s0;
       }
     }
-    if (s0 >= es - car_length - safety_distance && fabs(d0 - dtl) < 3) {
+    if (s0 >= es - cfg->car_length - cfg->safety_distance && fabs(d0 - dtl) < 3) {
       if (nid_tl == -1 || ns_tl > s0) {
         nid_tl = cars[c].id;
         nidx_tl = c;
@@ -925,22 +949,23 @@ static void plan_frame(const ppo_map *m, const pp_frames *in, const pp_plans *ou
   if (nid_tl == nid) nid_tl = -1;
 
   speedctl sc;
-  sc_init(&sc, speed); /* :1422 */
+  sc_init(cfg, &sc, speed); /* :1422 */
   if (nid != -1) {
     double ts, tt;
-    limit_speed(cars[nidx].vx, cars[nidx].vy, ns, es, speed, acc, 1, &ts, &tt, &flags);
+    limit_speed(cfg, cars[nidx].vx, cars[nidx].vy, ns, es, speed, acc, 1, &ts, &tt, &flags);
     sc_limit(&sc, ts, tt);
   }
   if (nid_tl != -1) {
     double ts, tt;
-    limit_speed(cars[nidx_tl].vx, cars[nidx_tl].vy, ns_tl, es, speed, acc, 0, &ts, &tt, &flags);
+    limit_speed(cfg, cars[nidx_tl].vx, cars[nidx_tl].vy, ns_tl, es, speed, acc, 0, &ts, &tt,
+                &flags);
     sc_limit(&sc, ts, tt);
   }
   if (out->target_speed) out->target_speed[f] = sc.target;
   if (out->target_time) out->target_time[f] = sc.time;
 
-  int np = build_trajectory(m, &rs, prev, nprev, ex, ey, in->ego_yaw_deg[f], target_lane, ed, evd,
-                            &sc, out->next_x + f * PP_PATH_LEN, out->next_y + f * PP_PATH_LEN,
+  int np = build_trajectory(m, cfg, &rs, prev, nprev, ex, ey, in->ego_yaw_deg[f], target_lane, ed,
+                            evd, &sc, out->next_x + f * PP_PATH_LEN, out->next_y + f * PP_PATH_LEN,
                             &flags);
   out->n_points[f] = np;
   out->ego_lane[f] = elane;
@@ -1001,26 +1026,27 @@ void ppo_map_table(ppo_map *m, double *out) { memcpy(out, m->t, (size_t)m->n * P
 
 typedef struct {
   const ppo_map *m;
+  const pp_config *cfg;
   const pp_frames *in;
   const pp_plans *out;
   int64_t lo, hi;
 } span_t;
 static void *span_main(void *arg) {
   span_t *sp = (span_t *)arg;
-  for (int64_t f = sp->lo; f < sp->hi; f++) plan_frame(sp->m, sp->in, sp->out, f);
+  for (int64_t f = sp->lo; f < sp->hi; f++) plan_frame(sp->m, sp->cfg, sp->in, sp->out, f);
   return NULL;
 }
 
 /* Plan n frames with `threads` host threads (contiguous spans; the map is
  * read-only here, per-frame reference state lives on the stack). */
-int ppo_plan_frames(ppo_map *m, const pp_frames *in, const pp_plans *out, int64_t n, int threads,
-                    int want_flags) {
+int ppo_plan_frames_cfg(ppo_map *m, const pp_config *cfg, const pp_frames *in, const pp_plans *out,
+                        int64_t n, int threads, int want_flags) {
   (void)want_flags;
-  if (!m || !in || !out) return PP_E_ARG;
+  if (!m || !cfg || !in || !out) return PP_E_ARG;
   if (threads < 1) threads = 1;
   if (threads > 1024) threads = 1024;
   if (threads == 1) {
-    span_t one = {m, in, out, 0, n};
+    span_t one = {m, cfg, in, out, 0, n};
     span_main(&one);
     return PP_OK;
   }
@@ -1031,7 +1057,7 @@ int ppo_plan_frames(ppo_map *m, const pp_frames *in, const pp_plans *out, int64_
   for (int t = 0; t < threads; t++) {
     int64_t lo = t * per, hi = lo + per < n ? lo + per : n;
     if (lo >= hi) break;
-    span_t s1 = {m, in, out, lo, hi};
+    span_t s1 = {m, cfg, in, out, lo, hi};
     sp[t] = s1;
     pthread_create(&tid[t], NULL, span_main, &sp[t]);
     started++;
@@ -1040,6 +1066,10 @@ int ppo_plan_frames(ppo_map *m, const pp_frames *in, const pp_plans *out, int64_
   free(tid);
   free(sp);
   return PP_OK;
+}
+int ppo_plan_frames(ppo_map *m, const pp_frames *in, const pp_plans *out, int64_t n, int threads,
+                    int want_flags) {
+  return ppo_plan_frames_cfg(m, &default_cfg, in, out, n, threads, want_flags);
 }
 
 void ppo_distancesq_pt_seg(const double *px, const double *py, const double *ax, const double *ay,
@@ -1184,10 +1214,10 @@ void ppo_get_xy(const double *s, const double *d, const double *ms, const double
   for (int64_t i = 0; i < n; i++) get_xy(s[i], d[i], ms, mx, my, nwp, &ox[i], &oy[i]);
 }
 
-void ppo_lane_change(const int32_t *car_id, const double *car_s, const double *car_vs,
-                     const int32_t *car_lane, int32_t nc, const int32_t *ego_lane,
-                     const int32_t *target_lane, const double *ego_s, const double *ego_vs,
-                     const double *dt0, int32_t *out, int64_t n) {
+void ppo_lane_change_cfg(const pp_config *cfg, const int32_t *car_id, const double *car_s,
+                         const double *car_vs, const int32_t *car_lane, int32_t nc,
+                         const int32_t *ego_lane, const int32_t *target_lane, const double *ego_s,
+                         const double *ego_vs, const double *dt0, int32_t *out, int64_t n) {
   for (int64_t i = 0; i < n; i++) {
     car_t cars[PP_MAX_CARS];
     int k = 0;
@@ -1208,35 +1238,50 @@ void ppo_lane_change(const int32_t *car_id, const double *car_s, const double *c
       cars[pos] = c;
     }
     uint32_t fl = 0;
-    out[i] = choose_lane(cars, k, ego_lane[i], target_lane[i], ego_s[i], ego_vs[i], dt0[i], 0, &fl);
+    out[i] = choose_lane(cfg, cars, k, ego_lane[i], target_lane[i], ego_s[i], ego_vs[i], dt0[i], &fl);
   }
 }
+void ppo_lane_change(const int32_t *car_id, const double *car_s, const double *car_vs,
+                     const int32_t *car_lane, int32_t nc, const int32_t *ego_lane,
+                     const int32_t *target_lane, const double *ego_s, const double *ego_vs,
+                     const double *dt0, int32_t *out, int64_t n) {
+  ppo_lane_change_cfg(&default_cfg, car_id, car_s, car_vs, car_lane, nc, ego_lane, target_lane,
+                      ego_s, ego_vs, dt0, out, n);
+}
 
-void ppo_limit_speed(const double *car_vx, const double *car_vy, const double *next_s,
-                     const double *ego_s, const double *ego_speed, const double *ego_acc,
-                     const int32_t *in_lane, double *ls_speed, double *ls_time, double *sc_speed_o,
-                     double *sc_time, uint32_t *flags, int64_t n) {
+void ppo_limit_speed_cfg(const pp_config *cfg, const double *car_vx, const double *car_vy,
+                         const double *next_s, const double *ego_s, const double *ego_speed,
+                         const double *ego_acc, const int32_t *in_lane, double *ls_speed,
+                         double *ls_time, double *sc_speed_o, double *sc_time, uint32_t *flags,
+                         int64_t n) {
   for (int64_t i = 0; i < n; i++) {
     uint32_t fl = 0;
-    limit_speed(car_vx[i], car_vy[i], next_s[i], ego_s[i], ego_speed[i], ego_acc[i], in_lane[i],
-                &ls_speed[i], &ls_time[i], &fl);
+    limit_speed(cfg, car_vx[i], car_vy[i], next_s[i], ego_s[i], ego_speed[i], ego_acc[i],
+                in_lane[i], &ls_speed[i], &ls_time[i], &fl);
     speedctl sc;
-    sc_init(&sc, ego_speed[i]);
+    sc_init(cfg, &sc, ego_speed[i]);
     sc_limit(&sc, ls_speed[i], ls_time[i]);
     sc_speed_o[i] = sc.target;
     sc_time[i] = sc.time;
     flags[i] = fl & (PP_F_COLLISION | PP_F_BRAKE | PP_F_MAXBRAKE | PP_F_ADJUST | PP_F_KEEP);
   }
 }
+void ppo_limit_speed(const double *car_vx, const double *car_vy, const double *next_s,
+                     const double *ego_s, const double *ego_speed, const double *ego_acc,
+                     const int32_t *in_lane, double *ls_speed, double *ls_time, double *sc_speed_o,
+                     double *sc_time, uint32_t *flags, int64_t n) {
+  ppo_limit_speed_cfg(&default_cfg, car_vx, car_vy, next_s, ego_s, ego_speed, ego_acc, in_lane,
+                      ls_speed, ls_time, sc_speed_o, sc_time, flags, n);
+}
 
 /* TrajectoryBuilder::build on explicit inputs (the reference point is the last
  * kept previous point, or the telemetry pose on a cold start). */
-void ppo_trajectory_build(ppo_map *m, const int32_t *prev_n, const double *prev_x,
-                          const double *prev_y, const double *ego_x, const double *ego_y,
-                          const double *yaw, const int32_t *target_lane, const double *ego_d,
-                          const double *ego_vd, const double *sc_start, const double *sc_target,
-                          const double *sc_time, double *out_x, double *out_y, int32_t *out_n,
-                          uint32_t *out_flags, int64_t n) {
+void ppo_trajectory_build_cfg(ppo_map *m, const pp_config *cfg, const int32_t *prev_n,
+                              const double *prev_x, const double *prev_y, const double *ego_x,
+                              const double *ego_y, const double *yaw, const int32_t *target_lane,
+                              const double *ego_d, const double *ego_vd, const double *sc_start,
+                              const double *sc_target, const double *sc_time, double *out_x,
+                              double *out_y, int32_t *out_n, uint32_t *out_flags, int64_t n) {
   const int K = PP_PREV_KEEP;
   for (int64_t i = 0; i < n; i++) {
     vec2 prev[PP_PREV_KEEP];
@@ -1254,10 +1299,20 @@ void ppo_trajectory_build(ppo_map *m, const int32_t *prev_n, const double *prev_
     sc.target = sc_target[i];
     sc.time = sc_time[i];
     uint32_t fl = 0;
-    out_n[i] = build_trajectory(m, &rs, prev, nprev, rx, ry, yaw[i], target_lane[i], ego_d[i],
+    out_n[i] = build_trajectory(m, cfg, &rs, prev, nprev, rx, ry, yaw[i], target_lane[i], ego_d[i],
                                 ego_vd[i], &sc, out_x + i * PP_PATH_LEN, out_y + i * PP_PATH_LEN, &fl);
     out_flags[i] = fl;
   }
+}
+void ppo_trajectory_build(ppo_map *m, const int32_t *prev_n, const double *prev_x,
+                          const double *prev_y, const double *ego_x, const double *ego_y,
+                          const double *yaw, const int32_t *target_lane, const double *ego_d,
+                          const double *ego_vd, const double *sc_start, const double *sc_target,
+                          const double *sc_time, double *out_x, double *out_y, int32_t *out_n,
+                          uint32_t *out_flags, int64_t n) {
+  ppo_trajectory_build_cfg(m, &default_cfg, prev_n, prev_x, prev_y, ego_x, ego_y, yaw, target_lane,
+                           ego_d, ego_vd, sc_start, sc_target, sc_time, out_x, out_y, out_n,
+                           out_flags, n);
 }
 
 /* ==========================================================================

@@ -71,6 +71,62 @@ def _i32(a):
     return np.ascontiguousarray(a, dtype=np.int32)
 
 
+def _cfg_fields(cfg):
+    return tuple(getattr(cfg, name) for name, _ in abi.Config._fields_ if name != "reserved")
+
+
+# Planner tunables the parity tests run besides the reference's literals:
+#   tight  every field moved; speed overrides, curvature adjustments, KEEP / ADJUST common
+#   loose  fast and hard-accelerating: ego speeds of 30-40 m/s in the rollouts
+#   max25  an integral max_speed, for the (int)max_speed truncation of the lane statistics
+#   edges  a relaxed_acc whose significand is all ones (no cached reciprocal shortcut), zero
+#          leeway and safety distance, a weak braking deceleration
+CONFIGS = {
+    "default": {},
+    "tight": dict(relaxed_acc=3.0, min_relaxed_acc_while_braking=2.5, maximum_acc=4.0,
+                  max_speed=17.5, car_length=5.5, safety_distance=4.0, keep_distance=25.0,
+                  keep_distance_leeway=3.0, test_fast_lane_change=1),
+    "loose": dict(relaxed_acc=30.0, maximum_acc=30.0, max_speed=40.0),
+    "max25": dict(max_speed=25.0),
+    "edges": dict(relaxed_acc=3.9999999999999996, min_relaxed_acc_while_braking=0.5,
+                  keep_distance_leeway=0.0, safety_distance=0.0),
+}
+
+
+def config(name: str = "default", **fields):
+    """abi.Config: the named entry of CONFIGS over the defaults, then `fields` over that."""
+    cfg = abi.default_config()
+    for k, v in {**CONFIGS[name], **fields}.items():
+        assert hasattr(cfg, k), k
+        setattr(cfg, k, v)
+    return cfg
+
+
+def hold_over(fb, plans, rng, frac=0.3, stale=True):
+    """Turn about `frac` of the matched car slots of `fb` (plans: a plan of fb with per-car
+    outputs) into cars held over from an earlier message (pp_frames::car_frozen_*): their
+    car_x / car_y become NaN, so only the frozen values can place them.  stale=False freezes a
+    slot at exactly its own matched values; stale=True moves s by up to 30 m, d by up to 1.5 m
+    (the lane follows d) and scales vs by 0.5-1.5.  Returns (frames, mask of frozen slots)."""
+    out = fb.slice(0, fb.n).add_frozen()
+    live = np.arange(fb.max_cars)[None, :] < fb.n_cars[:, None]
+    pick = live & (plans.car_lane >= 0) & (rng.random(live.shape) < frac)
+    k = int(pick.sum())
+    s, d, vs, vd = (getattr(plans, n)[pick] for n in ("car_s", "car_d", "car_vs", "car_vd"))
+    lane = plans.car_lane[pick]
+    if stale:
+        s = s + rng.uniform(-30.0, 30.0, k)
+        d = np.clip(d + rng.uniform(-1.5, 1.5, k), 0.1, 11.9)
+        lane = np.clip(np.floor(d / 4.0), 0, 2).astype(np.int32)
+        vs = vs * rng.uniform(0.5, 1.5, k)
+    out.car_frozen_lane[pick] = lane
+    out.car_frozen_s[pick], out.car_frozen_d[pick] = s, d
+    out.car_frozen_vs[pick], out.car_frozen_vd[pick] = vs, vd
+    out.car_x[pick] = np.nan
+    out.car_y[pick] = np.nan
+    return out, pick
+
+
 class Checker:
     def __init__(self, kind: str, map_csv: str = MAP_CSV):
         path, self.pre = _PATHS[kind]
@@ -91,6 +147,17 @@ class Checker:
     def _fn(self, name):
         return getattr(self.lib, self.pre + name)
 
+    def _cfg_call(self, name, cfg):
+        """(function, leading config argument) for a planning function: the oracle's _cfg entry
+        point with any config; the reference's own code knows only its literals."""
+        if cfg is None:
+            return self._fn(name), ()
+        if self.kind != "oracle":
+            if _cfg_fields(cfg) != _cfg_fields(abi.default_config()):
+                raise ValueError(f"checker {self.kind!r} plans with the default config only")
+            return self._fn(name), ()
+        return self._fn(name + "_cfg"), (C.byref(cfg),)
+
     def map_from_points(self, wx, wy):
         fn = self._fn("map_create")
         fn.restype = C.c_void_p
@@ -103,12 +170,10 @@ class Checker:
         self._fn("map_table")(self.map, _p(out))
         return out
 
-    def plan(self, frames, threads: int = 1, want_flags: bool = True, diag=True, cars=True):
+    def plan(self, frames, threads: int = 1, want_flags: bool = True, diag=True, cars=True,
+             cfg=None):
         plans = abi.PlanBatch(frames.n, frames.max_cars, diag=diag, cars=cars)
-        fs, ps = frames.struct(), plans.struct()
-        rc = self._fn("plan_frames")(self.map, C.byref(fs), C.byref(ps), C.c_int64(frames.n),
-                                     C.c_int(threads), C.c_int(1 if want_flags else 0))
-        assert rc == 0, rc
+        self.plan_into(frames, plans, threads, want_flags, cfg)
         return plans
 
     def plan_with_log(self, frames, log_path: str):
@@ -121,10 +186,11 @@ class Checker:
         assert rc == 0, rc
         return plans
 
-    def plan_into(self, frames, plans, threads: int = 1, want_flags: bool = False):
+    def plan_into(self, frames, plans, threads: int = 1, want_flags: bool = False, cfg=None):
         fs, ps = frames.struct(), plans.struct()
-        rc = self._fn("plan_frames")(self.map, C.byref(fs), C.byref(ps), C.c_int64(frames.n),
-                                     C.c_int(threads), C.c_int(1 if want_flags else 0))
+        fn, pre = self._cfg_call("plan_frames", cfg)
+        rc = fn(self.map, *pre, C.byref(fs), C.byref(ps), C.c_int64(frames.n), C.c_int(threads),
+                C.c_int(1 if want_flags else 0))
         assert rc == 0, rc
 
     # ---- unit functions ----
@@ -202,31 +268,32 @@ class Checker:
         return ox, oy
 
     def lane_change(self, car_id, car_s, car_vs, car_lane, ego_lane, target_lane, ego_s, ego_vs,
-                    dt0):
+                    dt0, cfg=None):
         car_id, car_lane = _i32(car_id), _i32(car_lane)
         car_s, car_vs = _f64(car_s), _f64(car_vs)
         ego_lane, target_lane = _i32(ego_lane), _i32(target_lane)
         ego_s, ego_vs, dt0 = _f64(ego_s), _f64(ego_vs), _f64(dt0)
         n, nc = car_id.shape
         out = np.zeros(n, np.int32)
-        self._fn("lane_change")(_p(car_id), _p(car_s), _p(car_vs), _p(car_lane), C.c_int32(nc),
-                                _p(ego_lane), _p(target_lane), _p(ego_s), _p(ego_vs), _p(dt0),
-                                _p(out), C.c_int64(n))
+        fn, pre = self._cfg_call("lane_change", cfg)
+        fn(*pre, _p(car_id), _p(car_s), _p(car_vs), _p(car_lane), C.c_int32(nc), _p(ego_lane),
+           _p(target_lane), _p(ego_s), _p(ego_vs), _p(dt0), _p(out), C.c_int64(n))
         return out
 
-    def limit_speed(self, car_vx, car_vy, next_s, ego_s, ego_speed, ego_acc, in_lane):
+    def limit_speed(self, car_vx, car_vy, next_s, ego_s, ego_speed, ego_acc, in_lane, cfg=None):
         a = [_f64(v) for v in (car_vx, car_vy, next_s, ego_s, ego_speed, ego_acc)]
         in_lane = _i32(in_lane)
         n = len(in_lane)
         outs = [np.zeros(n) for _ in range(4)]
         flags = np.zeros(n, np.uint32)
-        self._fn("limit_speed")(*[_p(v) for v in a], _p(in_lane), *[_p(o) for o in outs],
-                                _p(flags), C.c_int64(n))
+        fn, pre = self._cfg_call("limit_speed", cfg)
+        fn(*pre, *[_p(v) for v in a], _p(in_lane), *[_p(o) for o in outs], _p(flags),
+           C.c_int64(n))
         return dict(ls_speed=outs[0], ls_time=outs[1], sc_speed=outs[2], sc_time=outs[3],
                     flags=flags)
 
     def trajectory_build(self, prev_n, prev_x, prev_y, ego_x, ego_y, yaw, target_lane, ego_d,
-                         ego_vd, sc_start, sc_target, sc_time):
+                         ego_vd, sc_start, sc_target, sc_time, cfg=None):
         prev_n, target_lane = _i32(prev_n), _i32(target_lane)
         f = [_f64(v) for v in (prev_x, prev_y, ego_x, ego_y, yaw)]
         g = [_f64(v) for v in (ego_d, ego_vd, sc_start, sc_target, sc_time)]
@@ -235,9 +302,9 @@ class Checker:
         oy = np.full((n, abi.PATH_LEN), np.nan)
         on = np.zeros(n, np.int32)
         fl = np.zeros(n, np.uint32)
-        self._fn("trajectory_build")(self.map, _p(prev_n), *[_p(v) for v in f], _p(target_lane),
-                                     *[_p(v) for v in g], _p(ox), _p(oy), _p(on), _p(fl),
-                                     C.c_int64(n))
+        fn, pre = self._cfg_call("trajectory_build", cfg)
+        fn(self.map, *pre, _p(prev_n), *[_p(v) for v in f], _p(target_lane), *[_p(v) for v in g],
+           _p(ox), _p(oy), _p(on), _p(fl), C.c_int64(n))
         return ox, oy, on, fl
 
     # ---- simulator model of the closed-loop rollouts (oracle only) ----

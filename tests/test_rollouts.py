@@ -46,16 +46,20 @@ def cpu_state_from(pp, st):
 
 
 @pytest.mark.gpu
+@pytest.mark.parametrize("cfg_name", ["default", "loose", "max25"])
 @pytest.mark.parametrize("consume_k", [1, 3])
-def test_rollout_ticks_match_cpu_model_and_planner(pp, oracle, consume_k):
+def test_rollout_ticks_match_cpu_model_and_planner(pp, oracle, consume_k, cfg_name):
+    """Planner tunables reach the planning step of the loop: `loose` (max_speed 40, hard
+    acceleration) is where the ego drives at 30-40 m/s, speeds no synthetic frame has."""
+    cfg = checkers.config(cfg_name)
     n, c, seed, first, ticks = 192, 12, 77, 1000, 60
     m = pp.Map()
     ro = pp.Rollouts(m, n, c, seed=seed, first=first)
     prev = ro.state()
     assert prev.tick == 0 and (prev.path_n == 0).all()
-    respawns = 0
+    respawns, top_speed = 0, 0.0
     for t in range(ticks):
-        ro.run(1, consume_k)
+        ro.run(1, consume_k, cfg=cfg)
         frames, plans = ro.last()
         now = ro.state()
         # 1. the frame the device simulator built from the previous state
@@ -63,7 +67,8 @@ def test_rollout_ticks_match_cpu_model_and_planner(pp, oracle, consume_k):
         for k, a in frames.arrays().items():
             assert np.array_equal(a, getattr(want_frames, k)), (t, k)
         # 2. the plan for that frame (teacher-forced)
-        assert_plans_match(plans, oracle.plan(frames, threads=4), t)
+        assert_plans_match(plans, oracle.plan(frames, threads=4, cfg=cfg), t)
+        top_speed = max(top_speed, float(plans.ego_speed.max()))
         # 3. the simulator step given the device's plan
         cpu = cpu_state_from(pp, prev)
         oracle.sim_advance(cpu, c, seed, first, consume_k, plans)
@@ -77,6 +82,8 @@ def test_rollout_ticks_match_cpu_model_and_planner(pp, oracle, consume_k):
     first_state = pp.Rollouts(m, n, c, seed=seed, first=first).state()
     moved = np.hypot(prev.ego_x - first_state.ego_x, prev.ego_y - first_state.ego_y)
     assert moved.min() > 0.5 and respawns > 0
+    if cfg_name == "loose":
+        assert top_speed > 30.0
     stats = ro.stats().cpu().numpy()
     assert stats[0] == n * ticks and stats[1] == 50 * n * ticks
 
